@@ -2,6 +2,7 @@
 """bench.py -- IPCS time steps per second, 3D Taylor-Green P2-P1 on an N^3 box (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mesh 96] [--workload cavity]
+                   [--dump-outputs DIR]
 
 One "step" = one ``FractionalStep_AB_CN.solve(dt, nu, max_iter=1)`` (fracstep.py:660-696) on the
 z-extruded Taylor-Green problem of SURVEY.md 8(d): box [-1,1]^3, N^3 x 6 Kuhn tetrahedra, P2-P1,
@@ -138,6 +139,22 @@ class ClockSampler:
         return out
 
 
+DUMP_MAX_ENTRIES = 1 << 20  # per array (8 MiB in float64): at most 4 arrays, 32 MiB per run
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write each array as <out_dir>/<name>.npy in float64, so that two builds run with the same arguments can be
+    compared output for output.  An array longer than DUMP_MAX_ENTRIES is replaced by the entries at a fixed, seeded
+    sample of sorted indices (the same indices for the same array length).  The device reductions do not sum in a
+    fixed order: two runs of one build differ by about 1e-14 relative (B200, 48^3, 10 steps)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        if a.size > DUMP_MAX_ENTRIES:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ENTRIES, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def bc_series(solver, tg, t_first: float, n_steps: int):
     """g_i at the merged BC dofs for n_steps consecutive steps, evaluated on the host ahead of time."""
     out = []
@@ -248,6 +265,9 @@ def run_cavity(args):
     st1 = ctx.stats()
     launches = comm.allreduce(int(st1.kernel_launches - st0.kernel_launches))
     umax = comm.allreduce(float(np.abs(solver._u[0].x.array_ro()).max()), "max")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**{f"u{i}": solver._u[i].x.array_ro()[:solver._nV_owned] for i in range(3)},
+                                         "p": solver._p.x.array_ro()[:solver._nQ_owned]})
     peak, peak_kind = measured_peaks()
     ms_k, bytes_k = ctx.bench_kernel(3, 20)
     if rank != 0:
@@ -666,6 +686,9 @@ def run_ours(args):
               "norm_u": float(f"{np.sqrt(su):.15e}"), "norm_p": float(f"{np.sqrt(sp):.15e}")}
     if wl == "taylor-green-z":
         checks["max_abs_w"] = comm.allreduce(float(np.abs(solver._u[2].x.array_ro()).max()), "max")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**{f"u{i}": solver._u[i].x.array_ro()[:nVo] for i in range(gd)},
+                                         "p": solver._p.x.array_ro()[:nQo]})
 
     # ---- end to end through the public API: callable BCs on the host, H2D, D2H ------------------
     # the SAME K steps again (state re-initialised, solution histories forgotten, W untimed steps first), so that
@@ -832,7 +855,16 @@ def main():
     ap.add_argument("--scalar-ksp", default="auto", choices=["auto", "cg", "chebyshev"],
                     help="mass-solve method (auto = cg; chebyshev is reduction-free but needs ~3x the iterations once the "
                          "initial guesses are good)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the velocity components and the pressure of the last timed step as "
+                         "DIR/<name>.npy (float64; a fixed seeded sample of arrays longer than 2^20 entries); one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "assembly-strategies"):
+        ap.error("--dump-outputs applies to the time-stepping workloads of --impl ours")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs writes the state of one GPU: run it on a single rank")
     KRYLOV["pressure"]["pc_type"] = args.pressure_pc
     KRYLOV["scalar"]["ksp_type"] = args.scalar_ksp if args.scalar_ksp != "auto" else "cg"
     if args.workload == "taylor-green":
