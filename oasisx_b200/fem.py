@@ -67,7 +67,8 @@ def _class_order(x: np.ndarray, lattice) -> np.ndarray:
     """Dof order for lattice (box/rectangle) meshes: group the P2 dofs by the parity class of their
     half-step lattice index (vertices, and one class per edge direction), lexicographic inside a
     class.  Consecutive dofs then have the same stencil, which is what lets a 32-row slice of the
-    sliced-ELL operator gather 32 CONSECUTIVE vector entries per step (DESIGN.md, SpMM)."""
+    sliced-ELL operator gather 32 CONSECUTIVE vector entries per step (DESIGN.md, SpMM).  A permutation for any `x`:
+    on coordinates off the lattice (a deformed box) the classes mix, which costs SpMM speed, not correctness."""
     p0, h = lattice
     idx = np.rint((x - p0) / (0.5 * h)).astype(np.int64)
     cls = (idx[:, 0] & 1) + 2 * (idx[:, 1] & 1) + 4 * (idx[:, 2] & 1)
@@ -114,13 +115,46 @@ def lattice_dof_ids(hidx: np.ndarray, shape, degree: int, order: str) -> np.ndar
     return offset[cls] + g
 
 
+def lattice_node_coordinates(mesh) -> np.ndarray:
+    """(n_nodes, 3) coordinates the box/rectangle provider gives the geometry nodes: per axis, ``np.linspace`` over the
+    box evaluated at the node's lattice index -- bitwise what `mesh.create_box` / `create_rectangle` (and a slab of
+    either) store."""
+    idx, shape = lattice_node_index(mesh), mesh._shape
+    p0, p1 = mesh._box
+    x = np.zeros((len(idx), 3))
+    for a in range(len(shape)):
+        x[:, a] = np.linspace(p0[a], p1[a], shape[a] + 1)[idx[:, a]]
+    return x
+
+
+def is_deformed(mesh) -> bool:
+    """True if the nodes of a provider-built box/rectangle mesh are no longer where the provider put them: the mesh
+    was moved in place (``mesh.geometry.x[:, 0] = ...``, e.g. graded toward the walls).  Its topology, node numbering
+    and lattice attributes are still the box's, its coordinates are not.  O(n_nodes)."""
+    return not np.array_equal(mesh.geometry.x, lattice_node_coordinates(mesh))
+
+
+def _p2_coordinates_from_geometry(mesh, cell_dofs: np.ndarray, n_dofs: int) -> np.ndarray:
+    """P2 dof coordinates from the actual geometry: vertex dofs at their nodes, edge dofs at 0.5 * (x_a + x_b) of the
+    edge's end points (`_EDGE_VERTS` order) -- what the general route computes, for any numbering of the dofs."""
+    gx, cells, d = mesh.geometry.x, mesh.geometry.dofmap, mesh.geometry.dim
+    x = np.empty((n_dofs, 3))
+    x[cell_dofs[:, : d + 1]] = gx[cells]
+    for e, (a, b) in enumerate(_EDGE_VERTS[d]):
+        x[cell_dofs[:, d + 1 + e]] = 0.5 * (gx[cells[:, a]] + gx[cells[:, b]])
+    return x
+
+
 def _lattice_p2(mesh):
     """(dof coordinates, cell dofs) of the P2 space on a provider-built box/rectangle mesh in the stencil-class order,
     from closed forms: the 3^d lattice points of every cube get their dof numbers by `lattice_dof_ids`, a cell's ten
     (six) dofs are a fixed selection of them, and the coordinates of a class are a tensor product of per-axis tables.
     No edge table, no sort -- the general route spends most of the host set-up of a 96^3 box in np.unique over 37 M cell
     edges and a four-key lexsort of 7 M points.  Same numbers and bitwise the same coordinates as the general route
-    (tests/test_host.py)."""
+    (tests/test_host.py).
+
+    The numbering depends on the topology alone, the closed-form coordinates on the box.  A box deformed in place
+    keeps the first and not the second: there the coordinates are taken from the geometry instead."""
     d, shape = mesh.geometry.dim, mesh._shape
     p0, p1 = mesh._box
     # per-axis coordinate of a half-step index: a node's own coordinate, or the midpoint of its two neighbours --
@@ -155,6 +189,8 @@ def _lattice_p2(mesh):
         edges = [pts[tuple(cv[a][k] + cv[b][k] for k in range(d))] for a, b in _EDGE_VERTS[d]]
         cols.append(np.stack(verts + edges, axis=1))
     cell_dofs = np.stack(cols, axis=1).reshape(-1, cols[0].shape[1])  # (cube, cell in cube) -> rows
+    if is_deformed(mesh):
+        x = _p2_coordinates_from_geometry(mesh, cell_dofs, n)
     return x, cell_dofs
 
 
@@ -225,6 +261,8 @@ class FunctionSpace:
         new_of_old[order] = np.arange(len(order))
         self._x = np.ascontiguousarray(x[order])
         self.dofmap = DofMap(new_of_old[cell_dofs], IndexMap(len(order)), 1)
+        if degree == 1:
+            self._dof_nodes = order  # geometry node of every dof (the pressure multigrid's lattice indices)
 
     # -- dolfinx.fem.FunctionSpace surface -------------------------------------------------
     @property

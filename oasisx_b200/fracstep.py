@@ -198,7 +198,8 @@ class FractionalStep_AB_CN:
         Vs._b2_ctx = ctx  # a Projector on one of the solver's spaces shares its device context
         self._Q._scalar._b2_ctx = ctx
         ctx.build_patterns()
-        if deg_u == 2:  # tile-major schedule of the SELL slices (L1 reuse of the gathered vector)
+        if deg_u == 2:  # tile-major schedule of the SELL slices (L1 reuse of the gathered vector); any schedule is a
+            # permutation of the slices, so a lattice that no longer fits the coordinates (a deformed box) costs speed only
             lat = getattr(mesh, "_lattice", None) if getattr(mesh, "_dof_order", "class") == "class" else None
             ctx.set_slice_order(L.PAT_VV, _fem.slice_order(Vs.tabulate_dof_coordinates()[: self._nV_owned], self._nV_owned, lat))
         self._bc_dofs: list[np.ndarray] = []
@@ -242,8 +243,14 @@ class FractionalStep_AB_CN:
         if (solver_options.get("pressure") or {}).get("pc_type") in ("mg", "gamg", "hypre") and not self._bcs_p:
             from . import multigrid as _mg
 
+            dof_nodes = getattr(self._Q, "_dof_nodes", None)
+            if dof_nodes is None:  # P1: every local dof sits on the node its cells put it on
+                cell_nodes, cell_dofs = (self._lp.cell_nodes, self._lp.Q.cell_dofs) if self._lp is not None else (
+                    mesh.geometry.dofmap, self._Q.dofmap.list)
+                dof_nodes = np.empty(self._Q.num_dofs, dtype=np.int64)
+                dof_nodes[cell_dofs.ravel()] = cell_nodes.ravel()
             self._mg_levels = _mg.attach_pressure_multigrid(
-                ctx, mesh, self._Q.tabulate_dof_coordinates(), self._nQ_owned, **(options.get("multigrid") or {})
+                ctx, mesh, dof_nodes, self._nQ_owned, **(options.get("multigrid") or {})
             )
             if self._mg_levels == 0:
                 logger.warning("pc_type=mg requested but the mesh carries no nested hierarchy: using Jacobi")

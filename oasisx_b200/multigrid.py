@@ -15,6 +15,7 @@ from __future__ import annotations
 import numpy as np
 import scipy.sparse as sp
 
+from . import fem as _fem
 from . import mesh as _mesh
 
 
@@ -49,9 +50,12 @@ def lattice_prolongation(fine_shape, coarse_shape, rows: np.ndarray | None = Non
     return P
 
 
-def box_hierarchy(msh, min_cells: int = 2, max_levels: int = 16, first_rows: np.ndarray | None = None):
+def box_hierarchy(msh, min_cells: int = 2, max_levels: int = 16, first_rows: np.ndarray | None = None,
+                  fine_x: np.ndarray | None = None):
     """[(coarse mesh, P from the previous level)] for a provider-built box/rectangle mesh.  `first_rows`: lattice
-    indices of the fine nodes the FIRST prolongation is wanted for (its rows, in that order)."""
+    indices of the fine nodes the FIRST prolongation is wanted for (its rows, in that order).  `fine_x`: coordinates of
+    all fine nodes in the provider's (lexicographic) numbering, for a box deformed in place: every coarse node then
+    takes the coordinates of the fine node it coincides with (lattice index doubled) instead of the uniform box's."""
     shape = getattr(msh, "_shape", None)
     if shape is None:
         return []
@@ -62,23 +66,33 @@ def box_hierarchy(msh, min_cells: int = 2, max_levels: int = 16, first_rows: np.
     while len(out) < max_levels and all(n % 2 == 0 for n in fine) and min(fine) // 2 >= min_cells:
         coarse = tuple(n // 2 for n in fine)
         cm = (_mesh.create_rectangle if d == 2 else _mesh.create_box)(None, [list(p0), list(p1)], list(coarse))
+        if fine_x is not None:
+            cm.geometry.x[:] = fine_x[_node_ids(2 * _fem.lattice_node_index(cm), fine)]
+            fine_x = cm.geometry.x
         out.append((cm, lattice_prolongation(fine, coarse, first_rows if not out else None)))
         fine = coarse
     return out
 
 
-def attach_pressure_multigrid(ctx, msh, xQ_local: np.ndarray, n_owned: int, **config) -> int:
-    """Build the hierarchy for the pressure space whose LOCAL dof coordinates are `xQ_local` (owned
-    first) and register it with the context.  Returns the number of coarse levels."""
+def attach_pressure_multigrid(ctx, msh, dof_nodes: np.ndarray, n_owned: int, **config) -> int:
+    """Build the hierarchy for the pressure space whose LOCAL dofs (owned first) sit on the geometry nodes
+    `dof_nodes` and register it with the context.  Returns the number of coarse levels (0: the mesh carries no
+    hierarchy).
+
+    The lattice index of a dof comes from the provider's node numbering, not from its coordinates, so a box deformed
+    in place keeps its hierarchy.  Its coarse levels take their coordinates from the deformed fine geometry (one rank,
+    or several with the replicated mesh; a slab-local mesh cannot be deformed, see `slab.SlabFunctionSpace`)."""
     if getattr(msh, "_shape", None) is None:
         return 0
-    p0, h = msh._lattice
-    d = len(msh._shape)
-    idx = np.rint((xQ_local[:, :d] - p0[:d]) / h[:d]).astype(np.int64)  # fine lattice node of each local dof
-    levels = box_hierarchy(msh, first_rows=idx[:n_owned])  # only the rows of the owned dofs: no table of the global size
+    slab = hasattr(msh, "is_global_boundary")
+    if not (slab or getattr(msh, "_canonical", False)):
+        return 0  # nodes renumbered: the lattice index of a node is unknown
+    idx = _fem.lattice_node_index(msh)[dof_nodes]  # fine lattice node of each local dof
+    fine_x = msh.geometry.x if not slab and _fem.is_deformed(msh) else None
+    levels = box_hierarchy(msh, first_rows=idx[:n_owned], fine_x=fine_x)  # rows of the owned dofs only
     if not levels:
         return 0
-    n_local = xQ_local.shape[0]
+    n_local = len(dof_nodes)
     for lvl, (cm, P) in enumerate(levels):
         if lvl == 0:
             Pl = P.tocsr()

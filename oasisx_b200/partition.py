@@ -63,7 +63,7 @@ def cell_ranks(mesh, nranks: int) -> np.ndarray:
     cells = mesh.geometry.dofmap
     zc = mesh.geometry.x[cells][:, :, d - 1].mean(axis=1)
     lattice = getattr(mesh, "_lattice", None)
-    if lattice is not None:
+    if lattice is not None:  # any layer assignment is a valid partition: on a box deformed in place only the balance suffers
         p0, h = lattice
         layer = np.floor((zc - p0[d - 1]) / h[d - 1] + 1e-9).astype(np.int64)
     else:  # no lattice: rank the cells by centroid height and cut into equal chunks

@@ -197,6 +197,10 @@ class SlabFunctionSpace(fem.FunctionSpace):
     def __init__(self, mesh: SlabMesh, degree: int):
         if degree not in (1, 2):
             raise NotImplementedError("only Lagrange degree 1 and 2 are on the B200 hot path")
+        if fem.is_deformed(mesh):
+            # the P2 coordinates and the halo plans below come from the box's closed forms and from coordinates
+            raise NotImplementedError("a slab-local mesh moved in place is not supported: deform the replicated mesh "
+                                      "(B200_GLOBAL_MESH=1), which oasisx_b200.partition cuts from the actual geometry")
         self.mesh, self.degree, self.bs = mesh, degree, 1
         self.element = fem._Element(mesh.cell_name(), degree)
         self._scalar = self

@@ -88,6 +88,8 @@ class CpuIPCS:
         vdofs = np.ascontiguousarray(vdofs, np.int32)
         qdofs = np.ascontiguousarray(qdofs, np.int32)
         self.nV, self.nQ, self.xV, self.xQ = xV.shape[0], xQ.shape[0], xV, xQ
+        self._dof_nodes = np.empty(self.nQ, dtype=np.int64)  # P1: geometry node of every pressure dof
+        self._dof_nodes[qdofs.ravel()] = cells.ravel()
         self.h = C.c_void_p(L.ipcs_cpu_create(d, deg_v, x.shape[0], _p(x), cells.shape[0], _p(cells), self.nV, _p(vdofs),
                                               self.nQ, _p(qdofs)))
         self.bcs_u = bcs_u
@@ -148,10 +150,9 @@ class CpuIPCS:
         nnz = self.L.ipcs_cpu_nnz(self.h, 3)
         ip, ix = self.pattern(3, self.nQ)
         A = sp.csr_matrix((self.matrix(3, 0, nnz), ix, ip), shape=(self.nQ, self.nQ))
-        p0, h = msh._lattice
-        d = len(msh._shape)
-        idx = np.rint((self.xQ[:, :d] - p0[:d]) / h[:d]).astype(np.int64)
-        node_of_dof = mg._node_ids(idx, msh._shape)
+        from oasisx_b200 import fem
+
+        node_of_dof = mg._node_ids(fem.lattice_node_index(msh)[self._dof_nodes], msh._shape)  # also on a deformed box
         n_levels = 0
         for lvl, (cm, P) in enumerate(levels):
             Pl = sp.csr_matrix(P)[node_of_dof, :].tocsr() if lvl == 0 else sp.csr_matrix(P)

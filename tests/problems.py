@@ -123,6 +123,65 @@ def make_mesh(gdim: int, N: int, comm=None):
     return bmesh.create_box(comm, [[-1.0, -1.0, -1.0], [1.0, 1.0, 1.0]], [N, N, N])
 
 
+def _signed_dets(x, cells, gdim):
+    X = x[cells][:, :, :gdim]
+    return np.linalg.det(np.transpose(X[:, 1:] - X[:, :1], (0, 2, 1)))
+
+
+def _scramble(msh, N, seed, keep=None):
+    """`msh` rebuilt through ``Mesh(x, cells, gdim)``, so without lattice information: only the cells `keep` (all if
+    None), the interior vertices moved by up to 0.2 h (boundary vertices, found from the exterior facets, stay put:
+    Dirichlet data from a formula stays exact), node numbering, cell order and the vertex order inside every cell
+    permuted at random.  Both orientations occur; min |det J| > 0.1 of the undeformed cells'."""
+    gdim = msh.geometry.dim
+    rng = np.random.default_rng(seed)
+    cells = msh.geometry.dofmap.astype(np.int64)
+    if keep is not None:
+        cells = cells[keep]
+    used, cells = np.unique(cells, return_inverse=True)
+    cells = cells.reshape(-1, gdim + 1)
+    x = msh.geometry.x[used].copy()
+    tmp = bmesh.Mesh(x, cells, gdim)
+    onb = np.zeros(len(x), dtype=bool)
+    onb[np.unique(tmp.topology.entities(gdim - 1)[boundary_facets(tmp)])] = True
+    h = 2.0 / N
+    dirs = rng.normal(size=(len(x), gdim))
+    dirs /= np.linalg.norm(dirs, axis=1, keepdims=True)
+    x[:, :gdim] += np.where(onb, 0.0, 0.2 * h * rng.uniform(0.0, 1.0, len(x)))[:, None] * dirs
+    new_of_old = rng.permutation(len(x))
+    xn = np.empty_like(x)
+    xn[new_of_old] = x
+    cells = new_of_old[cells][rng.permutation(len(cells))]
+    cells = np.take_along_axis(cells, np.argsort(rng.uniform(size=cells.shape), axis=1), axis=1)
+    det = _signed_dets(xn, cells, gdim)
+    assert (det > 0).any() and (det < 0).any()
+    assert np.abs(det).min() > 0.1 * h**gdim
+    return bmesh.Mesh(xn[:, :gdim], cells, gdim)
+
+
+def jittered_mesh(gdim: int, N: int, seed: int = 0):
+    """The box/rectangle of `make_mesh` as an unstructured mesh: jittered interior, scrambled numbering, no lattice."""
+    return _scramble(make_mesh(gdim, N), N, seed)
+
+
+def l_shaped_mesh(gdim: int, N: int, seed: int = 0):
+    """`jittered_mesh` with the cells of the quadrant (octant) x, y (, z) > 0 removed: a re-entrant corner, and a
+    bounding box with an empty region.  Area 3 (volume 7)."""
+    msh = make_mesh(gdim, N)
+    cen = msh.geometry.x[msh.geometry.dofmap].mean(axis=1)[:, :gdim]
+    return _scramble(msh, N, seed, keep=np.flatnonzero(~(cen > 0).all(axis=1)))
+
+
+def mapped_box(gdim: int, N: int):
+    """The provider mesh graded toward its centre planes IN PLACE (x_a -> sign(x_a) |x_a|^1.5, the usual DOLFINx
+    idiom of moving ``mesh.geometry.x``): boundary planes fixed, volume unchanged, lattice attributes kept."""
+    msh = make_mesh(gdim, N)
+    x = msh.geometry.x
+    for a in range(gdim):
+        x[:, a] = np.sign(x[:, a]) * np.abs(x[:, a]) ** 1.5
+    return msh
+
+
 def boundary_facets(msh):
     d = msh.topology.dim
     msh.topology.create_connectivity(d - 1, d)
