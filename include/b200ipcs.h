@@ -273,7 +273,7 @@ int b2_l2_error_trig(b2_ctx* ctx, int vec, int64_t n_cells_owned, int n_q, const
  * `reps` launches (CUDA events).  out[6] = ms of {convection assembly, matvec, action}, then their algorithmic bytes. */
 int b2_bench_assembly_strategies(b2_ctx* ctx, double dt, double nu, int reps, double* out);
 /* Cell schedule of assemble_first (k_first_cells): out[4] = schedule built (0/1), congruence classes found, slab
- * thickness (b2_set_tuning "first_slab"), cells.  b2_set_tuning "first_order" 0 keeps the mesh order. */
+ * thickness in reference lengths (always 1), cells.  b2_set_tuning "first_order" 0 keeps the mesh order. */
 int b2_first_plan_info(b2_ctx* ctx, int64_t* out);
 int b2_get_stats(b2_ctx* ctx, b2_stats* out);
 /* Times `reps` launches of one hot kernel on the context's stream with CUDA events (device
@@ -283,9 +283,9 @@ int b2_get_stats(b2_ctx* ctx, b2_stats* out);
  * average ms per launch and the algorithmic bytes moved. */
 int b2_bench_kernel(b2_ctx* ctx, int kernel, int reps, double* ms_per_launch, double* bytes_per_launch);
 int b2_synchronize(b2_ctx* ctx);
-/* Launch-shape knobs for the hot kernels: "spmm_blocks_per_sm", "spmm_unroll", "spmm_stream", "spmm_min_slices"
- * (0 = fixed persistent SpMM grid), "spmm_mode" (!= 0 selects a diagnostic half-kernel and makes results
- * meaningless), "first_order" / "first_slab" (cell schedule of assemble_first), "peer_grid", "graphs", "mg_dense". */
+/* Alternative schedules kept as references for the tests: "first_order" (0: assemble_first in mesh order instead
+ * of the congruence-class cell schedule), "mg_dense" (0: the pressure multigrid smooths down to its coarsest level
+ * instead of solving the first small one exactly).  Any other key is an error. */
 int b2_set_tuning(b2_ctx* ctx, const char* key, int value);
 /* CUDA events on the context's stream (slots 0..7) for callers that time a region of stage calls. */
 int b2_event_record(b2_ctx* ctx, int slot);

@@ -159,8 +159,6 @@ struct DVec {
 
 struct b2_ctx {
   int device = 0, nranks = 1, rank = 0, sm = 148;
-  int spmm_blocks_per_sm = 8, spmm_unroll = 8, spmm_mode = 0, spmm_stream = 1;  // sweep: tools/sweep_spmm.py
-  int spmm_min_slices = 1;   // tuning "spmm_min_slices": 0 = round 1's fixed persistent grid (sm x spmm_blocks_per_sm), else equal shares
   cudaStream_t stream = nullptr;
   std::string err;
   int gdim = 0;
@@ -188,7 +186,6 @@ struct b2_ctx {
   double* d_red = nullptr;  // raw reduction totals awaiting the all-reduce (multi rank, NCCL path)
   // peer-memory collectives (common.cuh): arenas mapped through CUDA IPC, no NCCL call on the data path
   int use_peer = 1;         // B200_PEER=0 keeps the NCCL path (A/B measurements, boxes without P2P)
-  int peer_grid = 128;      // tuning "peer_grid": most blocks of a halo / vector-sum kernel (two values per thread)
   bool peer_on = false;     // segment 0 imported: halo + scalar all-reduce run through peer memory
   PeerSeg seg[2];           // 0: flags, scalar slots, halo staging; 1: staging of the replicated multigrid level
   PeerDev h_peer{};
@@ -216,7 +213,6 @@ struct b2_ctx {
   int maxlen_vv = 0;        // longest row of the P2xP2 pattern
   FirstPlanHost first;      // cell schedule of assemble_first (build_first_plan)
   int first_order = 1;      // tuning "first_order": 1 = congruence-class cell order (coalesced scatter), 0 = mesh order
-  int first_slab = 1;       // tuning "first_slab": slab thickness of the class interleaving, in reference edge lengths
   // CUDA graph of one multigrid-preconditioned CG iteration of the pressure solve (single rank): ~21 dependent
   // launches of a few microseconds each become one graph launch
   cudaGraphExec_t pcg_graph = nullptr;
@@ -224,7 +220,6 @@ struct b2_ctx {
   const double* pcg_graph_x = nullptr;
   const double* pcg_graph_b = nullptr;
   int pcg_graph_launches = 0;
-  int use_graphs = 1;  // tuning "graphs"
   DBuf<int> pbc_dofs;
   bool has_pbc = false;
   double vol = 0.0;  // sum of mQ over all ranks
@@ -283,6 +278,9 @@ namespace {
   } while (0)
 
 inline int blocks_for(int64_t n, int block) { return (int)std::max<int64_t>(1, (n + block - 1) / block); }
+
+// most blocks of a peer-memory halo / vector-sum kernel (two values per thread)
+constexpr int PEER_GRID_MAX = 128;
 
 // persistent grid for grid-stride kernels: enough blocks to fill the machine, never more than needed
 inline int pgrid(const b2_ctx* c, int64_t n_items, int block = 256, int per_sm = 8) {
@@ -422,7 +420,7 @@ void halo_forward(b2_ctx* c, int space, double* v, int K) {
   const int64_t ns = h.send_off.back(), nr = h.recv_off.back();
   if (c->peer_on) {  // one kernel: remote stores into the neighbours' staging, signal, wait, unpack
     // few, fat blocks: every block polls the neighbours' flags, and the exchange is latency-, not bandwidth-bound
-    const int grid = std::max(1, std::min(c->peer_grid, blocks_for(std::max(ns, nr) * K, 512)));
+    const int grid = std::min(PEER_GRID_MAX, blocks_for(std::max(ns, nr) * K, 512));
     B2_LAUNCH(c, k_halo_peer, grid, 256, c->ph[space], K, ld, v);
     c->stats.halo_exchanges++;
     c->stats.peer_kernels++;
@@ -467,52 +465,35 @@ inline RedCtl red_ptr(b2_ctx* c) {
   return c->peer_on ? RedCtl{nullptr, c->d_peer} : RedCtl{c->d_red, nullptr};
 }
 
-template <int K, int DOT, int UNROLL, int BLOCK>
-void launch_spmm_u(b2_ctx* c, const CSR& pat, const double* vals, const double* x, int ld, double* y, const double* w,
-                   KryState* st, int fin, const double* rscale) {
+template <int K, int DOT>
+void launch_spmm(b2_ctx* c, const CSR& pat, const double* vals, const double* x, int ld, double* y, const double* w,
+                 KryState* st, int fin, const double* rscale) {
+  constexpr int BLOCK = 256;
   const int n_slices = (pat.n_rows + 31) / 32;
   const int need = (n_slices + BLOCK / 32 - 1) / (BLOCK / 32);
   // Every warp takes the same whole number k of slices (k = 1 when the grid fits): a fixed persistent grid quantises
   // small operators -- the 1/4 or 1/8 slab of a multi-GPU run got 3.07 slices per warp, i.e. 3 or 4: 103 us against 86
-  // on the 96 x 96 x 12 slab (tools/exp_slab.py) -- and is no faster on large ones.  The cap is what the grid-wide
-  // reduction has room for (one set of partial sums per block).
+  // on the 96 x 96 x 12 slab -- and is no faster on large ones.  The cap is what the grid-wide reduction has room for
+  // (one set of partial sums per block).
   const int cap = (int)std::min<int64_t>(c->partials.n / 16, (int64_t)c->sm * 32);
   const int k_slices = std::max(1, (need + cap - 1) / cap);
-  const int grid = std::max(1, c->spmm_min_slices > 0 ? (need + k_slices - 1) / k_slices : std::min(need, c->sm * c->spmm_blocks_per_sm));
+  const int grid = std::max(1, (need + k_slices - 1) / k_slices);
   B2_REQUIRE(grid <= cap, "SpMM grid exceeds the reduction scratch");
-#define B2_SPMM(STREAM_, RS_)                                                                                            \
-  B2_LAUNCH(c, (k_spmm<K, DOT, UNROLL, BLOCK, STREAM_, RS_>), grid, BLOCK, pat.n_rows, pat.slice_ptr.p, pat.scols.p, vals,    \
-            pat.order.p, x, ld, y, w, st, fin, c->partials.p, c->d_counter, red_ptr(c), rscale)
-  if (c->spmm_stream) {
-    if (rscale != nullptr) B2_SPMM(true, true);
-    else B2_SPMM(true, false);
-  } else {
-    if (rscale != nullptr) B2_SPMM(false, true);
-    else B2_SPMM(false, false);
-  }
+#define B2_SPMM(RS_)                                                                                                   \
+  B2_LAUNCH(c, (k_spmm<K, DOT, BLOCK, RS_>), grid, BLOCK, pat.n_rows, pat.slice_ptr.p, pat.scols.p, vals, pat.order.p, x, \
+            ld, y, w, st, fin, c->partials.p, c->d_counter, red_ptr(c), rscale)
+  if (rscale != nullptr) B2_SPMM(true);
+  else B2_SPMM(false);
 #undef B2_SPMM
   if (DOT > 0) reduce_finish_host(c, fin, DOT * K);
-}
-
-template <int K, int DOT>
-void launch_spmm_t(b2_ctx* c, const CSR& pat, const double* vals, const double* x, int ld, double* y, const double* w,
-                   KryState* st, int fin, const double* rscale) {
-  if (c->spmm_mode != 0) {  // diagnostic halves of the kernel (tools/sweep_spmm.py)
-    int grid = pgrid(c, (int64_t)pat.n_rows, 256, 8);
-    if (c->spmm_mode == 1) B2_LAUNCH(c, (k_spmm_diag<K, 1>), grid, 256, pat.n_rows, pat.slice_ptr.p, pat.scols.p, vals, x, ld, y);
-    else B2_LAUNCH(c, (k_spmm_diag<K, 2>), grid, 256, pat.n_rows, pat.slice_ptr.p, pat.scols.p, vals, x, ld, y);
-    return;
-  }
-  if (c->spmm_unroll >= 8) launch_spmm_u<K, DOT, 8, 256>(c, pat, vals, x, ld, y, w, st, fin, rscale);
-  else launch_spmm_u<K, DOT, 4, 256>(c, pat, vals, x, ld, y, w, st, fin, rscale);
 }
 
 template <int K>
 void launch_spmm_k(b2_ctx* c, const CSR& pat, const double* vals, const double* x, int ld, double* y, const double* w,
                    KryState* st, int fin, int dot, const double* rscale) {
-  if (dot == 0) launch_spmm_t<K, 0>(c, pat, vals, x, ld, y, w, st, fin, rscale);
-  else if (dot == 1) launch_spmm_t<K, 1>(c, pat, vals, x, ld, y, w, st, fin, rscale);
-  else launch_spmm_t<K, 2>(c, pat, vals, x, ld, y, w, st, fin, rscale);
+  if (dot == 0) launch_spmm<K, 0>(c, pat, vals, x, ld, y, w, st, fin, rscale);
+  else if (dot == 1) launch_spmm<K, 1>(c, pat, vals, x, ld, y, w, st, fin, rscale);
+  else launch_spmm<K, 2>(c, pat, vals, x, ld, y, w, st, fin, rscale);
 }
 
 // rscale: optional row scaling of the result, y = diag(rscale) (A x)
@@ -765,7 +746,7 @@ double* mg_vcycle(b2_ctx* c, int l, const double* b, double* x, double* tmp, boo
             c->mg_omega, C.b.p, partial ? (double*)nullptr : C.x.p);
   if (partial) {  // coarse levels are replicated: sum the partial restrictions of the slabs
     if (c->peer_on && c->pvs_ready) {
-      B2_LAUNCH(c, k_peer_vecsum, std::max(1, std::min(c->peer_grid, blocks_for(C.n, 1024))), 256, c->pvs, C.b.p);
+      B2_LAUNCH(c, k_peer_vecsum, std::min(PEER_GRID_MAX, blocks_for(C.n, 1024)), 256, c->pvs, C.b.p);
       c->stats.peer_kernels++;
     } else {
       B2_REQUIRE(!c->peer_on, "peer path: import segment 1 (multigrid staging) before the first pressure solve");
@@ -828,7 +809,7 @@ void pcg_mg_solve(b2_ctx* c, const double* b, double* x, int32_t* reason, int32_
   };
   // Iterations 1, 2, ... are identical streams of small dependent kernels (all scalars live in device memory):
   // captured once into a CUDA graph and replayed.  Multi-rank contexts keep plain launches (NCCL calls in between).
-  const bool graphs = c->use_graphs && (c->nranks == 1 || (c->peer_on && c->pvs_ready));  // no NCCL call inside the body
+  const bool graphs = c->nranks == 1 || (c->peer_on && c->pvs_ready);  // no NCCL call inside the body
   for (int it = 0; it <= o.maxit; ++it) {
     if (it >= first_poll) {
       B2_CUDA(cudaMemcpyAsync(c->h_st, c->d_st, sizeof(KryState), cudaMemcpyDeviceToHost, c->stream));
@@ -1009,7 +990,7 @@ void build_first_plan(b2_ctx* c) {
     for (int k = 0; k < 3; ++k) kk.q[k] = k < d ? (int64_t)std::floor((cen[3 * e + k] - lo[k]) / h * 8.0) : 0;  // h/8 bins
   }
   const int zk = d - 1;
-  const int64_t slab = 8 * (int64_t)std::max(1, c->first_slab);  // bins per slab: first_slab reference lengths
+  const int64_t slab = 8;  // bins per slab: one reference length
   std::sort(keys.begin(), keys.end(), [&](const Key& a, const Key& b) {
     const int64_t sa = a.q[zk] / slab, sb = b.q[zk] / slab;
     if (sa != sb) return sa < sb;
@@ -2586,7 +2567,7 @@ int b2_first_plan_info(b2_ctx* c, int64_t* out) {
   return guarded(c, [&] {
     out[0] = c->first.ready ? 1 : 0;
     out[1] = c->first.n_classes;
-    out[2] = c->first_slab;
+    out[2] = 1;  // slab thickness of the class interleaving, in reference lengths
     out[3] = c->n_cells;
   });
 }
@@ -2638,16 +2619,9 @@ int b2_set_tuning(b2_ctx* c, const char* key, int value) {
   return guarded(c, [&] {
     c->cfg_version++;
     std::string k(key);
-    if (k == "spmm_blocks_per_sm") c->spmm_blocks_per_sm = std::max(1, std::min(value, 32));
-    else if (k == "spmm_unroll") c->spmm_unroll = value;
-    else if (k == "spmm_min_slices") c->spmm_min_slices = std::max(0, value);
-    else if (k == "spmm_mode") c->spmm_mode = value;
-    else if (k == "spmm_stream") c->spmm_stream = value;
-    else if (k == "mg_dense") c->mg_dense_on = value;
-    else if (k == "graphs") c->use_graphs = value;
-    else if (k == "peer_grid") c->peer_grid = std::max(1, std::min(value, 148));
-    else if (k == "first_order" || k == "first_slab") {
-      (k == "first_order" ? c->first_order : c->first_slab) = std::max(0, value);
+    if (k == "mg_dense") c->mg_dense_on = value;
+    else if (k == "first_order") {
+      c->first_order = std::max(0, value);
       if (c->preassembled) build_first_plan(c);
     }
     else throw B2Error(-2, "unknown tuning key " + k);
@@ -2696,7 +2670,7 @@ int b2_bench_kernel(b2_ctx* c, int kernel, int reps, double* ms_per_launch, doub
         case 12: allreduce_sum(c, c->d_sums, 3); break;
         case 13:
           B2_REQUIRE(c->peer_on && c->pvs_ready, "vector-sum benchmark needs the peer path with a multigrid attached");
-          B2_LAUNCH(c, k_peer_vecsum, std::max(1, std::min(c->peer_grid, blocks_for(c->mg[0].n, 1024))), 256, c->pvs, c->mg[0].b.p);
+          B2_LAUNCH(c, k_peer_vecsum, std::min(PEER_GRID_MAX, blocks_for(c->mg[0].n, 1024)), 256, c->pvs, c->mg[0].b.p);
           break;
         default: throw B2Error(-2, "unknown bench kernel");
       }

@@ -304,15 +304,15 @@ __global__ void k_sell_convert(int n_rows, const int* __restrict__ rowptr, const
 // ---- SELL SpMM: y_k[row] = sum_t vals[slot] * x_k[cols[slot]], k < K ------------------------------
 //   DOT == 0: no reduction          DOT == 1: sums[k] = y_k . w_k
 //   DOT == 2: sums[k] = y_k . w_k , sums[K+k] = y_k . y_k
-// Persistent grid: warp w of the grid walks slices w, w + nwarps, ...  The t-loop is unrolled by 4:
-// four independent (column -> gather) chains per thread keep enough loads in flight to cover HBM
+// Persistent grid: warp w of the grid walks slices w, w + nwarps, ...  The t-loop is unrolled by 8:
+// eight independent (column -> gather) chains per thread keep enough loads in flight to cover HBM
 // latency at < 100% occupancy.
 // Scheduling: `order` lists the slices tile by tile (all stencil classes of one small spatial tile
 // are adjacent in the list, fem.slice_order); a block takes blockDim/32 consecutive list entries at
 // a time, so the warps of a block gather from the same neighbourhood of x concurrently and share
 // those lines in L1 instead of each pulling them through the L2 fabric.
 // MINB: resident blocks per SM the register allocation is bounded for (8 x 256 threads = 32 registers, 6 = 40).
-template <int K, int DOT, int UNROLL, int BLOCK, bool STREAM, bool RS = false, int MINB = 2048 / BLOCK>
+template <int K, int DOT, int BLOCK, bool RS = false, int MINB = 2048 / BLOCK>
 __global__ void __launch_bounds__(BLOCK, MINB)
 k_spmm(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ cols,
        const double* __restrict__ vals, const int* __restrict__ order, const double* __restrict__ x, int ld,
@@ -322,6 +322,7 @@ k_spmm(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ co
   const int lane = threadIdx.x & 31;
   const int wib = threadIdx.x >> 5;
   constexpr int WPB = BLOCK / 32;
+  constexpr int UNROLL = 8;
   const int n_slices = (n_rows + 31) >> 5;
   constexpr int ND = DOT == 0 ? 1 : DOT * K;
   // the running dot products live in shared memory between slices: keeping them in registers across
@@ -348,8 +349,8 @@ k_spmm(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ co
       double v[UNROLL];
 #pragma unroll
       for (int u = 0; u < UNROLL; ++u) {
-        c[u] = STREAM ? ld_stream(cp + ((t + u) << 5)) : __ldg(cp + ((t + u) << 5));
-        v[u] = STREAM ? ld_stream(vp + ((t + u) << 5)) : __ldg(vp + ((t + u) << 5));
+        c[u] = ld_stream(cp + ((t + u) << 5));
+        v[u] = ld_stream(vp + ((t + u) << 5));
       }
       double xv[UNROLL][K];
 #pragma unroll
@@ -362,8 +363,8 @@ k_spmm(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ co
         for (int k = 0; k < K; ++k) acc[k] = fma(v[u], xv[u][k], acc[k]);
     }
     for (; t < len; ++t) {
-      const int c = STREAM ? ld_stream(cp + (t << 5)) : __ldg(cp + (t << 5));
-      const double v = STREAM ? ld_stream(vp + (t << 5)) : __ldg(vp + (t << 5));
+      const int c = ld_stream(cp + (t << 5));
+      const double v = ld_stream(vp + (t << 5));
 #pragma unroll
       for (int k = 0; k < K; ++k) acc[k] = fma(v, __ldg(x + (size_t)k * ld + c), acc[k]);
     }
@@ -397,42 +398,6 @@ k_spmm(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ co
 #pragma unroll
     for (int i = 0; i < ND; ++i) dots[i] = sdots[i][threadIdx.x];
     reduce_finish<ND>(dots, partials, counter, fin, st, red_out);
-  }
-}
-
-// Diagnostic variants of the SpMM (b2_set_tuning "spmm_mode"): 1 = stream values/columns only (no
-// gather), 2 = gather only (values taken as 1).  Results are meaningless; they time the two halves.
-template <int K, int MODE>
-__global__ void __launch_bounds__(256)
-k_spmm_diag(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ cols,
-            const double* __restrict__ vals, const double* __restrict__ x, int ld, double* __restrict__ y) {
-  const int lane = threadIdx.x & 31;
-  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int nwarps = (gridDim.x * blockDim.x) >> 5;
-  const int n_slices = (n_rows + 31) >> 5;
-  for (int s = warp; s < n_slices; s += nwarps) {
-    const int base = __ldg(slice_ptr + s);
-    const int len = (__ldg(slice_ptr + s + 1) - base) >> 5;
-    const int row = (s << 5) + lane;
-    double acc[K];
-#pragma unroll
-    for (int k = 0; k < K; ++k) acc[k] = 0.0;
-#pragma unroll 4
-    for (int t = 0; t < len; ++t) {
-      const int c = __ldg(cols + base + lane + (t << 5));
-      if constexpr (MODE == 1) {
-        const double v = __ldg(vals + base + lane + (t << 5));
-#pragma unroll
-        for (int k = 0; k < K; ++k) acc[k] = fma(v, (double)(c + k), acc[k]);
-      } else {
-#pragma unroll
-        for (int k = 0; k < K; ++k) acc[k] += __ldg(x + (size_t)k * ld + c);
-      }
-    }
-    if (row < n_rows) {
-#pragma unroll
-      for (int k = 0; k < K; ++k) y[(size_t)k * ld + row] = acc[k];
-    }
   }
 }
 

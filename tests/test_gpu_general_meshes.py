@@ -370,34 +370,13 @@ def test_medium_jittered_box_matches_the_cpu_port(medium):
         assert _seen("medium_cpu_port", relerr(s._p.x.array_ro(), c.get(cpu.P))) <= 1e-8, n
 
 
-def test_spmm_launch_variants_are_bitwise_equal(medium):
-    """The SpMM tuning grid (unroll, stream, min slices, blocks per SM) changes how rows are distributed over the
-    GPU, not the order of the FMAs inside a row: every variant gives the same bits, and the scipy product to 1e-13."""
+def test_spmm_matches_scipy_on_the_medium_jittered_box(medium):
+    """M x, K x and A x (after assemble_first) through the device SpMM against the scipy product to 1e-13."""
     msh, tg, s, dt, nu = medium
     s.assemble_first(dt, nu)
     x = np.random.default_rng(3).uniform(-1, 1, s._Vi[0][0].num_dofs)
-    mats = {"M": s._M, "K": s._K, "A": s._A}
-    ref = {k: _csr(m) @ x for k, m in mats.items()}
-    first = {}
-    try:
-        for unroll in (4, 8):
-            for stream in (0, 1):
-                for min_slices in (0, 1):
-                    for bps in (1, 8):
-                        for key, v in (("spmm_unroll", unroll), ("spmm_stream", stream), ("spmm_min_slices", min_slices),
-                                       ("spmm_blocks_per_sm", bps)):
-                            s._ctx.set_tuning(key, v)
-                        for k, m in mats.items():
-                            y = np.zeros(len(x))
-                            m.mult(x, y)
-                            assert _seen("spmm_variants", relerr(y, ref[k])) <= 1e-13, (k, unroll, stream, min_slices, bps)
-                            if k in first:
-                                np.testing.assert_array_equal(y, first[k], err_msg=str((k, unroll, stream, min_slices, bps)))
-                            else:
-                                first[k] = y
-    finally:
-        for key, v in (("spmm_unroll", 8), ("spmm_stream", 1), ("spmm_min_slices", 1), ("spmm_blocks_per_sm", 8)):
-            s._ctx.set_tuning(key, v)
+    for k, m in {"M": s._M, "K": s._K, "A": s._A}.items():
+        assert _seen("spmm", relerr(mult(m, x), _csr(m) @ x)) <= 1e-13, k
 
 
 def test_dof_orders_give_the_same_fields():

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Sweep SpMM launch shapes / cache policies / schedules on the GPU.  Usage: python tools/sweep_spmm.py [mesh]"""
+"""Sweep the tile size of the SpMM slice schedule on the GPU.  Usage: python tools/sweep_spmm.py [mesh]"""
 import os
 import sys
 
