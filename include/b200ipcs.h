@@ -190,7 +190,23 @@ int b2_declare_pressure_bcs(b2_ctx* ctx, int any);
 int b2_pressure_mg_add_level(b2_ctx* ctx, int64_t n_nodes, const double* x, int64_t n_cells, const int32_t* cell_nodes,
                              int64_t n_fine_rows, const int32_t* P_indptr, const int32_t* P_indices, const double* P_vals,
                              const int32_t* R_indptr, const int32_t* R_indices, const double* R_vals);
+/* nu_pre, nu_post and coarse_sweeps apply to both kinds of hierarchy; omega is the damping of GEOMETRIC levels only
+ * (an algebraic hierarchy damps every level, the fine one included, with its own 4 / (3 rho_l)). */
 int b2_pressure_mg_configure(b2_ctx* ctx, int nu_pre, int nu_post, int coarse_sweeps, double omega);
+/* Smoothed-aggregation algebraic multigrid built on the device from the assembled pressure matrix Ap, for meshes
+ * without a nested hierarchy (pc_type gamg / hypre).  Strength graph: every nonzero off-diagonal entry.  Aggregates:
+ * MIS(2) of that graph with hash keys (Bell, Dalton and Olson 2012).  P = (I - 4/(3 rho) D^-1 A) T with T the
+ * aggregate indicator, R = P^T, A_c = R A P, repeated until a level has at most 5000 dofs (solved exactly), the
+ * coarsening ratio drops below 2, or 15 coarse levels; rho = 20 power iterations on D^-1 A.  Deterministic: the same
+ * Ap gives the same hierarchy bit for bit.  Call after b2_preassemble on a context without multigrid levels, on one
+ * rank, without pressure Dirichlet dofs (the coarse solve relies on the constant null space); otherwise an error. */
+int b2_pressure_amg_build(b2_ctx* ctx);
+/* out[7] = {n, nnz(A_l), nnz(P_l), algebraic (0/1), solved densely (0/1), omega_l, rho_hat_l} of level `level`
+ * (0 = the fine level: nnz(P) = 0; rho_hat = 0 on geometric levels). */
+int b2_pressure_mg_level_info(b2_ctx* ctx, int level, double* out);
+/* Test hook: level >= 1, what = 0: A_l as CSR with sorted columns, 1: P_l, 2: R_l (indptr, indices, vals; sizes from
+ * b2_pressure_mg_level_info); 3 (algebraic levels): `indices` receives the aggregate of every dof of level - 1. */
+int b2_pressure_mg_get_level(b2_ctx* ctx, int level, int what, int32_t* indptr, int32_t* indices, double* vals);
 
 /* ---- _preassemble (fracstep.py:360-409) ----------------------------------------------- */
 int b2_preassemble(b2_ctx* ctx, const double* body_force, int low_memory, int rotational);
@@ -247,7 +263,8 @@ int b2_project_solve(b2_ctx* ctx, double* x, int32_t* reasons);
 int b2_project_set_bcs(b2_ctx* ctx, int target_space, int n_comp, int64_t n, const int32_t* dofs, const double* values);
 /* KSPSolver.solve (ksp.py:71-78): Mat x = b with the options of solver slot `solver`, then scatter_forward;
  * b and x are host vectors of the operator's space (owned + ghosts), x is the initial guess when
- * ksp_initial_guess_nonzero is set.  Square operators only (B2_MAT_M, _K, _A, _AP, _MQ). */
+ * ksp_initial_guess_nonzero is set.  Square operators only (B2_MAT_M, _K, _A, _AP, _MQ).  A solve on the pressure
+ * slot reports its iterations in b2_stats.its_pressure. */
 int b2_ksp_solve(b2_ctx* ctx, int solver, int mat, const double* b, double* x, int32_t* reason);
 
 /* ---- functionals (assemble_scalar, demo/taylor_green.py:204-207) ----------------------- */

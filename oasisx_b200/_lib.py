@@ -27,7 +27,8 @@ SYMBOLS = [
     "b2_abi_version", "b2_device_count", "b2_nccl_unique_id", "b2_create", "b2_destroy", "b2_last_error",
     "b2_host_alloc", "b2_host_free", "b2_set_mesh", "b2_set_space", "b2_set_halo", "b2_set_global_sizes",
     "b2_first_plan_info", "b2_bench_assembly_strategies", "b2_peer_export", "b2_peer_import", "b2_peer_disable", "b2_peer_enabled",
-    "b2_build_patterns", "b2_pattern_nnz", "b2_pattern_sell_slots", "b2_set_slice_order", "b2_pressure_mg_add_level", "b2_pressure_mg_configure", "b2_get_pattern", "b2_set_velocity_bc_dofs",
+    "b2_build_patterns", "b2_pattern_nnz", "b2_pattern_sell_slots", "b2_set_slice_order", "b2_pressure_mg_add_level", "b2_pressure_mg_configure", "b2_pressure_amg_build",
+    "b2_pressure_mg_level_info", "b2_pressure_mg_get_level", "b2_get_pattern", "b2_set_velocity_bc_dofs",
     "b2_set_velocity_bc_values", "b2_set_velocity_bc_series", "b2_select_bc_step", "b2_reset_time_history", "b2_profiler_range", "b2_set_pressure_bc_dofs", "b2_declare_pressure_bcs", "b2_preassemble", "b2_set_vector", "b2_get_vector",
     "b2_get_matrix_values", "b2_mat_mult", "b2_set_solver_option", "b2_assemble_first", "b2_tentative_assemble",
     "b2_tentative_solve", "b2_pressure_assemble", "b2_pressure_solve", "b2_velocity_update", "b2_step_begin", "b2_step",
@@ -103,6 +104,9 @@ def load_library() -> C.CDLL:
         "b2_set_slice_order": (i32, [vp, i32, i64, vp]),
         "b2_pressure_mg_add_level": (i32, [vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp]),
         "b2_pressure_mg_configure": (i32, [vp, i32, i32, i32, dbl]),
+        "b2_pressure_amg_build": (i32, [vp]),
+        "b2_pressure_mg_level_info": (i32, [vp, i32, vp]),
+        "b2_pressure_mg_get_level": (i32, [vp, i32, i32, vp, vp, vp]),
         "b2_get_pattern": (i32, [vp, i32, vp, vp]),
         "b2_set_velocity_bc_dofs": (i32, [vp, i32, i64, vp]),
         "b2_set_velocity_bc_values": (i32, [vp, i32, i64, vp]),
@@ -244,6 +248,39 @@ class Context:
 
     def pressure_mg_configure(self, nu_pre=1, nu_post=1, coarse_sweeps=16, omega=0.85):
         self._check(self.lib.b2_pressure_mg_configure(self._h, nu_pre, nu_post, coarse_sweeps, omega), "b2_pressure_mg_configure")
+
+    def pressure_amg_build(self):
+        """Smoothed-aggregation hierarchy from the assembled pressure matrix (after preassemble, one rank)."""
+        self._check(self.lib.b2_pressure_amg_build(self._h), "b2_pressure_amg_build")
+
+    MG_LEVEL_INFO = ("n", "nnz_A", "nnz_P", "algebraic", "dense", "omega", "rho_hat")
+
+    def pressure_mg_level_info(self, level: int) -> dict:
+        out = np.zeros(7, dtype=np.float64)
+        self._check(self.lib.b2_pressure_mg_level_info(self._h, level, _ptr(out)), "b2_pressure_mg_level_info")
+        d = dict(zip(self.MG_LEVEL_INFO, out.tolist()))
+        for k in ("n", "nnz_A", "nnz_P", "algebraic", "dense"):
+            d[k] = int(d[k])
+        return d
+
+    def pressure_mg_get_level(self, level: int, what: int):
+        """what = 0: A_l, 1: P_l, 2: R_l as scipy CSR; 3: the aggregate of every dof of level - 1 (int32 array)."""
+        import scipy.sparse as sp
+
+        info = self.pressure_mg_level_info(level)
+        n, nf = info["n"], self.pressure_mg_level_info(level - 1)["n"]
+        if what == 3:
+            agg = np.empty(nf, dtype=np.int32)
+            self._check(self.lib.b2_pressure_mg_get_level(self._h, level, 3, None, _ptr(agg), None), "b2_pressure_mg_get_level")
+            return agg
+        shape = {0: (n, n), 1: (nf, n), 2: (n, nf)}[what]
+        nnz = info["nnz_A"] if what == 0 else info["nnz_P"]
+        indptr = np.empty(shape[0] + 1, dtype=np.int32)
+        indices = np.empty(nnz, dtype=np.int32)
+        vals = np.empty(nnz, dtype=np.float64)
+        self._check(self.lib.b2_pressure_mg_get_level(self._h, level, what, _ptr(indptr), _ptr(indices), _ptr(vals)),
+                    "b2_pressure_mg_get_level")
+        return sp.csr_matrix((vals, indices, indptr), shape=shape)
 
     def pattern(self, which: int, n_rows: int):
         nnz = self.lib.b2_pattern_nnz(self._h, which)

@@ -19,6 +19,7 @@
 #include "elem.cuh"
 #include "linalg.cuh"
 #include "mg.cuh"
+#include "amg.cuh"
 
 namespace {
 
@@ -117,6 +118,11 @@ struct MgLevel {
   // transfer operators to/from the previous (finer) level, CSR with scalar values
   CSR P, R;  // P: rows = owned dofs of the finer level, cols = this level;  R = P^T
   DBuf<double> Pv, Rv;
+  // algebraic levels (b2_pressure_amg_build): own damping 4 / (3 rho), rho = estimated spectral radius of D^-1 A, and
+  // the aggregate of every dof of the finer level.  Geometric levels keep omega = 0: they smooth with ctx->mg_omega.
+  bool algebraic = false;
+  double omega = 0.0, rho = 0.0;
+  DBuf<int> agg;
 };
 
 // one IPC-exported allocation of this rank and the peers' mappings of theirs
@@ -173,6 +179,7 @@ struct b2_ctx {
   // 6/7 is the optimal damping of the 7-point stencil the Kuhn P1 stiffness reduces to); b2_pressure_mg_configure overrides
   int mg_pre = 1, mg_post = 1, mg_coarse = 16;
   double mg_omega = 0.85;
+  double mg_omega0 = 0.0, mg_rho0 = 0.0;  // fine-level damping and rho(D^-1 Ap) of an algebraic hierarchy (0: geometric)
   DBuf<double> mg_x0, mg_t0;  // fine-level work vectors (n_local of Q)
   DBuf<MgDev> mg_dev;         // device descriptors of the coarse levels (index = level - 1)
   int mg_dev_levels = 0;      // number of levels the descriptor array was built for
@@ -394,6 +401,28 @@ void build_sell(b2_ctx* c, CSR& pat) {
   pat.scols.zero(c->stream);
   pat.diag_t.alloc(n_rows);
   B2_LAUNCH(c, k_sell_fill_cols, blocks_for(n_rows, 256), 256, n_rows, pat.rowptr.p, pat.cols.p, pat.slice_ptr.p, pat.scols.p, pat.diag_t.p, pat.n_cols);
+  B2_CUDA(cudaStreamSynchronize(c->stream));
+}
+
+// Assembly with a fixed summation order: k_assemble_square's (slot, value) pairs in cell order, stably sorted by slot,
+// each slot summed sequentially.  The same mesh gives the same bits on every run (atomicAdd does not).
+template <typename Launch>
+void assemble_in_fixed_order(b2_ctx* c, int64_t n_pairs, int64_t slots, double* vals, Launch&& launch) {
+  B2_REQUIRE(slots < 0xffffffffll, "operator too large for 32-bit slot keys");
+  DBuf<unsigned> k0, k1;
+  DBuf<double> v0, v1;
+  k0.alloc(n_pairs); k1.alloc(n_pairs);
+  v0.alloc(n_pairs); v1.alloc(n_pairs);
+  B2_CUDA(cudaMemsetAsync(k0.p, 0xff, sizeof(unsigned) * (size_t)n_pairs, c->stream));
+  launch(k0.p, v0.p);
+  cub::DoubleBuffer<unsigned> kb(k0.p, k1.p);
+  cub::DoubleBuffer<double> vb(v0.p, v1.p);
+  size_t bytes = 0;
+  B2_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, kb, vb, n_pairs, 0, 32, c->stream));
+  DBuf<char> tmp;
+  tmp.alloc((int64_t)bytes);
+  B2_CUDA(cub::DeviceRadixSort::SortPairs(tmp.p, bytes, kb, vb, n_pairs, 0, 32, c->stream));
+  B2_LAUNCH(c, k_sum_slot_runs, blocks_for(n_pairs, 256), 256, n_pairs, kb.Current(), vb.Current(), vals);
   B2_CUDA(cudaStreamSynchronize(c->stream));
 }
 
@@ -628,7 +657,14 @@ struct MgView {
   int n, ld;
   const CSR* pat;
   const double *A, *dinv;
+  double omega;
 };
+
+// Jacobi damping of level l: its own on an algebraic hierarchy, the configured one on a geometric one
+double mg_level_omega(const b2_ctx* c, int l) {
+  const double w = l == 0 ? c->mg_omega0 : c->mg[l - 1].omega;
+  return w > 0.0 ? w : c->mg_omega;
+}
 
 void cgz_finish(b2_ctx* c, int fin, int n);
 
@@ -639,17 +675,17 @@ void mg_sweeps(b2_ctx* c, const MgView& L, bool fine, const double* b, double*& 
   const int g = pgrid(c, L.n, 256, 8);
   int s = 0;
   if (from_zero && n_sweeps > 0) {
-    if (!first_done) B2_LAUNCH(c, k_mg_first, pgrid(c, L.n), 256, (int64_t)L.n, L.dinv, b, c->mg_omega, x);
+    if (!first_done) B2_LAUNCH(c, k_mg_first, pgrid(c, L.n), 256, (int64_t)L.n, L.dinv, b, L.omega, x);
     s = 1;
   }
   for (; s < n_sweeps; ++s) {
     if (fine) halo_forward(c, B2_SPACE_Q, x, 1);
     if (rz_fin >= 0 && s == n_sweeps - 1) {
-      B2_LAUNCH(c, k_mg_sweep_rz, g, 256, L.n, L.pat->slice_ptr.p, L.pat->scols.p, L.A, L.dinv, b, x, c->mg_omega, tmp, rz_fin, c->d_st,
+      B2_LAUNCH(c, k_mg_sweep_rz, g, 256, L.n, L.pat->slice_ptr.p, L.pat->scols.p, L.A, L.dinv, b, x, L.omega, tmp, rz_fin, c->d_st,
                 c->partials.p, c->d_counter, red_ptr(c));
       cgz_finish(c, rz_fin, 1);
     } else {
-      B2_LAUNCH(c, k_mg_sweep<false>, g, 256, L.n, L.pat->slice_ptr.p, L.pat->scols.p, L.A, L.dinv, b, x, c->mg_omega, tmp);
+      B2_LAUNCH(c, k_mg_sweep<false>, g, 256, L.n, L.pat->slice_ptr.p, L.pat->scols.p, L.A, L.dinv, b, x, L.omega, tmp);
     }
     std::swap(x, tmp);
   }
@@ -662,8 +698,10 @@ void mg_build_descriptors(b2_ctx* c) {
   for (int i = 0; i < nl; ++i) {
     MgLevel& M = c->mg[i];
     h[i] = {M.n, M.P.n_rows, M.pat.slice_ptr.p, M.pat.scols.p, M.A.p, M.dinv.p, M.x.p, M.b.p, M.tmp.p,
-            M.P.rowptr.p, M.P.cols.p, M.Pv.p, M.R.rowptr.p, M.R.cols.p, M.Rv.p};
-    if (M.n <= 8192 && c->mg_small_from == (1 << 30)) c->mg_small_from = i + 1;
+            M.P.rowptr.p, M.P.cols.p, M.Pv.p, M.R.rowptr.p, M.R.cols.p, M.Rv.p, M.omega};
+    // an algebraic hierarchy ends at its exactly solved level: the single-block sub-cycle must not smooth over it
+    const bool past_dense = !M.algebraic || c->mg_dense_level < 0 || i > c->mg_dense_level;
+    if (M.n <= 8192 && past_dense && c->mg_small_from == (1 << 30)) c->mg_small_from = i + 1;
   }
   if (nl - (c->mg_small_from - 1) > 15) c->mg_small_from = 1 << 30;  // shared pointer tables hold 16 levels
   c->mg_dev.alloc(nl);
@@ -699,6 +737,21 @@ void mg_build_dense(b2_ctx* c, int i) {
   c->mg_dense_level = i;
 }
 
+// the end of every new coarse level, however its operator L.A (SELL) was made: inverse diagonal, work vectors, the
+// exact solve if it is the first small level, and the fine-level work vectors with the first level
+void mg_level_finish(b2_ctx* c, MgLevel& L) {
+  L.dinv.alloc(L.n);
+  B2_LAUNCH(c, k_inv_diag, blocks_for(L.n, 256), 256, L.n, L.pat.slice_ptr.p, L.pat.diag_t.p, L.A.p, L.dinv.p);
+  for (auto* v : {&L.x, &L.b, &L.r, &L.tmp}) { v->alloc(L.n); v->zero(c->stream); }
+  if (c->mg_dense_level < 0 && L.n <= c->mg_dense_max) mg_build_dense(c, (int)c->mg.size() - 1);
+  if (c->mg.size() == 1) {
+    c->mg_x0.alloc(c->sp[B2_SPACE_Q].n_local()); c->mg_x0.zero(c->stream);
+    c->mg_t0.alloc(c->sp[B2_SPACE_Q].n_local()); c->mg_t0.zero(c->stream);
+  }
+}
+
+void amg_build(b2_ctx* c);
+
 // x_l <- V-cycle(b_l), zero initial guess.  Returns the buffer that holds the result.
 // first_done: x already holds omega D^-1 b; rz_fin >= 0 (level 0 only): fuse the PCG product r.z into the last post-sweep
 // -- *rz_done tells the caller whether that happened.
@@ -724,10 +777,10 @@ double* mg_vcycle(b2_ctx* c, int l, const double* b, double* x, double* tmp, boo
   MgView L;
   if (fine) {
     const CSR& qq = c->pat[B2_PAT_QQ];
-    L = {qq.n_rows, qq.n_cols, &qq, c->Ap.p, c->dinvAp.p};
+    L = {qq.n_rows, qq.n_cols, &qq, c->Ap.p, c->dinvAp.p, mg_level_omega(c, 0)};
   } else {
     MgLevel& M = c->mg[l - 1];
-    L = {M.n, M.n, &M.pat, M.A.p, M.dinv.p};
+    L = {M.n, M.n, &M.pat, M.A.p, M.dinv.p, mg_level_omega(c, l)};
   }
   const bool coarsest = (l == (int)c->mg.size());
   if (coarsest) {
@@ -743,7 +796,7 @@ double* mg_vcycle(b2_ctx* c, int l, const double* b, double* x, double* tmp, boo
   // a replicated level); partial sums of several slabs are added up first
   const bool partial = fine && c->nranks > 1;
   B2_LAUNCH(c, k_mg_restrict, blocks_for((int64_t)C.n * 8, 256), 256, C.n, C.R.rowptr.p, C.R.cols.p, C.Rv.p, tmp, C.dinv.p,
-            c->mg_omega, C.b.p, partial ? (double*)nullptr : C.x.p);
+            mg_level_omega(c, l + 1), C.b.p, partial ? (double*)nullptr : C.x.p);
   if (partial) {  // coarse levels are replicated: sum the partial restrictions of the slabs
     if (c->peer_on && c->pvs_ready) {
       B2_LAUNCH(c, k_peer_vecsum, std::min(PEER_GRID_MAX, blocks_for(C.n, 1024)), 256, c->pvs, C.b.p);
@@ -788,7 +841,8 @@ void pcg_mg_solve(b2_ctx* c, const double* b, double* x, int32_t* reason, int32_
     q0 = q;
   }
   // the first smoothing sweep of every V-cycle (x0 = omega D^-1 r) is written by the kernel that updates r
-  B2_LAUNCH(c, k_cgz_init_x0, g, 256, n, b, q0, x, r, c->dinvAp.p, c->mg_omega, c->mg_x0.p, c->d_st, c->partials.p, c->d_counter, red_ptr(c));
+  const double omega0 = mg_level_omega(c, 0);
+  B2_LAUNCH(c, k_cgz_init_x0, g, 256, n, b, q0, x, r, c->dinvAp.p, omega0, c->mg_x0.p, c->d_st, c->partials.p, c->d_counter, red_ptr(c));
   cgz_finish(c, FIN_CGZ_INIT, 2);
   // The device decides convergence; the host only has to stop enqueueing.  Iteration counts barely change
   // from one time step to the next, so nothing is polled (no pipeline drain) until one iteration short of
@@ -804,7 +858,7 @@ void pcg_mg_solve(b2_ctx* c, const double* b, double* x, int32_t* reason, int32_
     }
     B2_LAUNCH(c, k_cgz_p, g, 256, n, z, p, c->d_st);
     spmm(c, qq, c->Ap.p, 1, p, q, p, c->d_st, FIN_CG_PQ, 1, B2_SPACE_Q);
-    B2_LAUNCH(c, k_cgz_update_x0, g, 256, n, p, q, x, r, c->dinvAp.p, c->mg_omega, c->mg_x0.p, c->d_st, c->partials.p, c->d_counter, red_ptr(c));
+    B2_LAUNCH(c, k_cgz_update_x0, g, 256, n, p, q, x, r, c->dinvAp.p, omega0, c->mg_x0.p, c->d_st, c->partials.p, c->d_counter, red_ptr(c));
     cgz_finish(c, FIN_CGZ_UPDATE, 1);
   };
   // Iterations 1, 2, ... are identical streams of small dependent kernels (all scalars live in device memory):
@@ -1423,8 +1477,12 @@ void do_preassemble(b2_ctx* c, const double* body_force, int low_memory, int rot
               V.cell_dofs.p, vv.n_rows, vv.rowptr.p, vv.cols.p, vv.slice_ptr.p, c->M.p);                       // :373
     B2_LAUNCH(c, (k_assemble_square<D, DEG, B2_FORM_STIFF_V>), blocks_for(nc * E::NV, 128), 128, nc, c->x.p, c->cell_nodes.p,
               V.cell_dofs.p, vv.n_rows, vv.rowptr.p, vv.cols.p, vv.slice_ptr.p, c->Kst.p);                     // :375
-    B2_LAUNCH(c, (k_assemble_square<D, DEG, B2_FORM_STIFF_Q>), blocks_for(nc * E::NQ, 128), 128, nc, c->x.p, c->cell_nodes.p,
-              Q.cell_dofs.p, qq.n_rows, qq.rowptr.p, qq.cols.p, qq.slice_ptr.p, c->Ap.p);                      // :379
+    // :379 -- in a fixed order: the algebraic multigrid (b2_pressure_amg_build) is built from Ap, and the same mesh must give
+    // the same hierarchy on every run
+    assemble_in_fixed_order(c, nc * E::NQ * E::NQ, qq.slots, c->Ap.p, [&](unsigned* slot, double* val) {
+      B2_LAUNCH(c, (k_assemble_square<D, DEG, B2_FORM_STIFF_Q>), blocks_for(nc * E::NQ, 128), 128, nc, c->x.p, c->cell_nodes.p,
+                Q.cell_dofs.p, qq.n_rows, qq.rowptr.p, qq.cols.p, qq.slice_ptr.p, c->Ap.p, slot, val);
+    });
     if (c->rotational)
       B2_LAUNCH(c, (k_assemble_square<D, DEG, B2_FORM_MASS_Q>), blocks_for(nc * E::NQ, 128), 128, nc, c->x.p, c->cell_nodes.p,
                 Q.cell_dofs.p, qq.n_rows, qq.rowptr.p, qq.cols.p, qq.slice_ptr.p, c->MQ.p);                    // function.py:63-71
@@ -1851,9 +1909,6 @@ int b2_pressure_mg_add_level(b2_ctx* c, int64_t n_nodes, const double* x, int64_
     else
       B2_LAUNCH(c, (k_assemble_square<3, 1, B2_FORM_STIFF_Q>), blocks_for(n_cells * 4, 128), 128, n_cells, dx.p, dcells.p, dcells.p,
                 L.n, L.pat.rowptr.p, L.pat.cols.p, L.pat.slice_ptr.p, L.A.p);
-    L.dinv.alloc(L.n);
-    B2_LAUNCH(c, k_inv_diag, blocks_for(L.n, 256), 256, L.n, L.pat.slice_ptr.p, L.pat.diag_t.p, L.A.p, L.dinv.p);
-    for (auto* v : {&L.x, &L.b, &L.r, &L.tmp}) { v->alloc(L.n); v->zero(c->stream); }
     auto upload_csr = [&](CSR& m, DBuf<double>& vals, int rows, int cols, const int32_t* ip, const int32_t* ix, const double* vv) {
       int nnz = ip[rows];
       m.n_rows = rows; m.n_cols = cols; m.nnz = nnz;
@@ -1873,10 +1928,64 @@ int b2_pressure_mg_add_level(b2_ctx* c, int64_t n_nodes, const double* x, int64_
         if (R_indptr[r + 1] > R_indptr[r]) { c->mg_lo = std::min(c->mg_lo, r); c->mg_hi = std::max(c->mg_hi, r + 1); }
       if (c->mg_hi <= c->mg_lo) c->mg_lo = c->mg_hi = 0;
     }
-    if (c->mg_dense_level < 0 && L.n <= c->mg_dense_max) mg_build_dense(c, (int)c->mg.size() - 1);
-    if (c->mg.size() == 1) {
-      c->mg_x0.alloc(c->sp[B2_SPACE_Q].n_local()); c->mg_x0.zero(c->stream);
-      c->mg_t0.alloc(c->sp[B2_SPACE_Q].n_local()); c->mg_t0.zero(c->stream);
+    mg_level_finish(c, L);
+    B2_CUDA(cudaStreamSynchronize(c->stream));
+  });
+}
+
+int b2_pressure_amg_build(b2_ctx* c) {
+  return guarded(c, [&] {
+    B2_REQUIRE(c->preassembled, "b2_pressure_amg_build: call it after b2_preassemble");
+    B2_REQUIRE(c->mg.empty(), "b2_pressure_amg_build: the context already has a multigrid hierarchy");
+    B2_REQUIRE(c->nranks == 1, "b2_pressure_amg_build: the algebraic multigrid runs on one rank only");
+    B2_REQUIRE(!c->has_pbc, "b2_pressure_amg_build: the pressure has Dirichlet dofs (the coarse solve assumes the constant null space)");
+    amg_build(c);
+  });
+}
+
+int b2_pressure_mg_level_info(b2_ctx* c, int level, double* out) {
+  return guarded(c, [&] {
+    B2_REQUIRE(c->preassembled, "multigrid levels exist after b2_preassemble");
+    B2_REQUIRE(level >= 0 && level <= (int)c->mg.size(), "no such multigrid level");
+    if (level == 0) {
+      const CSR& qq = c->pat[B2_PAT_QQ];
+      const double v[7] = {(double)qq.n_rows, (double)qq.nnz, 0.0, c->mg_omega0 > 0.0 ? 1.0 : 0.0, 0.0, mg_level_omega(c, 0), c->mg_rho0};
+      std::memcpy(out, v, sizeof(v));
+      return;
+    }
+    const MgLevel& M = c->mg[level - 1];
+    const bool dense = level - 1 == c->mg_dense_level && c->mg_dense_on;
+    const double v[7] = {(double)M.n, (double)M.pat.nnz, (double)M.P.nnz, M.algebraic ? 1.0 : 0.0, dense ? 1.0 : 0.0,
+                         mg_level_omega(c, level), M.rho};
+    std::memcpy(out, v, sizeof(v));
+  });
+}
+
+int b2_pressure_mg_get_level(b2_ctx* c, int level, int what, int32_t* indptr, int32_t* indices, double* vals) {
+  return guarded(c, [&] {
+    B2_REQUIRE(level >= 1 && level <= (int)c->mg.size(), "no such coarse multigrid level");
+    B2_REQUIRE(what >= 0 && what <= 3, "what: 0 = A, 1 = P, 2 = R, 3 = aggregates");
+    MgLevel& M = c->mg[level - 1];
+    auto d2h = [&](void* dst, const void* src, size_t bytes) {
+      if (bytes) B2_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream));
+    };
+    if (what == 3) {
+      B2_REQUIRE(M.algebraic, "aggregates exist on algebraic levels only");
+      d2h(indices, M.agg.p, sizeof(int) * M.P.n_rows);
+    } else {
+      const CSR& m = what == 0 ? M.pat : (what == 1 ? M.P : M.R);
+      d2h(indptr, m.rowptr.p, sizeof(int) * (m.n_rows + 1));
+      d2h(indices, m.cols.p, sizeof(int) * m.nnz);
+      if (what == 0) {
+        DBuf<double> v;
+        v.alloc(m.nnz);
+        B2_LAUNCH(c, k_sell_convert, blocks_for(m.n_rows, 256), 256, m.n_rows, m.rowptr.p, m.slice_ptr.p, 0, M.A.p, v.p,
+                  (const double*)nullptr);
+        d2h(vals, v.p, sizeof(double) * m.nnz);
+        B2_CUDA(cudaStreamSynchronize(c->stream));
+      } else {
+        d2h(vals, (what == 1 ? M.Pv : M.Rv).p, sizeof(double) * m.nnz);
+      }
     }
     B2_CUDA(cudaStreamSynchronize(c->stream));
   });
@@ -2089,6 +2198,219 @@ void csr_values(b2_ctx* c, int mat, int comp, DBuf<double>& out, const CSR** pat
     B2_LAUNCH(c, k_extract, pgrid(c, pat->nnz), 256, pat->nnz, stride, comp, v->p, out.p);
   }
   *pat_out = pat;
+}
+
+// ---- smoothed-aggregation AMG set-up (amg.cuh) ----------------------------------------------------
+template <typename T>
+T read_scalar(b2_ctx* c, const T* d) {
+  T h{};
+  B2_CUDA(cudaMemcpyAsync(&h, d, sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+  B2_CUDA(cudaStreamSynchronize(c->stream));
+  return h;
+}
+
+template <typename T>
+void exclusive_sum(b2_ctx* c, const T* in, T* out, int64_t n) {
+  size_t bytes = 0;
+  B2_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, n, c->stream));
+  DBuf<char> tmp;
+  tmp.alloc((int64_t)bytes);
+  B2_CUDA(cub::DeviceScan::ExclusiveSum(tmp.p, bytes, in, out, n, c->stream));
+}
+
+// n pairs (row << 32 | col, value) in a deterministic generation order -> CSR with sorted columns; the values of equal
+// keys are summed sequentially in that order (stable radix sort, one thread per run), so the result is the same bit
+// for bit on every run.  The pair buffers are consumed.
+void amg_pairs_to_csr(b2_ctx* c, DBuf<unsigned long long>& keys, DBuf<double>& vals, int64_t n, int n_rows, int n_cols,
+                      CSR& out, DBuf<double>& out_vals) {
+  B2_REQUIRE(n < (1ll << 31), "algebraic multigrid: sparse product too large for int32 indices");
+  DBuf<unsigned long long> k2;
+  DBuf<double> v2;
+  k2.alloc(n);
+  v2.alloc(n);
+  int row_bits = 1;
+  while ((1ll << row_bits) <= (int64_t)n_rows) ++row_bits;
+  cub::DoubleBuffer<unsigned long long> kb(keys.p, k2.p);
+  cub::DoubleBuffer<double> vb(vals.p, v2.p);
+  size_t bytes = 0;
+  B2_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, kb, vb, n, 0, 32 + row_bits, c->stream));
+  DBuf<char> tmp;
+  tmp.alloc((int64_t)bytes);
+  B2_CUDA(cub::DeviceRadixSort::SortPairs(tmp.p, bytes, kb, vb, n, 0, 32 + row_bits, c->stream));
+  DBuf<int> head, run;
+  head.alloc(n + 1);
+  run.alloc(n + 1);
+  B2_LAUNCH(c, k_amg_heads, blocks_for(n + 1, 256), 256, n, kb.Current(), head.p);
+  exclusive_sum(c, head.p, run.p, n + 1);
+  const int n_unique = read_scalar(c, run.p + n);
+  DBuf<unsigned long long> uk;
+  uk.alloc(n_unique);
+  out_vals.alloc(n_unique);
+  B2_LAUNCH(c, k_amg_reduce_runs, blocks_for(n, 256), 256, n, kb.Current(), vb.Current(), head.p, run.p, uk.p, out_vals.p);
+  out.n_rows = n_rows;
+  out.n_cols = n_cols;
+  out.nnz = n_unique;
+  out.rowptr.alloc(n_rows + 1);
+  out.cols.alloc(n_unique);
+  B2_LAUNCH(c, k_keys_to_csr, blocks_for((int64_t)n_unique + 1, 256), 256, (int64_t)n_unique, uk.p, n_rows, out.rowptr.p, out.cols.p);
+  B2_CUDA(cudaStreamSynchronize(c->stream));
+}
+
+// C = A B (CSR, sorted columns) by expansion into one pair per product, sort and reduce
+void amg_spgemm(b2_ctx* c, const CSR& A, const double* va, const CSR& B, const double* vb, CSR& C, DBuf<double>& vc) {
+  const int64_t nnz = A.nnz;
+  DBuf<int> rows;
+  DBuf<int64_t> cnt, off;
+  rows.alloc(nnz);
+  cnt.alloc(nnz + 1);
+  off.alloc(nnz + 1);
+  cnt.zero(c->stream);
+  B2_LAUNCH(c, k_amg_entry_rows, blocks_for(A.n_rows, 256), 256, A.n_rows, A.rowptr.p, rows.p);
+  B2_LAUNCH(c, k_amg_product_counts, blocks_for(nnz, 256), 256, nnz, A.cols.p, B.rowptr.p, cnt.p);
+  exclusive_sum(c, cnt.p, off.p, nnz + 1);
+  const int64_t total = read_scalar(c, off.p + nnz);
+  DBuf<unsigned long long> keys;
+  DBuf<double> vals;
+  keys.alloc(total);
+  vals.alloc(total);
+  B2_LAUNCH(c, k_amg_expand, blocks_for(nnz, 256), 256, nnz, rows.p, A.cols.p, va, B.rowptr.p, B.cols.p, vb, off.p, keys.p, vals.p);
+  amg_pairs_to_csr(c, keys, vals, total, A.n_rows, B.n_cols, C, vc);
+}
+
+void amg_transpose(b2_ctx* c, const CSR& A, const double* va, CSR& T, DBuf<double>& vt) {
+  DBuf<int> rows;
+  rows.alloc(A.nnz);
+  DBuf<unsigned long long> keys;
+  DBuf<double> vals;
+  keys.alloc(A.nnz);
+  vals.alloc(A.nnz);
+  B2_LAUNCH(c, k_amg_entry_rows, blocks_for(A.n_rows, 256), 256, A.n_rows, A.rowptr.p, rows.p);
+  B2_LAUNCH(c, k_amg_transpose_keys, blocks_for(A.nnz, 256), 256, A.nnz, rows.p, A.cols.p, va, keys.p, vals.p);
+  amg_pairs_to_csr(c, keys, vals, A.nnz, A.n_cols, A.n_rows, T, vt);
+}
+
+// rho(D^-1 A) from 20 power iterations (normalised on the device, no host round trip; sums in a fixed order), reported as the Rayleigh
+// quotient x^T A x / x^T D x of the last iterate: D^-1 A is self-adjoint in the D inner product, so the estimate is
+// a lower bound whose error is quadratic in the iterate's
+double amg_spectral_radius(b2_ctx* c, const CSR& A, const double* va, const double* dinv) {
+  const int n = A.n_rows;
+  DBuf<double> x, y, y2, sums;
+  x.alloc(n);
+  y.alloc(n);
+  y2.alloc(n);
+  sums.alloc(3);
+  B2_LAUNCH(c, k_amg_seed, blocks_for(n, 256), 256, n, x.p);
+  for (int k = 0; k < 20; ++k) {
+    B2_LAUNCH(c, k_amg_power, blocks_for(n, 256), 256, n, A.rowptr.p, A.cols.p, va, dinv, x.p, k == 0 ? nullptr : sums.p,
+              y.p, y2.p);
+    B2_LAUNCH(c, k_amg_sum, 1, 1024, n, y2.p, sums.p);
+    std::swap(x.p, y.p);
+  }
+  B2_LAUNCH(c, k_amg_rayleigh, blocks_for(n, 256), 256, n, A.rowptr.p, A.cols.p, va, dinv, x.p, y.p, y2.p);
+  B2_LAUNCH(c, k_amg_sum, 1, 1024, n, y.p, sums.p + 1);
+  B2_LAUNCH(c, k_amg_sum, 1, 1024, n, y2.p, sums.p + 2);
+  double h[3];
+  B2_CUDA(cudaMemcpyAsync(h, sums.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+  B2_CUDA(cudaStreamSynchronize(c->stream));
+  B2_REQUIRE(h[2] > 0.0 && h[1] > 0.0, "algebraic multigrid: spectral radius estimate failed");
+  return h[1] / h[2];
+}
+
+// MIS(2) aggregation of the strength graph of A; returns the number of aggregates
+int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, DBuf<int>& agg) {
+  const int n = A.n_rows;
+  B2_REQUIRE(n < (1 << 30), "algebraic multigrid: at most 2^30 dofs");
+  const int g = blocks_for(n, 256);
+  DBuf<int> state, cnt, flag, id, agg1;
+  DBuf<unsigned long long> t0, m1, m2;
+  state.alloc(n);
+  cnt.alloc(1);
+  t0.alloc(n);
+  m1.alloc(n);
+  m2.alloc(n);
+  B2_LAUNCH(c, k_amg_init, g, 256, n, state.p);
+  for (int round = 0;; ++round) {
+    B2_REQUIRE(round <= n, "algebraic multigrid: MIS(2) did not terminate");
+    cnt.zero(c->stream);
+    B2_LAUNCH(c, k_amg_tuples, g, 256, n, state.p, t0.p);
+    B2_LAUNCH(c, k_amg_max_hop, g, 256, n, A.rowptr.p, A.cols.p, va, t0.p, m1.p);
+    B2_LAUNCH(c, k_amg_max_hop, g, 256, n, A.rowptr.p, A.cols.p, va, m1.p, m2.p);
+    B2_LAUNCH(c, k_amg_mis_update, g, 256, n, state.p, t0.p, m2.p, cnt.p);
+    if (read_scalar(c, cnt.p) == 0) break;
+  }
+  flag.alloc(n + 1);
+  id.alloc(n + 1);
+  flag.zero(c->stream);
+  B2_LAUNCH(c, k_amg_root_flags, g, 256, n, state.p, flag.p);
+  exclusive_sum(c, flag.p, id.p, (int64_t)n + 1);
+  const int nc = read_scalar(c, id.p + n);
+  agg1.alloc(n);
+  agg.alloc(n);
+  cnt.zero(c->stream);
+  B2_LAUNCH(c, k_amg_pass1, g, 256, n, A.rowptr.p, A.cols.p, va, state.p, id.p, agg1.p);
+  B2_LAUNCH(c, k_amg_pass2, g, 256, n, A.rowptr.p, A.cols.p, va, agg1.p, agg.p, cnt.p);
+  B2_REQUIRE(read_scalar(c, cnt.p) == 0, "algebraic multigrid: a node was left without an aggregate");
+  return nc;
+}
+
+// Smoothed-aggregation hierarchy from the assembled Ap, coarsened until a level is small enough for the exact dense
+// solve, the coarsening ratio drops below 2, or 15 coarse levels (the single-block sub-cycle's tables hold 16).
+void amg_build(b2_ctx* c) {
+  c->cfg_version++;
+  const CSR& qq = c->pat[B2_PAT_QQ];
+  DBuf<double> vals;  // values of the current operator in CSR order
+  const CSR* pat = nullptr;
+  csr_values(c, B2_MAT_AP, 0, vals, &pat);
+  const CSR* A = &qq;
+  const double* dinv = c->dinvAp.p;
+  c->mg_rho0 = amg_spectral_radius(c, *A, vals.p, dinv);
+  c->mg_omega0 = 4.0 / (3.0 * c->mg_rho0);
+  double omega_p = c->mg_omega0;
+  c->mg.reserve(16);  // A points into c->mg below
+  while (c->mg.size() < 15) {
+    const int n = A->n_rows;
+    DBuf<int> agg;
+    const int nc = amg_aggregate(c, *A, vals.p, agg);
+    if (nc >= n) break;  // no coarsening at all
+    // P = (I - omega_P D^-1 A) T
+    CSR T;
+    DBuf<double> tv, sv;
+    T.n_rows = n;
+    T.n_cols = nc;
+    T.nnz = n;
+    T.rowptr.alloc(n + 1);
+    T.cols.alloc(n);
+    tv.alloc(n);
+    B2_LAUNCH(c, k_amg_tentative, blocks_for(n + 1, 256), 256, n, agg.p, T.rowptr.p, T.cols.p, tv.p);
+    sv.alloc(A->nnz);
+    B2_LAUNCH(c, k_amg_smoother, blocks_for(n, 256), 256, n, A->rowptr.p, A->cols.p, vals.p, dinv, omega_p, sv.p);
+    c->mg.emplace_back();
+    MgLevel& L = c->mg.back();
+    L.algebraic = true;
+    L.n = nc;
+    L.agg = std::move(agg);
+    amg_spgemm(c, *A, sv.p, T, tv.p, L.P, L.Pv);
+    amg_transpose(c, L.P, L.Pv.p, L.R, L.Rv);
+    // A_c = R (A P)
+    CSR AP;
+    DBuf<double> apv, acv;
+    amg_spgemm(c, *A, vals.p, L.P, L.Pv.p, AP, apv);
+    amg_spgemm(c, L.R, L.Rv.p, AP, apv.p, L.pat, acv);
+    build_sell(c, L.pat);
+    L.A.alloc(L.pat.slots);
+    L.A.zero(c->stream);
+    B2_LAUNCH(c, k_sell_convert, blocks_for(nc, 256), 256, nc, L.pat.rowptr.p, L.pat.slice_ptr.p, 1, acv.p, L.A.p,
+              (const double*)nullptr);
+    mg_level_finish(c, L);
+    L.rho = amg_spectral_radius(c, L.pat, acv.p, L.dinv.p);
+    L.omega = 4.0 / (3.0 * L.rho);
+    omega_p = L.omega;
+    vals = std::move(acv);
+    A = &L.pat;
+    dinv = L.dinv.p;
+    if (nc <= c->mg_dense_max || 2 * (int64_t)nc > n) break;
+  }
+  B2_CUDA(cudaStreamSynchronize(c->stream));
 }
 
 }  // namespace
@@ -2446,6 +2768,7 @@ int b2_ksp_solve(b2_ctx* c, int solver, int mat, const double* b, double* x, int
     } else {
       krylov_solve(c, solver, *pat, v->p, dinv.p, sp, 1, db.p, dx.p, reason, &its, c->wproj);
     }
+    if (solver == B2_SOLVER_PRESSURE) c->stats.its_pressure = its;
     halo_forward(c, sp, dx.p, 1);  // x.x.scatter_forward(), ksp.py:77
     B2_CUDA(cudaMemcpyAsync(x, dx.p, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
     B2_CUDA(cudaStreamSynchronize(c->stream));

@@ -105,12 +105,15 @@ __device__ __forceinline__ size_t sell_slot_of(const int* __restrict__ slice_ptr
 // ---- one-off (pre)assembly kernels: one thread per (cell, local row) -----------------------
 enum { B2_FORM_MASS_V = 0, B2_FORM_STIFF_V = 1, B2_FORM_MASS_Q = 2, B2_FORM_STIFF_Q = 3 };
 
+// pair_slot != nullptr: instead of adding into vals, entry (cell, i, j) writes its SELL slot and value to
+// pair_slot/pair_val[(cell * ND + i) * ND + j] (sum_slot_pairs adds them up in a fixed order)
 template <int D, int DEG, int FORM>
 __global__ void k_assemble_square(int64_t n_cells, const double* __restrict__ x,
                                   const int* __restrict__ cell_nodes, const int* __restrict__ cdofs,
                                   int n_rows_owned, const int* __restrict__ rowptr,
                                   const int* __restrict__ cols, const int* __restrict__ slice_ptr,
-                                  double* __restrict__ vals) {
+                                  double* __restrict__ vals, unsigned* __restrict__ pair_slot = nullptr,
+                                  double* __restrict__ pair_val = nullptr) {
   using E = El<D, DEG>;
   constexpr bool onV = (FORM == B2_FORM_MASS_V || FORM == B2_FORM_STIFF_V);
   constexpr int ND = onV ? E::NV : E::NQ;
@@ -152,8 +155,24 @@ __global__ void k_assemble_square(int64_t n_cells, const double* __restrict__ x,
         for (int b = 0; b < D; ++b) v += G[a][b] * E::SQ(a, b, i, j);
     }
     int pos = csr_find(cols, lo, hi, dofs[j]);
-    atomicAdd(vals + sell_slot_of(slice_ptr, row, pos - lo), v);
+    if (pair_slot != nullptr) {
+      pair_slot[t * ND + j] = (unsigned)sell_slot_of(slice_ptr, row, pos - lo);
+      pair_val[t * ND + j] = v;
+    } else {
+      atomicAdd(vals + sell_slot_of(slice_ptr, row, pos - lo), v);
+    }
   }
+}
+
+// after a stable sort of the (slot, value) pairs by slot: the first pair of every slot adds up its run sequentially
+// and stores the sum; slot 0xffffffff marks pairs nobody wrote (rows owned by another rank)
+__global__ void k_sum_slot_runs(int64_t n, const unsigned* __restrict__ slot, const double* __restrict__ v,
+                                double* __restrict__ vals) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n || slot[t] == 0xffffffffu || (t > 0 && slot[t] == slot[t - 1])) return;
+  double acc = v[t];
+  for (int64_t u = t + 1; u < n && slot[u] == slot[t]; ++u) acc += v[u];
+  vals[slot[t]] = acc;
 }
 
 // P_c[j,q] = int psi_q d_c phi_j and G_c[j,q] = int d_c psi_q phi_j on the V x Q pattern; the D

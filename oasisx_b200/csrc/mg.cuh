@@ -94,6 +94,7 @@ struct MgDev {
   const double* Pval;  // rows: dofs of the finer level, cols: this level
   const int *Rptr, *Rcol;
   const double* Rval;  // rows: this level, cols: dofs of the finer level
+  double omega;        // damping of an algebraic level; 0: the kernel's omega argument (geometric levels)
 };
 
 __device__ __forceinline__ double mg_row_dot(const MgDev& L, int row, const double* x) {
@@ -134,7 +135,7 @@ k_mg_small_cycle(const MgDev* __restrict__ lv, int l0, int l_last, int pre, int 
   // down
   for (int l = l0; l <= l_last; ++l) {
     const MgDev L = lv[l];
-    double* x = mg_block_sweeps(L, L.x, L.tmp, l == l_last ? coarse : pre, true, omega);
+    double* x = mg_block_sweeps(L, L.x, L.tmp, l == l_last ? coarse : pre, true, L.omega > 0.0 ? L.omega : omega);
     double* tmp = (x == L.x) ? L.tmp : L.x;
     if (threadIdx.x == 0) { xs[l - l0] = x; ts[l - l0] = tmp; }
     if (l < l_last) {
@@ -162,7 +163,7 @@ k_mg_small_cycle(const MgDev* __restrict__ lv, int l0, int l_last, int pre, int 
       x[r] = acc;
     }
     __syncthreads();
-    x = mg_block_sweeps(L, x, tmp, post, false, omega);
+    x = mg_block_sweeps(L, x, tmp, post, false, L.omega > 0.0 ? L.omega : omega);
     if (threadIdx.x == 0) xs[l - l0] = x;
     __syncthreads();
   }

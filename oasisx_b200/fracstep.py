@@ -238,9 +238,12 @@ class FractionalStep_AB_CN:
             # equivalent is the null-space-projected CG run to the "exact" tolerance
             self._solver_p.updateOptions({"ksp_type": "preonly", "pc_type": "lu"})
 
-        # optional geometric multigrid for the pressure ("pc_type": "mg"): hierarchy from the provider
+        # optional multigrid for the pressure: "mg" takes the geometric hierarchy of a provider box; "gamg" / "hypre"
+        # take it too where it exists and otherwise, on one rank, the algebraic hierarchy built from Ap
         self._mg_levels = 0
-        if (solver_options.get("pressure") or {}).get("pc_type") in ("mg", "gamg", "hypre") and not self._bcs_p:
+        self._mg_kind = None  # "geometric" | "algebraic" | None
+        pc_p = (solver_options.get("pressure") or {}).get("pc_type")
+        if pc_p in ("mg", "gamg", "hypre") and not self._bcs_p:
             from . import multigrid as _mg
 
             dof_nodes = getattr(self._Q, "_dof_nodes", None)
@@ -249,9 +252,13 @@ class FractionalStep_AB_CN:
                     mesh.geometry.dofmap, self._Q.dofmap.list)
                 dof_nodes = np.empty(self._Q.num_dofs, dtype=np.int64)
                 dof_nodes[cell_dofs.ravel()] = cell_nodes.ravel()
-            self._mg_levels = _mg.attach_pressure_multigrid(
-                ctx, mesh, dof_nodes, self._nQ_owned, **(options.get("multigrid") or {})
-            )
+            mg_config = options.get("multigrid") or {}
+            self._mg_levels = _mg.attach_pressure_multigrid(ctx, mesh, dof_nodes, self._nQ_owned, **mg_config)
+            if self._mg_levels:
+                self._mg_kind = "geometric"
+            elif pc_p != "mg" and self._nranks == 1:
+                self._mg_levels = _mg.attach_pressure_amg(ctx, **mg_config)
+                self._mg_kind = "algebraic" if self._mg_levels else None
             if self._mg_levels == 0:
                 logger.warning("pc_type=mg requested but the mesh carries no nested hierarchy: using Jacobi")
             elif self._nranks > 1 and ctx.peer_enabled():

@@ -9,12 +9,16 @@ on the coarse mesh by the library (``b2_pressure_mg_add_level``).
 
 For meshes that come from DOLFINx the same C entry point accepts any nested hierarchy (e.g. from
 ``dolfinx.mesh.refine`` [ext]) as long as P/R are supplied.
+
+Meshes without such a hierarchy get a smoothed-aggregation algebraic multigrid built on the device from the assembled
+pressure matrix instead (:func:`attach_pressure_amg`); the V-cycle is the same.
 """
 from __future__ import annotations
 
 import numpy as np
 import scipy.sparse as sp
 
+from . import _lib
 from . import fem as _fem
 from . import mesh as _mesh
 
@@ -106,3 +110,20 @@ def attach_pressure_multigrid(ctx, msh, dof_nodes: np.ndarray, n_owned: int, **c
     if config:
         ctx.pressure_mg_configure(**config)
     return len(levels)
+
+
+def attach_pressure_amg(ctx, **config) -> int:
+    """Build the smoothed-aggregation hierarchy of the assembled pressure matrix on the device
+    (``b2_pressure_amg_build``: one rank, no pressure Dirichlet dofs) and apply `config` as
+    :func:`attach_pressure_multigrid` does (its ``omega`` only damps geometric levels).  Returns the number of coarse
+    levels."""
+    ctx.pressure_amg_build()
+    if config:
+        ctx.pressure_mg_configure(**config)
+    n = 0
+    while True:  # level_info fails past the coarsest level
+        try:
+            ctx.pressure_mg_level_info(n + 1)
+        except _lib.B200Error:
+            return n
+        n += 1
