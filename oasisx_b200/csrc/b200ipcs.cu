@@ -29,8 +29,7 @@ struct CSR {
   DBuf<int> rowptr, cols;
   int n_rows = 0, n_cols = 0;
   int64_t nnz = 0;
-  int lpr = 8;  // lanes per row used by the rectangular CSR kernels on this pattern
-  // SELL-32 layout of the same pattern (square operators only; see linalg.cuh)
+  // SELL-32 layout of the same pattern, where build_sell made one (every operator pattern but Q x V; see linalg.cuh)
   DBuf<int> slice_ptr, scols, diag_t, order;  // order: optional tile-major slice schedule
   int64_t slots = 0;
   bool has_sell() const { return slice_ptr.p != nullptr; }
@@ -205,9 +204,8 @@ struct b2_ctx {
   unsigned long long* h_peer_err = nullptr;  // pinned copy of the arena's error word
   bool patterns_built = false, preassembled = false;
   bool low_memory = false, rotational = false;
-  // matrices (values in pattern order)
+  // matrices: values in the SELL slots of their pattern, P and G component-major; D in CSR order, [nnz][gdim]
   DBuf<double> M, Kst, A, Ap, MQ, P, G, D;
-  DBuf<double> Psell, Gsell;  // P, G once more in sliced-ELL slots, component-major (the form the step multiplies with)
   DBuf<double> dinvA, dinvM, dinvAp, dinvMQ, onesV, onesQ;
   // boundary conditions
   DBuf<int> bc_dofs[B2_MAXK];
@@ -374,12 +372,10 @@ void build_pattern_raw(b2_ctx* c, int64_t n_cells, const int* rdofs, int nr, con
   out.cols.alloc(nnz);
   B2_CUDA(cudaMemcpyAsync(out.cols.p, cols_tmp.p, sizeof(int) * (size_t)nnz, cudaMemcpyDeviceToDevice, c->stream));
   B2_CUDA(cudaStreamSynchronize(c->stream));
-  double avg = n_rows ? (double)nnz / n_rows : 0.0;
-  out.lpr = avg >= 48 ? 16 : (avg >= 20 ? 8 : 4);
 }
 
-// SELL-32 companion of a square CSR pattern: slice offsets (in slots), padded column indices,
-// position of the diagonal in each row.
+// SELL-32 companion of a CSR pattern: slice offsets (in slots), padded column indices, position of the
+// diagonal in each row (-1 where the row has none).
 void build_sell(b2_ctx* c, CSR& pat) {
   const int n_rows = pat.n_rows;
   const int n_slices = (n_rows + 31) / 32;
@@ -1110,20 +1106,26 @@ void stage_assemble_first(b2_ctx* c, double dt, double nu) {
   c->fresh_step = true;
 }
 
-template <int K>
+// out_k = add_k + scale * Op_k xq for every direction k, Op = P or G (vals = c->P.p or c->G.p)
 void rect_vq(b2_ctx* c, const double* vals, const double* xq, const double* add, double scale, double* out) {
   const CSR& vq = c->pat[B2_PAT_VQ];
   const int ld = (int)c->sp[B2_SPACE_V].n_local();
-  const double* sell = vals == c->P.p ? c->Psell.p : (vals == c->G.p ? c->Gsell.p : nullptr);
-  if (sell != nullptr && vq.has_sell()) {
-    B2_LAUNCH(c, k_rect_vq_sell<K>, blocks_for(vq.n_rows, 256), 256, vq.n_rows, vq.slice_ptr.p, vq.scols.p, sell, (int64_t)vq.slots, xq,
-              add, ld, scale, out);
-    return;
-  }
-  if (vq.lpr >= 8)
-    B2_LAUNCH(c, (k_rect_vq<K, 8>), blocks_for((int64_t)vq.n_rows * 8, 256), 256, vq.n_rows, vq.rowptr.p, vq.cols.p, vals, xq, add, ld, scale, out);
+  const int grid = blocks_for(vq.n_rows, 256);
+  if (c->gdim == 2)
+    B2_LAUNCH(c, k_rect_vq_sell<2>, grid, 256, vq.n_rows, vq.slice_ptr.p, vq.scols.p, vals, (int64_t)vq.slots, xq, add, ld, scale, out);
   else
-    B2_LAUNCH(c, (k_rect_vq<K, 4>), blocks_for((int64_t)vq.n_rows * 4, 256), 256, vq.n_rows, vq.rowptr.p, vq.cols.p, vals, xq, add, ld, scale, out);
+    B2_LAUNCH(c, k_rect_vq_sell<3>, grid, 256, vq.n_rows, vq.slice_ptr.p, vq.scols.p, vals, (int64_t)vq.slots, xq, add, ld, scale, out);
+}
+
+// out = scale * sum_k D_k xv_k, rows flagged in zero_row (if given) set to 0
+void rect_qv(b2_ctx* c, const double* xv, double scale, const uint8_t* zero_row, double* out) {
+  const CSR& qv = c->pat[B2_PAT_QV];
+  const int ld = (int)c->sp[B2_SPACE_V].n_local();
+  const int grid = blocks_for((int64_t)qv.n_rows * 16, 256);
+  if (c->gdim == 2)
+    B2_LAUNCH(c, (k_rect_qv<2, 16>), grid, 256, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p, xv, ld, scale, zero_row, out);
+  else
+    B2_LAUNCH(c, (k_rect_qv<3, 16>), grid, 256, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p, xv, ld, scale, zero_row, out);
 }
 
 // matrix-free element vectors of the low-memory strategy (elem.cuh: k_lowmem_vector)
@@ -1159,8 +1161,7 @@ void stage_tentative_assemble(b2_ctx* c) {
     lowmem_vector(c, 0, ps, 1.0, c->vec(B2_VEC_RHS1));
     return;
   }
-  if (c->gdim == 2) rect_vq<2>(c, c->P.p, ps, c->vec(B2_VEC_BFIRST), 1.0, c->vec(B2_VEC_RHS1));
-  else rect_vq<3>(c, c->P.p, ps, c->vec(B2_VEC_BFIRST), 1.0, c->vec(B2_VEC_RHS1));
+  rect_vq(c, c->P.p, ps, c->vec(B2_VEC_BFIRST), 1.0, c->vec(B2_VEC_RHS1));
 }
 
 void apply_velocity_bcs(b2_ctx* c, double* v) {
@@ -1253,7 +1254,6 @@ void stage_tentative_solve(b2_ctx* c, double* diff, int32_t* reasons, bool defer
 
 void stage_pressure_assemble(b2_ctx* c, double dt) {
   require_ready(c);
-  const CSR& qv = c->pat[B2_PAT_QV];
   double* u = c->vec(B2_VEC_U);
   halo_forward(c, B2_SPACE_V, u, c->gdim);
   const uint8_t* zr = c->has_pbc ? c->is_bc_q.p : nullptr;
@@ -1264,12 +1264,7 @@ void stage_pressure_assemble(b2_ctx* c, double dt) {
     if (zr) B2_LAUNCH(c, k_zero_rows_q, blocks_for(Q.n_owned, 256), 256, Q.n_owned, zr, c->vec(B2_VEC_B2));
     return;
   }
-  const int grid = blocks_for((int64_t)qv.n_rows * 16, 256);
-  const int ld = (int)c->sp[B2_SPACE_V].n_local();
-  if (c->gdim == 2)
-    B2_LAUNCH(c, (k_rect_qv<2, 16>), grid, 256, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p, u, ld, -1.0 / dt, zr, c->vec(B2_VEC_B2));
-  else
-    B2_LAUNCH(c, (k_rect_qv<3, 16>), grid, 256, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p, u, ld, -1.0 / dt, zr, c->vec(B2_VEC_B2));
+  rect_qv(c, u, -1.0 / dt, zr, c->vec(B2_VEC_B2));
 }
 
 void stage_pressure_solve(b2_ctx* c, double nu, int32_t* reason) {
@@ -1308,21 +1303,17 @@ void stage_pressure_solve(b2_ctx* c, double nu, int32_t* reason) {
   if (c->rotational) {
     // ps = Proj_Q(p + dp - xi nu div u): MQ ps = MQ (p + dp) - 0.5 nu sum_i D_i u_i   (:238-247,593-602)
     const CSR& qq = c->pat[B2_PAT_QQ];
-    const CSR& qv = c->pat[B2_PAT_QV];
     double *t0 = c->wq[3].p, *rhs = c->vec(B2_VEC_B2);
     B2_LAUNCH(c, k_lincomb2, pgrid(c, n), 256, n, 1.0, p, 1.0, dp, t0);
     halo_forward(c, B2_SPACE_Q, t0, 1);
     double* u = c->vec(B2_VEC_U);
-    const int grid = blocks_for((int64_t)qv.n_rows * 16, 256);
     // rhs <- -0.5 nu sum_i D_i u_i (reusing b2 as scratch: it is rebuilt by the next pressure_assemble)
-    const int ldv = (int)c->sp[B2_SPACE_V].n_local();
     if (c->low_memory) {
       B2_CUDA(cudaMemsetAsync(rhs, 0, sizeof(double) * Q.n_local(), c->stream));
       lowmem_vector(c, 2, u, -0.5 * nu, rhs);
-    } else if (c->gdim == 2)
-      B2_LAUNCH(c, (k_rect_qv<2, 16>), grid, 256, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p, u, ldv, -0.5 * nu, (const uint8_t*)nullptr, rhs);
-    else
-      B2_LAUNCH(c, (k_rect_qv<3, 16>), grid, 256, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p, u, ldv, -0.5 * nu, (const uint8_t*)nullptr, rhs);
+    } else {
+      rect_qv(c, u, -0.5 * nu, nullptr, rhs);
+    }
     double* mq = c->wq[2].p;  // q work vector is free between solves
     spmm(c, qq, c->MQ.p, 1, t0, mq);
     B2_LAUNCH(c, k_lincomb2, pgrid(c, n), 256, n, 1.0, mq, 1.0, rhs, rhs);
@@ -1341,8 +1332,7 @@ void stage_velocity_update(b2_ctx* c, double dt, int32_t* reasons) {
   spmm(c, c->pat[B2_PAT_VV], c->M.p, K, u, b3, nullptr, nullptr, FIN_NONE, 0, B2_SPACE_V);  // :638
   halo_forward(c, B2_SPACE_Q, dp, 1);
   if (c->low_memory) lowmem_vector(c, 1, dp, -dt, b3);  // :617-622: b3 -= dt int d(dp)/dx_i v
-  else if (K == 2) rect_vq<2>(c, c->G.p, dp, b3, -dt, b3);  // :642-645
-  else rect_vq<3>(c, c->G.p, dp, b3, -dt, b3);
+  else rect_vq(c, c->G.p, dp, b3, -dt, b3);  // :642-645
   int32_t its[B2_MAXK] = {0, 0, 0};
   const bool extrap = c->ksp[B2_SOLVER_SCALAR].extrapolate_guess;
   const int64_t nl = c->sp[B2_SPACE_V].n_local() * K;
@@ -1456,8 +1446,8 @@ void do_preassemble(b2_ctx* c, const double* body_force, int low_memory, int rot
   c->A.alloc(vv.slots); c->A.zero(c->stream);
   c->Ap.alloc(qq.slots); c->Ap.zero(c->stream);
   if (!c->low_memory) {  // the 3d rectangular operator families exist only in the matrix-vector strategy (:392-404)
-    c->P.alloc(vq.nnz * K); c->P.zero(c->stream);
-    c->G.alloc(vq.nnz * K); c->G.zero(c->stream);
+    c->P.alloc(vq.slots * K); c->P.zero(c->stream);
+    c->G.alloc(vq.slots * K); c->G.zero(c->stream);
     c->D.alloc(qv.nnz * K); c->D.zero(c->stream);
   }
   if (c->rotational) { c->MQ.alloc(qq.slots); c->MQ.zero(c->stream); }
@@ -1488,15 +1478,9 @@ void do_preassemble(b2_ctx* c, const double* body_force, int low_memory, int rot
                 Q.cell_dofs.p, qq.n_rows, qq.rowptr.p, qq.cols.p, qq.slice_ptr.p, c->MQ.p);                    // function.py:63-71
     if (!c->low_memory) {
       B2_LAUNCH(c, (k_assemble_PG<D, DEG>), blocks_for(nc * E::NV, 128), 128, nc, c->x.p, c->cell_nodes.p, V.cell_dofs.p,
-                Q.cell_dofs.p, vq.n_rows, vq.rowptr.p, vq.cols.p, c->P.p, c->G.p);              // :395,399
+                Q.cell_dofs.p, vq.n_rows, vq.rowptr.p, vq.cols.p, vq.slice_ptr.p, (int64_t)vq.slots, c->P.p, c->G.p);  // :395,399
       B2_LAUNCH(c, (k_assemble_D<D, DEG>), blocks_for(nc * E::NQ, 128), 128, nc, c->x.p, c->cell_nodes.p, V.cell_dofs.p,
                 Q.cell_dofs.p, qv.n_rows, qv.rowptr.p, qv.cols.p, c->D.p);                      // :403
-      if (vq.has_sell()) {
-        c->Psell.alloc(vq.slots * D); c->Psell.zero(c->stream);
-        c->Gsell.alloc(vq.slots * D); c->Gsell.zero(c->stream);
-        B2_LAUNCH(c, k_rect_to_sell<D>, blocks_for(vq.n_rows, 256), 256, vq.n_rows, vq.rowptr.p, vq.slice_ptr.p, (int64_t)vq.slots, c->P.p, c->Psell.p);
-        B2_LAUNCH(c, k_rect_to_sell<D>, blocks_for(vq.n_rows, 256), 256, vq.n_rows, vq.rowptr.p, vq.slice_ptr.p, (int64_t)vq.slots, c->G.p, c->Gsell.p);
-      }
     }
     B2_LAUNCH(c, (k_assemble_loads<D, DEG>), blocks_for(nc, 128), 128, nc, c->x.p, c->cell_nodes.p, V.cell_dofs.p, Q.cell_dofs.p,
               (int)V.n_owned, (int)Q.n_owned, (int)V.n_local(), f[0], f[1], f[2], c->vec(B2_VEC_B0), c->vec(B2_VEC_MQ));  // :387-390
@@ -1545,17 +1529,24 @@ void do_preassemble(b2_ctx* c, const double* body_force, int low_memory, int rot
   c->preassembled = true;
 }
 
-const DBuf<double>* matrix_values(b2_ctx* c, int mat, const CSR** pat, int* stride) {
-  *stride = 1;
+// how a matrix' values are stored (linalg.cuh, "storage")
+enum class Layout {
+  Sell,           // square operators: one value per SELL slot of the pattern
+  SellByComp,     // P, G: SELL slots, direction k at vals + k * slots
+  CsrInterleaved  // D: CSR positions, the gdim directions of a nonzero side by side ([nnz][gdim])
+};
+
+const DBuf<double>* matrix_values(b2_ctx* c, int mat, const CSR** pat, Layout* layout) {
+  *layout = Layout::Sell;
   switch (mat) {
     case B2_MAT_M: *pat = &c->pat[B2_PAT_VV]; return &c->M;
     case B2_MAT_K: *pat = &c->pat[B2_PAT_VV]; return &c->Kst;
     case B2_MAT_A: *pat = &c->pat[B2_PAT_VV]; return &c->A;
     case B2_MAT_AP: *pat = &c->pat[B2_PAT_QQ]; return &c->Ap;
     case B2_MAT_MQ: *pat = &c->pat[B2_PAT_QQ]; return &c->MQ;
-    case B2_MAT_P: *pat = &c->pat[B2_PAT_VQ]; *stride = c->gdim; return &c->P;
-    case B2_MAT_G: *pat = &c->pat[B2_PAT_VQ]; *stride = c->gdim; return &c->G;
-    case B2_MAT_D: *pat = &c->pat[B2_PAT_QV]; *stride = c->gdim; return &c->D;
+    case B2_MAT_P: *pat = &c->pat[B2_PAT_VQ]; *layout = Layout::SellByComp; return &c->P;
+    case B2_MAT_G: *pat = &c->pat[B2_PAT_VQ]; *layout = Layout::SellByComp; return &c->G;
+    case B2_MAT_D: *pat = &c->pat[B2_PAT_QV]; *layout = Layout::CsrInterleaved; return &c->D;
     default: throw B2Error(-2, "unknown matrix id");
   }
 }
@@ -2024,7 +2015,7 @@ int b2_build_patterns(b2_ctx* c) {
     build_pattern(c, Q, Q, c->pat[B2_PAT_QQ]);
     build_sell(c, c->pat[B2_PAT_VV]);
     build_sell(c, c->pat[B2_PAT_QQ]);
-    build_sell(c, c->pat[B2_PAT_VQ]);  // P_i / G_i products run on the sliced-ELL form too (component-major values)
+    build_sell(c, c->pat[B2_PAT_VQ]);  // P_i / G_i live in the sliced-ELL form too (component-major values)
     c->patterns_built = true;
   });
 }
@@ -2182,20 +2173,20 @@ int b2_get_vector(b2_ctx* c, int vec, int comp, double* host, int64_t n) {
 
 namespace {
 
-// CSR-ordered copy of a matrix' values (SELL operators are converted; A is un-row-scaled)
+// CSR-ordered copy of a matrix' values (direction comp of P, G, D)
 void csr_values(b2_ctx* c, int mat, int comp, DBuf<double>& out, const CSR** pat_out) {
   const CSR* pat = nullptr;
-  int stride = 1;
-  const DBuf<double>* v = matrix_values(c, mat, &pat, &stride);
+  Layout layout;
+  const DBuf<double>* v = matrix_values(c, mat, &pat, &layout);
   B2_REQUIRE(v->p != nullptr, "matrix not assembled (rotational/low-memory option?)");
+  B2_REQUIRE(layout == Layout::Sell || (comp >= 0 && comp < c->gdim), "bad component");
   out.alloc(pat->nnz);
-  if (stride == 1) {
-    B2_REQUIRE(pat->has_sell(), "square operator without SELL layout");
-    B2_LAUNCH(c, k_sell_convert, blocks_for(pat->n_rows, 256), 256, pat->n_rows, pat->rowptr.p, pat->slice_ptr.p, 0, v->p,
-              out.p, (const double*)nullptr);
+  if (layout == Layout::CsrInterleaved) {
+    B2_LAUNCH(c, k_extract, pgrid(c, pat->nnz), 256, pat->nnz, c->gdim, comp, v->p, out.p);
   } else {
-    B2_REQUIRE(comp >= 0 && comp < stride, "bad component");
-    B2_LAUNCH(c, k_extract, pgrid(c, pat->nnz), 256, pat->nnz, stride, comp, v->p, out.p);
+    const double* vals = layout == Layout::SellByComp ? v->p + (size_t)comp * pat->slots : v->p;
+    B2_LAUNCH(c, k_sell_convert, blocks_for(pat->n_rows, 256), 256, pat->n_rows, pat->rowptr.p, pat->slice_ptr.p, 0, vals,
+              out.p, (const double*)nullptr);
   }
   *pat_out = pat;
 }
@@ -2429,28 +2420,40 @@ int b2_get_matrix_values(b2_ctx* c, int mat, int comp, double* host) {
   });
 }
 
-// y = Mat * x: square operators through the production SpMM, rectangular ones through a CSR row kernel
+// y = Mat * x through the products of the time step: the SELL SpMM for square operators; rect_vq for P_i and G_i (every
+// direction computed, direction comp returned); rect_qv for D_i (the other directions of its input set to zero)
 int b2_mat_mult(b2_ctx* c, int mat, int comp, const double* x, double* y) {
   return guarded(c, [&] {
     B2_REQUIRE(c->preassembled, "matrices exist after b2_preassemble");
     const CSR* pat = nullptr;
-    int stride = 1;
-    const DBuf<double>* v = matrix_values(c, mat, &pat, &stride);
+    Layout layout;
+    const DBuf<double>* v = matrix_values(c, mat, &pat, &layout);
     B2_REQUIRE(v->p != nullptr, "matrix not assembled");
+    B2_REQUIRE(layout == Layout::Sell || (comp >= 0 && comp < c->gdim), "bad component");
+    const int64_t nv = c->sp[B2_SPACE_V].n_local();  // ld of velocity-space vectors
     DBuf<double> dx, dy;
-    dx.alloc(pat->n_cols);
-    dy.alloc(pat->n_rows);
-    B2_CUDA(cudaMemcpyAsync(dx.p, x, sizeof(double) * pat->n_cols, cudaMemcpyHostToDevice, c->stream));
-    if (stride == 1) {
-      spmm(c, *pat, v->p, 1, dx.p, dy.p);  // the production SELL kernel
+    const double* yk = nullptr;
+    if (layout == Layout::Sell) {
+      dx.alloc(pat->n_cols);
+      dy.alloc(pat->n_rows);
+      B2_CUDA(cudaMemcpyAsync(dx.p, x, sizeof(double) * pat->n_cols, cudaMemcpyHostToDevice, c->stream));
+      spmm(c, *pat, v->p, 1, dx.p, dy.p);
+      yk = dy.p;
+    } else if (layout == Layout::SellByComp) {
+      dx.alloc(pat->n_cols);
+      dy.alloc(c->gdim * nv);
+      B2_CUDA(cudaMemcpyAsync(dx.p, x, sizeof(double) * pat->n_cols, cudaMemcpyHostToDevice, c->stream));
+      rect_vq(c, v->p, dx.p, nullptr, 1.0, dy.p);
+      yk = dy.p + comp * nv;
     } else {
-      DBuf<double> vals;
-      const CSR* p2 = nullptr;
-      csr_values(c, mat, comp, vals, &p2);
-      B2_LAUNCH(c, (k_rect_vq<1, 4>), blocks_for((int64_t)pat->n_rows * 4, 256), 256, pat->n_rows, pat->rowptr.p, pat->cols.p,
-                vals.p, dx.p, (const double*)nullptr, pat->n_rows, 1.0, dy.p);
+      dx.alloc(c->gdim * nv);
+      dx.zero(c->stream);
+      dy.alloc(pat->n_rows);
+      B2_CUDA(cudaMemcpyAsync(dx.p + comp * nv, x, sizeof(double) * pat->n_cols, cudaMemcpyHostToDevice, c->stream));
+      rect_qv(c, dx.p, 1.0, nullptr, dy.p);
+      yk = dy.p;
     }
-    B2_CUDA(cudaMemcpyAsync(y, dy.p, sizeof(double) * pat->n_rows, cudaMemcpyDeviceToHost, c->stream));
+    B2_CUDA(cudaMemcpyAsync(y, yk, sizeof(double) * pat->n_rows, cudaMemcpyDeviceToHost, c->stream));
     B2_CUDA(cudaStreamSynchronize(c->stream));
   });
 }
@@ -2746,9 +2749,9 @@ int b2_ksp_solve(b2_ctx* c, int solver, int mat, const double* b, double* x, int
     B2_REQUIRE(mat == B2_MAT_M || mat == B2_MAT_K || mat == B2_MAT_A || mat == B2_MAT_AP || mat == B2_MAT_MQ, "square operators only");
     if (mat == B2_MAT_MQ) ensure_mq(c);
     const CSR* pat = nullptr;
-    int stride = 1;
-    const DBuf<double>* v = matrix_values(c, mat, &pat, &stride);
-    const int sp = (mat == B2_MAT_AP || mat == B2_MAT_MQ) ? B2_SPACE_Q : B2_SPACE_V;
+    Layout layout;
+    const DBuf<double>* v = matrix_values(c, mat, &pat, &layout);
+    const int sp =(mat == B2_MAT_AP || mat == B2_MAT_MQ) ? B2_SPACE_Q : B2_SPACE_V;
     const int64_t n = c->sp[sp].n_local();
     ensure_proj_work(c, n);
     DBuf<double> db, dx, dinv;

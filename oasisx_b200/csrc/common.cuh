@@ -68,6 +68,11 @@ __device__ __forceinline__ int ld_stream(const int* p) {
   return v;
 }
 
+// SELL-32 slot of entry t of row `row` (the sliced-ELL layout: linalg.cuh, "storage")
+__device__ __forceinline__ size_t sell_slot(const int* __restrict__ slice_ptr, int row, int t) {
+  return (size_t)__ldg(slice_ptr + (row >> 5)) + ((size_t)t << 5) + (row & 31);
+}
+
 // ---- warp / block reductions ------------------------------------------------------------
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

@@ -97,11 +97,6 @@ __device__ __forceinline__ int csr_find(const int* __restrict__ cols, int lo, in
   return lo;
 }
 
-// SELL-32 slot of entry t of row `row` (see linalg.cuh)
-__device__ __forceinline__ size_t sell_slot_of(const int* __restrict__ slice_ptr, int row, int t) {
-  return (size_t)__ldg(slice_ptr + (row >> 5)) + ((size_t)t << 5) + (row & 31);
-}
-
 // ---- one-off (pre)assembly kernels: one thread per (cell, local row) -----------------------
 enum { B2_FORM_MASS_V = 0, B2_FORM_STIFF_V = 1, B2_FORM_MASS_Q = 2, B2_FORM_STIFF_Q = 3 };
 
@@ -156,10 +151,10 @@ __global__ void k_assemble_square(int64_t n_cells, const double* __restrict__ x,
     }
     int pos = csr_find(cols, lo, hi, dofs[j]);
     if (pair_slot != nullptr) {
-      pair_slot[t * ND + j] = (unsigned)sell_slot_of(slice_ptr, row, pos - lo);
+      pair_slot[t * ND + j] = (unsigned)sell_slot(slice_ptr, row, pos - lo);
       pair_val[t * ND + j] = v;
     } else {
-      atomicAdd(vals + sell_slot_of(slice_ptr, row, pos - lo), v);
+      atomicAdd(vals + sell_slot(slice_ptr, row, pos - lo), v);
     }
   }
 }
@@ -175,13 +170,14 @@ __global__ void k_sum_slot_runs(int64_t n, const unsigned* __restrict__ slot, co
   vals[slot[t]] = acc;
 }
 
-// P_c[j,q] = int psi_q d_c phi_j and G_c[j,q] = int d_c psi_q phi_j on the V x Q pattern; the D
-// direction values of one nonzero are stored contiguously ([nnz][D]).
+// P_c[j,q] = int psi_q d_c phi_j and G_c[j,q] = int d_c psi_q phi_j in the SELL-32 slots of the V x Q
+// pattern, component-major: direction c at vals + c * slots (the form k_rect_vq_sell reads; pads stay 0).
 template <int D, int DEG>
 __global__ void k_assemble_PG(int64_t n_cells, const double* __restrict__ x,
                               const int* __restrict__ cell_nodes, const int* __restrict__ vdofs,
                               const int* __restrict__ qdofs, int n_rows_owned,
                               const int* __restrict__ rowptr, const int* __restrict__ cols,
+                              const int* __restrict__ slice_ptr, int64_t slots,
                               double* __restrict__ Pvals, double* __restrict__ Gvals) {
   using E = El<D, DEG>;
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -193,7 +189,7 @@ __global__ void k_assemble_PG(int64_t n_cells, const double* __restrict__ x,
   Geo<D> g = cell_geometry<D>(x, cell_nodes + c * (D + 1));
   int lo = rowptr[row], hi = rowptr[row + 1];
   for (int q = 0; q < E::NQ; ++q) {
-    int pos = csr_find(cols, lo, hi, qdofs[c * E::NQ + q]);
+    const size_t s = sell_slot(slice_ptr, row, csr_find(cols, lo, hi, qdofs[c * E::NQ + q]) - lo);
 #pragma unroll
     for (int k = 0; k < D; ++k) {
       double p = 0, gg = 0;
@@ -202,8 +198,8 @@ __global__ void k_assemble_PG(int64_t n_cells, const double* __restrict__ x,
         p += g.Kinv[dl][k] * E::PX(dl, j, q);
         gg += g.Kinv[dl][k] * E::GX(dl, j, q);
       }
-      atomicAdd(Pvals + (size_t)pos * D + k, g.detJ * p);
-      atomicAdd(Gvals + (size_t)pos * D + k, g.detJ * gg);
+      atomicAdd(Pvals + (size_t)k * slots + s, g.detJ * p);
+      atomicAdd(Gvals + (size_t)k * slots + s, g.detJ * gg);
     }
   }
 }

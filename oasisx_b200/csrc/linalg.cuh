@@ -246,19 +246,16 @@ __global__ void k_halo_unpack(int n_neighbors, const int64_t* __restrict__ recv_
 
 // ---- storage ------------------------------------------------------------------------------------
 // Vectors: component-major (SoA): component k of a velocity-space vector lives at v + k*ld, ld = dofs
-// of the space incl. ghosts.  Square operators (M, K, A on VxV; Ap, MQ on QxQ): sliced ELLPACK with
-// 32-row slices ("SELL-32"): entry t of row r is at slice_ptr[r/32] + 32*t + r%32, rows padded to
-// the longest row of their slice with (col = r, val = 0).  One thread owns one row; at step t the 32
-// lanes of a warp read 32 consecutive values and 32 consecutive column indices (2 + 1 L1 wavefronts)
-// and, because the host numbers dofs by stencil class (fem._class_order), their 32 gathered vector
-// entries are (nearly) consecutive too.  No cross-lane reduction is needed.  The CSR pattern of
-// create_matrix stays the public face (b2_get_pattern); CSR position p of row r maps to the SELL
-// slot slice_ptr[r/32] + 32*(p - rowptr[r]) + r%32.
+// of the space incl. ghosts.  Square operators (M, K, A on VxV; Ap, MQ on QxQ) and P_i, G_i on VxQ (the
+// directions one after the other, vals + i*slots): sliced ELLPACK with 32-row slices ("SELL-32"): entry t
+// of row r is at slice_ptr[r/32] + 32*t + r%32, rows padded to the longest row of their slice with
+// (col = r, or 0 past the last column, val = 0).  D_i (QxV) is CSR with [nnz][K] values.  One thread
+// owns one row; at step t the 32 lanes of a warp read 32 consecutive values and 32 consecutive column
+// indices (2 + 1 L1 wavefronts) and, because the host numbers dofs by stencil class (fem._class_order),
+// their 32 gathered vector entries are (nearly) consecutive too.  No cross-lane reduction is needed.
+// The CSR pattern of create_matrix stays the public face (b2_get_pattern); CSR position p of row r maps
+// to the SELL slot slice_ptr[r/32] + 32*(p - rowptr[r]) + r%32 (sell_slot, common.cuh).
 // ld_stream (common.cuh): streaming loads for the matrix stream (values, columns)
-
-__device__ __forceinline__ size_t sell_slot(const int* __restrict__ slice_ptr, int row, int t) {
-  return (size_t)__ldg(slice_ptr + (row >> 5)) + ((size_t)t << 5) + (row & 31);
-}
 
 __global__ void k_sell_slice_len(int n_rows, const int* __restrict__ rowptr, int* __restrict__ slice_entries) {
   int s = blockIdx.x * blockDim.x + threadIdx.x;
@@ -457,42 +454,11 @@ k_matvec_rhs(int n_rows, const int* __restrict__ slice_ptr, const int* __restric
   }
 }
 
-// ---- rectangular products on the V x Q and Q x V CSR patterns ([nnz][K] values) -----------------
-// out_k[row] = add_k[row] + scale * sum_p vals[p][k] * xq[cols[p]]   (P_i ps, G_i dp)
-template <int K, int LPR>
-__global__ void __launch_bounds__(256)
-k_rect_vq(int n_rows, const int* __restrict__ rowptr, const int* __restrict__ cols,
-          const double* __restrict__ vals, const double* __restrict__ xq, const double* add, int ld,
-          double scale, double* out) {
-  const int lane = threadIdx.x % LPR;
-  const int row = (blockIdx.x * blockDim.x + threadIdx.x) / LPR;
-  double acc[K];
-#pragma unroll
-  for (int k = 0; k < K; ++k) acc[k] = 0.0;
-  if (row < n_rows) {
-    const int end = __ldg(rowptr + row + 1);
-    for (int p = __ldg(rowptr + row) + lane; p < end; p += LPR) {
-      const double xv = __ldg(xq + __ldg(cols + p));
-#pragma unroll
-      for (int k = 0; k < K; ++k) acc[k] = fma(__ldg(vals + (size_t)p * K + k), xv, acc[k]);
-    }
-  }
-#pragma unroll
-  for (int o = LPR / 2; o > 0; o >>= 1)
-#pragma unroll
-    for (int k = 0; k < K; ++k) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
-  if (row < n_rows && lane == 0) {
-#pragma unroll
-    for (int k = 0; k < K; ++k) {
-      const double a = add != nullptr ? add[(size_t)k * ld + row] : 0.0;
-      out[(size_t)k * ld + row] = fma(scale, acc[k], a);
-    }
-  }
-}
-
-// The same products on the sliced-ELL form of the V x Q pattern with COMPONENT-MAJOR values (vals + k * slots): the
-// P2 rows have only 4-14 entries, so the CSR kernel above (4-8 lanes per row, [nnz][K] values) runs at 0.56 of the HBM
-// peak; one thread per row over coalesced streams reads (8 K + 4) bytes per slot and nothing else.
+// ---- rectangular products -------------------------------------------------------------------------
+// out_k[row] = add_k[row] + scale * sum_t vals[k * slots + slot] * xq[cols[slot]]   (P_i ps, G_i dp)
+// on the sliced-ELL form of the V x Q pattern with COMPONENT-MAJOR values (vals + k * slots): the P2 rows have only
+// 4-14 entries, so a CSR kernel (4-8 lanes per row, [nnz][K] values) ran at 0.56 of the HBM peak; one thread per row
+// over coalesced streams reads (8 K + 4) bytes per slot and nothing else.
 template <int K>
 __global__ void __launch_bounds__(256, 4)
 k_rect_vq_sell(int n_rows, const int* __restrict__ slice_ptr, const int* __restrict__ cols, const double* __restrict__ vals,
@@ -525,20 +491,7 @@ k_rect_vq_sell(int n_rows, const int* __restrict__ slice_ptr, const int* __restr
   }
 }
 
-// [nnz][K] CSR values -> component-major sliced-ELL slots (pads stay 0)
-template <int K>
-__global__ void k_rect_to_sell(int n_rows, const int* __restrict__ rowptr, const int* __restrict__ slice_ptr, int64_t slots,
-                               const double* __restrict__ in, double* __restrict__ out) {
-  const int row = blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= n_rows) return;
-  const int start = rowptr[row], n = rowptr[row + 1] - start;
-  const size_t base = (size_t)slice_ptr[row >> 5] + (row & 31);
-  for (int t = 0; t < n; ++t)
-#pragma unroll
-    for (int k = 0; k < K; ++k) out[(size_t)k * slots + base + ((size_t)t << 5)] = in[(size_t)(start + t) * K + k];
-}
-
-// out[q] = scale * sum_p sum_k vals[p][k] * xv_k[cols[p]]            (sum_i D_i u_i)
+// out[q] = scale * sum_p sum_k vals[p][k] * xv_k[cols[p]]            (sum_i D_i u_i, CSR [nnz][K] values)
 template <int K, int LPR>
 __global__ void __launch_bounds__(256)
 k_rect_qv(int n_rows, const int* __restrict__ rowptr, const int* __restrict__ cols,

@@ -132,8 +132,10 @@ def test_mat_mult_matches_oracle(kind, gdim, deg):
     o = make_oracle(msh, deg, tg, 0.01)
     rng = np.random.default_rng(0)
     xv, xq = rng.uniform(-1, 1, o.nV), rng.uniform(-1, 1, o.nQ)
-    for dev, ref, x in [(s._M, o.M, xv), (s._K, o.K, xv), (s._Ap, o.Ap, xq), (s._p_vdxi_Mat[1], o.P[1], xq),
-                        (s._divu_Mat[0], o.D[0], xv)]:
+    cases = [(s._M, o.M, xv), (s._K, o.K, xv), (s._Ap, o.Ap, xq)]
+    for i in range(gdim):
+        cases += [(s._p_vdxi_Mat[i], o.P[i], xq), (s._grad_p_Mat[i], o.G[i], xq), (s._divu_Mat[i], o.D[i], xv)]
+    for dev, ref, x in cases:
         y = np.zeros(ref.shape[0])
         dev.mult(x, y)
         assert _seen("mat_mult", relerr(y, ref @ x)) <= 1e-13
