@@ -222,6 +222,14 @@ int b2_get_matrix_values(b2_ctx* ctx, int mat, int comp, double* host);
 int b2_mat_mult(b2_ctx* ctx, int mat, int comp, const double* x, double* y);
 
 /* ---- solver options (ksp.py:38-53; SURVEY.md Appendix G) ------------------------------ */
+/* GMRES keys (solver slots TENTATIVE, SCALAR and PROJECTOR; ksp_type gmres on the PRESSURE slot fails):
+ *   ksp_type gmres                       restarted GMRES(m), left preconditioned with pc_type jacobi (or none);
+ *   ksp_gmres_restart m                  restart length, 1 <= m <= 100 (default 30), anything else fails;
+ *   ksp_gmres_cgs_refinement_type t      refine_never (default): one classical Gram-Schmidt pass per step;
+ *                                        refine_always: two passes; refine_ifneeded runs two passes as well.
+ * ksp_gmres_modifiedgramschmidt is not built and, like every unknown key, ignored.  Iterations count Arnoldi steps
+ * over all restarts; the convergence test compares the Arnoldi residual estimate (and, at each restart, the true
+ * preconditioned residual) with max(rtol |D^-1 b|, atol). */
 int b2_set_solver_option(b2_ctx* ctx, int solver, const char* key, const char* value);
 
 /* ---- the stages, one-to-one with the reference methods -------------------------------- */

@@ -8,7 +8,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "csrc", "b200ipcs.cu")
 LIB = os.path.join(HERE, "libb200ipcs.so")
-DEPS = [SRC] + [os.path.join(HERE, "csrc", f) for f in ("common.cuh", "elem.cuh", "linalg.cuh", "mg.cuh", "amg.cuh", "ref_tables.h")] + [
+DEPS = [SRC] + [os.path.join(HERE, "csrc", f) for f in ("common.cuh", "elem.cuh", "linalg.cuh", "mg.cuh", "amg.cuh", "gmres.cuh", "ref_tables.h")] + [
     os.path.join(os.path.dirname(HERE), "include", "b200ipcs.h")
 ]
 

@@ -8,6 +8,7 @@
 #include <nccl.h>  // types only: the library is dlopen'ed when a multi-rank context is created
 
 #include <algorithm>
+#include <cctype>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -20,6 +21,7 @@
 #include "linalg.cuh"
 #include "mg.cuh"
 #include "amg.cuh"
+#include "gmres.cuh"
 
 namespace {
 
@@ -44,7 +46,9 @@ struct Space {
 };
 
 struct KSPOpts {
-  int type = 0;  // 0 = cg, 1 = bcgs, 2 = chebyshev (mass solves: needs eig bounds, b2_set_solver_option ksp_chebyshev_eigenvalues)
+  int type = 0;  // 0 = cg, 1 = bcgs, 2 = chebyshev (mass solves: needs eig bounds, b2_set_solver_option ksp_chebyshev_eigenvalues), 3 = gmres
+  int restart = 30;     // GMRES restart length m (ksp_gmres_restart)
+  bool cgs2 = false;    // GMRES: a second classical Gram-Schmidt pass (ksp_gmres_cgs_refinement_type refine_always)
   double eig_lo = 0.0, eig_hi = 0.0;  // bounds of the spectrum of D^-1 A for type 2
   int pc = 0;    // 0 = jacobi, 1 = none, 2 = multigrid (pressure only, needs b2_pressure_mg_add_level)
   double rtol = 1e-5, atol = 1e-50;
@@ -255,6 +259,8 @@ struct b2_ctx {
   bool step_begun = false;  // b2_step_begin was called for the step b2_step is about to finish
   KryState* d_st = nullptr;
   KryState* h_st = nullptr;  // pinned
+  GmresState* d_gm = nullptr;  // GMRES Hessenberg / Givens state, allocated by the first GMRES solve
+  DBuf<double> gm_V;           // GMRES basis: m+1 vectors of K components, vector i component k at (i K + k) ld
   double* d_sums = nullptr;  // small device scratch for reductions (16 doubles)
   double* h_sums = nullptr;  // pinned
   DBuf<double> partials;
@@ -580,6 +586,80 @@ void krylov_init(b2_ctx* c, const KSPOpts& o, const CSR& pat, const double* vals
   }
 }
 
+// GMRES(m), left Jacobi (gmres.cuh).  Every active component is at the same Arnoldi index j, so the host knows where
+// the cycles close and enqueues the solution update and the restart residual without reading the device; the state is
+// read back once per batch of steps, as for the other methods.
+template <int K>
+void gmres_solve(b2_ctx* c, const KSPOpts& o, const CSR& pat, const double* vals, const double* dinv, int space,
+                 const double* b, double* x, double* q) {
+  const int64_t n = pat.n_rows;
+  const int ld = pat.n_cols, m = o.restart;
+  const size_t need = (size_t)(m + 1) * K * ld;
+  if ((size_t)c->gm_V.n < need) c->gm_V.alloc((int64_t)need);  // 96^3, m = 30, K = 3: 5.3 GB
+  if (c->d_gm == nullptr) B2_CUDA(cudaMalloc(&c->d_gm, sizeof(GmresState)));
+  GmresState* gs = c->d_gm;
+  KryState* st = c->d_st;
+  double* V = c->gm_V.p;
+  auto vec = [&](int i) { return V + (size_t)i * K * ld; };
+  const int here = c->nranks == 1;  // one rank: the scalar updates run in the reducing kernels' last block
+  const int g = pgrid(c, n, 256, 8);
+  const int gd = (int)std::min<int64_t>(c->sm, (n + 511) / 512);  // k_gmres_dots: one set of (m+1) K partials per block
+  constexpr int CH = 8;
+  auto residual = [&](bool init) {  // v_0 = D^-1 (b - A x) / |.|
+    const double* q0 = nullptr;
+    if (!init || o.nonzero_guess) {
+      spmm(c, pat, vals, K, x, q, nullptr, init ? nullptr : st, FIN_NONE, 0, space, dinv);
+      q0 = q;
+    }
+    B2_LAUNCH(c, k_gmres_residual<K>, g, 256, n, ld, b, q0, dinv, x, vec(0), (int)init, here, gs, st, c->partials.p, c->d_counter);
+    if (!here) {
+      allreduce_sum(c, gs->tot, 2 * K);
+      B2_LAUNCH(c, k_gmres_fin, 1, 1, init ? GM_FIN_INIT : GM_FIN_RESTART, gs, st, 0, 1, 1);
+    }
+    B2_LAUNCH(c, k_gmres_scale<K>, g, 256, n, ld, vec(0), gs, st);
+  };
+  auto step = [&](int j) {
+    double* w = vec(j + 1);
+    spmm(c, pat, vals, K, vec(j), w, nullptr, st, FIN_NONE, 0, space, dinv);  // w = D^-1 A v_j
+    const int passes = o.cgs2 ? 2 : 1;
+    for (int pass = 0; pass < passes; ++pass) {
+      const int first = pass == 0, last = pass == passes - 1;
+      B2_LAUNCH(c, (k_gmres_dots<K, CH>), gd, 512, n, ld, V, j, w, gs, st, c->partials.p, c->d_counter);
+      if (!here) allreduce_sum(c, gs->hcol, (j + 1) * K);
+      B2_LAUNCH(c, k_gmres_orth<K>, g, 256, n, ld, V, j, w, first, last, here, gs, st, c->partials.p, c->d_counter);
+      if (!here) {
+        allreduce_sum(c, gs->tot, K);
+        B2_LAUNCH(c, k_gmres_fin, 1, 1, GM_FIN_ORTH, gs, st, j, first, last);
+      }
+    }
+    B2_LAUNCH(c, k_gmres_scale<K>, g, 256, n, ld, w, gs, st);
+  };
+  auto close_cycle = [&]() {  // x += V y for every component that took steps in this cycle (not gated by `done`)
+    B2_LAUNCH(c, k_gmres_backsolve, 1, 32, gs, K);
+    B2_LAUNCH(c, k_gmres_update_x<K>, g, 256, n, ld, V, x, gs);
+  };
+  residual(true);
+  int j = 0, launched = 0;
+  int chunk = std::max(1, o.expected_its);
+  for (;;) {
+    for (int s = 0; s < chunk; ++s) {
+      step(j);
+      if (++j == m) {
+        close_cycle();
+        residual(false);
+        j = 0;
+      }
+    }
+    launched += chunk;
+    B2_CUDA(cudaMemcpyAsync(c->h_st, c->d_st, sizeof(KryState), cudaMemcpyDeviceToHost, c->stream));
+    B2_CUDA(cudaStreamSynchronize(c->stream));
+    c->stats.bytes_d2h += sizeof(KryState);
+    if (c->h_st->done || launched > o.maxit + 1) break;
+    chunk = std::max(2, std::min(launched / 4, 16));
+  }
+  close_cycle();
+}
+
 // Solves K systems  A x_k = b_k  (interleaved storage) with the options of solver `which`.
 void chebyshev_solve(b2_ctx* c, int which, const CSR& pat, const double* vals, const double* dinv, int space, int K,
                      const double* b, double* x, int32_t* reasons, int32_t* its);
@@ -592,9 +672,9 @@ void krylov_solve(b2_ctx* c, int which, const CSR& pat, const double* vals, cons
     return;
   }
   DBuf<double>* w = work != nullptr ? work : (space == B2_SPACE_V ? c->wv : c->wq);
-  // CG: Jacobi through dinv in the vector kernels.  BiCGStab: left preconditioning D^-1 A x = D^-1 b -- dinv scales
-  // the right-hand side in k_bcgs_init and every operator application in the SpMM epilogue (the matrix is stored as
-  // assembled).  pc_type none: dinv = 1.
+  // CG: Jacobi through dinv in the vector kernels.  BiCGStab and GMRES: left preconditioning D^-1 A x = D^-1 b -- dinv
+  // scales the right-hand side in k_bcgs_init / k_gmres_residual and every operator application in the SpMM epilogue
+  // (the matrix is stored as assembled).  pc_type none: dinv = 1.
   const double* dinv = (o.pc != 1) ? dinv_jacobi : (space == B2_SPACE_V ? c->onesV.p : c->onesQ.p);
   double *r = w[0].p, *p = w[1].p, *q = w[2].p, *t = nullptr, *rhat = nullptr;
   if (o.type == 1) {
@@ -611,6 +691,10 @@ void krylov_solve(b2_ctx* c, int which, const CSR& pat, const double* vals, cons
   B2_CUDA(cudaMemcpyAsync(c->d_st, c->h_st, sizeof(KryState), cudaMemcpyHostToDevice, c->stream));
   auto run = [&](auto kc) {
     constexpr int KK = decltype(kc)::value;
+    if (o.type == 3) {
+      gmres_solve<KK>(c, o, pat, vals, dinv, space, b, x, q);
+      return;
+    }
     krylov_init<KK>(c, o, pat, vals, dinv, space, b, x, r, p, q, rhat);
     int chunk = std::max(1, o.expected_its);
     int launched = 0;
@@ -1647,6 +1731,7 @@ void b2_destroy(b2_ctx* c) {
   cudaFreeHost(c->h_sums);
   cudaFree(c->d_counter);
   cudaFree(c->d_red);
+  cudaFree(c->d_gm);
   if (c->pcg_graph) cudaGraphExecDestroy(c->pcg_graph);
   for (auto& sg : c->seg) {
     for (int q = 0; q < B2_MAXR; ++q)
@@ -2467,7 +2552,11 @@ int b2_set_solver_option(b2_ctx* c, int solver, const char* key, const char* val
       if (v == "cg") o.type = 0;
       else if (v == "bcgs" || v == "bicgstab") o.type = 1;
       else if (v == "preonly") { /* direct solve requested: keep the Krylov default, tighten below */ }
-      else if (v == "gmres") o.type = 1;  // nonsymmetric Krylov available here is BiCGStab
+      else if (v == "gmres") {
+        // the pressure solve is CG (with multigrid or Jacobi); PETSc would accept GMRES there
+        B2_REQUIRE(solver != B2_SOLVER_PRESSURE, "ksp_type gmres is not available for the pressure solve (cg only)");
+        o.type = 3;
+      }
       else if (v == "chebyshev") {
         B2_REQUIRE(solver == B2_SOLVER_SCALAR || solver == B2_SOLVER_PROJECTOR, "chebyshev is for the SPD mass solves");
         o.type = 2;
@@ -2480,6 +2569,18 @@ int b2_set_solver_option(b2_ctx* c, int solver, const char* key, const char* val
       else if (v == "mg" || v == "gamg" || v == "hypre") o.pc = (solver == B2_SOLVER_PRESSURE) ? 2 : 0;
       else if (v == "lu" || v == "cholesky") { o.pc = 0; o.rtol = 1e-12; o.atol = 1e-50; }  // "exact" solve (Appendix G)
       else throw B2Error(-5, "unsupported pc_type " + v + " (jacobi | none | mg | gamg | hypre | lu | cholesky)");  // PETSc errors on an unknown PC type too
+    } else if (k == "ksp_gmres_restart") {
+      const int m = std::stoi(v);
+      B2_REQUIRE(m >= 1 && m <= B2_GMRES_MAXM, "ksp_gmres_restart must be in 1.." + std::to_string(B2_GMRES_MAXM));
+      o.restart = m;
+    } else if (k == "ksp_gmres_cgs_refinement_type") {
+      std::string u = v;
+      for (auto& ch : u) ch = (char)std::tolower((unsigned char)ch);
+      if (u.rfind("ksp_gmres_cgs_", 0) == 0) u = u.substr(14);  // PETSc also accepts the enum's C name
+      // refine_ifneeded runs the second pass always (no estimate of the cancellation is made)
+      if (u == "refine_never") o.cgs2 = false;
+      else if (u == "refine_ifneeded" || u == "refine_always") o.cgs2 = true;
+      else throw B2Error(-5, "unsupported ksp_gmres_cgs_refinement_type " + v + " (refine_never | refine_ifneeded | refine_always)");
     } else if (k == "ksp_rtol") o.rtol = std::stod(v);
     else if (k == "ksp_atol") o.atol = std::stod(v);
     else if (k == "ksp_max_it") o.maxit = std::stoi(v);

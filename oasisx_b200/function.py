@@ -85,7 +85,8 @@ class Projector:
         # which device space carries this degree in that context (a solver's context may be P1-P1)
         self._slot = self._space_slot(space)
         for k, v in (petsc_options or {}).items():
-            if k in ("ksp_type", "pc_type", "ksp_rtol", "ksp_atol", "ksp_max_it"):
+            if k in ("ksp_type", "pc_type", "ksp_rtol", "ksp_atol", "ksp_max_it", "ksp_gmres_restart",
+                     "ksp_gmres_cgs_refinement_type"):
                 self._ctx.set_solver_option(L.SOLVER_PROJECTOR, k, v)
         degree = int((metadata or {}).get("quadrature_degree", 4))
         self._pts, self._w = simplex_rule(space.mesh.geometry.dim, degree)

@@ -12,7 +12,7 @@ import logging
 logger = logging.getLogger("oasisx")
 
 _UNDERSTOOD = {"ksp_type", "pc_type", "ksp_rtol", "ksp_atol", "ksp_max_it", "ksp_initial_guess_nonzero", "b200_guess",
-               "ksp_chebyshev_eigenvalues", "b200_block_rtol"}
+               "ksp_chebyshev_eigenvalues", "b200_block_rtol", "ksp_gmres_restart", "ksp_gmres_cgs_refinement_type"}
 
 
 class KSPSolver:
@@ -33,8 +33,6 @@ class KSPSolver:
             return
         for k, v in options.items():
             if k in _UNDERSTOOD:
-                if k == "ksp_type" and str(v) == "gmres":
-                    logger.warning("%sksp_type=gmres: the device Krylov stack solves nonsymmetric systems with BiCGStab", self._prefix)
                 self._ctx.set_solver_option(self._slot, k, v)
             else:
                 logger.debug("option %s%s=%s ignored by the B200 Krylov stack", self._prefix, k, v)
