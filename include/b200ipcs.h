@@ -198,11 +198,23 @@ int b2_pressure_mg_configure(b2_ctx* ctx, int nu_pre, int nu_post, int coarse_sw
  * MIS(2) of that graph with hash keys (Bell, Dalton and Olson 2012).  P = (I - 4/(3 rho) D^-1 A) T with T the
  * aggregate indicator, R = P^T, A_c = R A P, repeated until a level has at most 5000 dofs (solved exactly), the
  * coarsening ratio drops below 2, or 15 coarse levels; rho = 20 power iterations on D^-1 A.  Deterministic: the same
- * Ap gives the same hierarchy bit for bit.  Call after b2_preassemble on a context without multigrid levels, on one
- * rank, without pressure Dirichlet dofs (the coarse solve relies on the constant null space); otherwise an error. */
+ * Ap gives the same hierarchy bit for bit.  Call after b2_preassemble on a context without multigrid levels and
+ * without pressure Dirichlet dofs (the coarse solve relies on the constant null space); otherwise an error.
+ * Several ranks (collective; b2_set_pressure_global_ids first; one rank takes the same path once it has been given
+ * global ids, numbering the hierarchy by them): the owned rows of Ap of all ranks are gathered over
+ * NCCL into the global matrix, and every rank builds the same hierarchy from it.  Levels 2 and below are global and
+ * replicated; level 1 keeps this rank's part only: P_1 the rows of its owned dofs (local order), R_1 = P_1^T with
+ * local columns (ghost columns empty), the aggregates of its owned dofs.  Set-up memory on every GPU: the global
+ * matrix and its sort buffers (DESIGN.md section 2). */
 int b2_pressure_amg_build(b2_ctx* ctx);
+/* Global index of every local pressure dof, owned then ghost (n = n_owned + n_ghost), for the multi-rank algebraic
+ * multigrid.  Collective on several ranks.  Every index lies in [0, n_global) (b2_set_global_sizes; n_global <= 2^31,
+ * the pair keys of the set-up are row << 32 | col), no rank lists an index twice, and the owned indices of all ranks
+ * cover 0 .. n_global-1 exactly once; otherwise an error on every rank. */
+int b2_set_pressure_global_ids(b2_ctx* ctx, int64_t n, const int64_t* gids);
 /* out[7] = {n, nnz(A_l), nnz(P_l), algebraic (0/1), solved densely (0/1), omega_l, rho_hat_l} of level `level`
- * (0 = the fine level: nnz(P) = 0; rho_hat = 0 on geometric levels). */
+ * (0 = the fine level: nnz(P) = 0; rho_hat = 0 on geometric levels).  On several ranks n and nnz of level 0 and
+ * nnz(P_1) are this rank's. */
 int b2_pressure_mg_level_info(b2_ctx* ctx, int level, double* out);
 /* Test hook: level >= 1, what = 0: A_l as CSR with sorted columns, 1: P_l, 2: R_l (indptr, indices, vals; sizes from
  * b2_pressure_mg_level_info); 3 (algebraic levels): `indices` receives the aggregate of every dof of level - 1. */

@@ -28,6 +28,7 @@ SYMBOLS = [
     "b2_host_alloc", "b2_host_free", "b2_set_mesh", "b2_set_space", "b2_set_halo", "b2_set_global_sizes",
     "b2_first_plan_info", "b2_bench_assembly_strategies", "b2_peer_export", "b2_peer_import", "b2_peer_disable", "b2_peer_enabled",
     "b2_build_patterns", "b2_pattern_nnz", "b2_pattern_sell_slots", "b2_set_slice_order", "b2_pressure_mg_add_level", "b2_pressure_mg_configure", "b2_pressure_amg_build",
+    "b2_set_pressure_global_ids",
     "b2_pressure_mg_level_info", "b2_pressure_mg_get_level", "b2_get_pattern", "b2_set_velocity_bc_dofs",
     "b2_set_velocity_bc_values", "b2_set_velocity_bc_series", "b2_select_bc_step", "b2_reset_time_history", "b2_profiler_range", "b2_set_pressure_bc_dofs", "b2_declare_pressure_bcs", "b2_preassemble", "b2_set_vector", "b2_get_vector",
     "b2_get_matrix_values", "b2_mat_mult", "b2_set_solver_option", "b2_assemble_first", "b2_tentative_assemble",
@@ -105,6 +106,7 @@ def load_library() -> C.CDLL:
         "b2_pressure_mg_add_level": (i32, [vp, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp]),
         "b2_pressure_mg_configure": (i32, [vp, i32, i32, i32, dbl]),
         "b2_pressure_amg_build": (i32, [vp]),
+        "b2_set_pressure_global_ids": (i32, [vp, i64, vp]),
         "b2_pressure_mg_level_info": (i32, [vp, i32, vp]),
         "b2_pressure_mg_get_level": (i32, [vp, i32, i32, vp, vp, vp]),
         "b2_get_pattern": (i32, [vp, i32, vp, vp]),
@@ -250,8 +252,15 @@ class Context:
         self._check(self.lib.b2_pressure_mg_configure(self._h, nu_pre, nu_post, coarse_sweeps, omega), "b2_pressure_mg_configure")
 
     def pressure_amg_build(self):
-        """Smoothed-aggregation hierarchy from the assembled pressure matrix (after preassemble, one rank)."""
+        """Smoothed-aggregation hierarchy from the assembled pressure matrix (after preassemble; on several ranks
+        after :meth:`set_pressure_global_ids`, collectively)."""
         self._check(self.lib.b2_pressure_amg_build(self._h), "b2_pressure_amg_build")
+
+    def set_pressure_global_ids(self, l2g):
+        """Global index of every local pressure dof, owned then ghost (``LocalSpace.l2g``); collective on several
+        ranks.  Raises B200Error on every rank unless the owned indices of all ranks cover 0 .. n_global-1 once."""
+        g = np.ascontiguousarray(l2g, dtype=np.int64)
+        self._check(self.lib.b2_set_pressure_global_ids(self._h, g.size, _ptr(g)), "b2_set_pressure_global_ids")
 
     MG_LEVEL_INFO = ("n", "nnz_A", "nnz_P", "algebraic", "dense", "omega", "rho_hat")
 

@@ -57,7 +57,8 @@ def halo_plan_from_index_map(index_map, comm, ghosts=None, owners=None) -> HaloP
     wanted = {int(q): ghosts[owners == q] for q in np.unique(owners)}  # what I need from rank q
     all_wanted = comm.allgather(wanted)  # all_wanted[r][q] = globals rank r needs from q
     me = comm.rank
-    send = {r: w[me] for r, w in enumerate(all_wanted) if me in w and len(w[me])}
+    # np.asarray: oasisx_b200.comm.HostComm carries the arrays as plain lists
+    send = {r: np.asarray(w[me], dtype=np.int64) for r, w in enumerate(all_wanted) if me in w and len(w[me])}
     neighbors = np.array(sorted(set(wanted) | set(send)), dtype=np.int32)
     send_off, recv_off, send_idx = [0], [0], []
     for q in neighbors:

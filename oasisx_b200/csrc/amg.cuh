@@ -1,6 +1,7 @@
 // amg.cuh -- kernels of the smoothed-aggregation algebraic multigrid set-up (b2_pressure_amg_build): strength graph,
 // MIS(2) aggregation (Bell, Dalton and Olson 2012), power iteration for rho(D^-1 A), and the expand-sort-reduce sparse
-// products behind P = (I - omega D^-1 A) T, R = P^T and A_c = R (A P).  Every step is deterministic: no floating-point
+// products behind P = (I - omega D^-1 A) T, R = P^T and A_c = R (A P), and on several ranks the gather of the global
+// fine matrix and the cut of level 1 back to each rank's owned rows.  Every step is deterministic: no floating-point
 // atomics, sums are taken sequentially in an order fixed by a stable sort, and the reductions of the power iteration
 // run in one block in a fixed order (k_amg_sum).  The V-cycle that uses the hierarchy is mg.cuh's.
 #pragma once
@@ -216,6 +217,50 @@ __global__ void k_amg_heads(int64_t n, const unsigned long long* __restrict__ ke
   const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t > n) return;
   head[t] = t < n && (t == 0 || keys[t] != keys[t - 1]);
+}
+
+// ---- several ranks: the global matrix gathered from every rank's owned rows, level 1 cut back to the owned rows -----
+// (global row << 32 | global col, a_ij) for every entry of this rank's owned rows; gid = global id of every local dof
+__global__ void k_amg_global_pairs(int n, const int* __restrict__ rp, const int* __restrict__ ci, const double* __restrict__ va,
+                                   const int* __restrict__ gid, unsigned long long* __restrict__ keys, double* __restrict__ vals) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const unsigned long long r = (unsigned long long)(unsigned)gid[i] << 32;
+  for (int p = rp[i]; p < rp[i + 1]; ++p) {
+    keys[p] = r | (unsigned)gid[ci[p]];
+    vals[p] = va[p];
+  }
+}
+
+// dinv_i = 1 / a_ii of a CSR matrix (every row of the gathered Ap holds its diagonal)
+__global__ void k_amg_inv_diag(int n, const int* __restrict__ rp, const int* __restrict__ ci, const double* __restrict__ va,
+                               double* __restrict__ dinv) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  for (int p = rp[i]; p < rp[i + 1]; ++p)
+    if (ci[p] == i) dinv[i] = 1.0 / va[p];
+}
+
+// len[i] = length of row gid[i] of a CSR matrix
+__global__ void k_amg_row_lengths(int n, const int* __restrict__ rp, const int* __restrict__ gid, int* __restrict__ len) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) len[i] = rp[gid[i] + 1] - rp[gid[i]];
+}
+
+// row i of the output = row gid[i] of (rp, ci, va), and agg_out[i] = agg[gid[i]]: the rows of the global P_1 and the
+// aggregates of this rank's owned dofs, in local order
+__global__ void k_amg_gather_rows(int n, const int* __restrict__ rp, const int* __restrict__ ci, const double* __restrict__ va,
+                                  const int* __restrict__ agg, const int* __restrict__ gid, const int* __restrict__ rp_out,
+                                  int* __restrict__ ci_out, double* __restrict__ va_out, int* __restrict__ agg_out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int g = gid[i];
+  int o = rp_out[i];
+  for (int p = rp[g]; p < rp[g + 1]; ++p, ++o) {
+    ci_out[o] = ci[p];
+    va_out[o] = va[p];
+  }
+  agg_out[i] = agg[g];
 }
 
 // one thread per run: the run's key and the sequential sum of its values, in sorted (= stable generation) order

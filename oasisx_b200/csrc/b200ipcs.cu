@@ -72,6 +72,7 @@ struct NcclApi {
   ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
   const char* (*GetErrorString)(ncclResult_t) = nullptr;
   void load() {
     if (lib) return;
@@ -93,6 +94,7 @@ struct NcclApi {
     Send = (decltype(Send))sym("ncclSend");
     Recv = (decltype(Recv))sym("ncclRecv");
     AllReduce = (decltype(AllReduce))sym("ncclAllReduce");
+    AllGather = (decltype(AllGather))sym("ncclAllGather");
     GetErrorString = (decltype(GetErrorString))sym("ncclGetErrorString");
   }
 };
@@ -231,6 +233,7 @@ struct b2_ctx {
   int pcg_graph_launches = 0;
   DBuf<int> pbc_dofs;
   bool has_pbc = false;
+  DBuf<int> q_gid;  // global id of every local pressure dof (b2_set_pressure_global_ids): the multi-rank algebraic set-up
   double vol = 0.0;  // sum of mQ over all ranks
   std::map<int, DVec> vecs;
   // Krylov work space
@@ -483,6 +486,41 @@ void allreduce_sum(b2_ctx* c, double* d, int n) {
   }
   B2_NCCL(g_nccl.AllReduce(d, d, (size_t)n, ncclDouble, ncclSum, c->comm, c->stream));
   c->stats.allreduces++;
+}
+
+// k int64 values of every rank, in rank order (set-up only)
+std::vector<int64_t> allgather_i64(b2_ctx* c, const int64_t* mine, int k) {
+  std::vector<int64_t> out(mine, mine + k);
+  if (c->nranks == 1) return out;
+  DBuf<int64_t> d;
+  d.alloc((int64_t)k * (c->nranks + 1));
+  out.resize((size_t)k * c->nranks);
+  B2_CUDA(cudaMemcpyAsync(d.p, mine, sizeof(int64_t) * k, cudaMemcpyHostToDevice, c->stream));
+  B2_NCCL(g_nccl.AllGather(d.p, d.p + k, (size_t)k, ncclInt64, c->comm, c->stream));
+  B2_CUDA(cudaMemcpyAsync(out.data(), d.p + k, sizeof(int64_t) * k * c->nranks, cudaMemcpyDeviceToHost, c->stream));
+  B2_CUDA(cudaStreamSynchronize(c->stream));
+  return out;
+}
+
+// The blocks of every rank, counts[q] elements of `bytes` each, concatenated in rank order into `recv` on the device
+// (set-up only): grouped ncclSend/ncclRecv with every other rank, this rank's own block copied in place.
+void allgatherv(b2_ctx* c, const void* send, const std::vector<int64_t>& counts, void* recv, ncclDataType_t type, size_t bytes) {
+  const int me = c->rank;
+  int64_t off = 0;
+  for (int q = 0; q < me; ++q) off += counts[q];
+  if (counts[me] > 0)
+    B2_CUDA(cudaMemcpyAsync((char*)recv + off * bytes, send, counts[me] * bytes, cudaMemcpyDeviceToDevice, c->stream));
+  if (c->nranks > 1) {
+    B2_NCCL(g_nccl.GroupStart());
+    off = 0;
+    for (int q = 0; q < c->nranks; ++q) {
+      if (q != me && counts[me] > 0) B2_NCCL(g_nccl.Send(send, (size_t)counts[me], type, q, c->comm, c->stream));
+      if (q != me && counts[q] > 0) B2_NCCL(g_nccl.Recv((char*)recv + off * bytes, (size_t)counts[q], type, q, c->comm, c->stream));
+      off += counts[q];
+    }
+    B2_NCCL(g_nccl.GroupEnd());
+  }
+  B2_CUDA(cudaStreamSynchronize(c->stream));
 }
 
 // after a reducing Krylov kernel: (multi rank) all-reduce the raw totals and run the scalar update
@@ -830,7 +868,19 @@ void mg_level_finish(b2_ctx* c, MgLevel& L) {
   }
 }
 
-void amg_build(b2_ctx* c);
+// The range of level-1 dofs this rank's restriction writes nonzeros into (rows of R_1 that are not empty): what the
+// peer-memory sum of the partial restrictions pushes to the other ranks.
+void mg_set_restrict_range(b2_ctx* c, const int32_t* R_indptr, int n) {
+  c->mg_lo = n;
+  c->mg_hi = 0;
+  for (int r = 0; r < n; ++r)
+    if (R_indptr[r + 1] > R_indptr[r]) { c->mg_lo = std::min(c->mg_lo, r); c->mg_hi = std::max(c->mg_hi, r + 1); }
+  if (c->mg_hi <= c->mg_lo) c->mg_lo = c->mg_hi = 0;
+}
+
+void csr_values(b2_ctx* c, int mat, int comp, DBuf<double>& out, const CSR** pat_out);
+void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0);
+void amg_build_gathered(b2_ctx* c);
 
 // x_l <- V-cycle(b_l), zero initial guess.  Returns the buffer that holds the result.
 // first_done: x already holds omega D^-1 b; rz_fin >= 0 (level 0 only): fuse the PCG product r.z into the last post-sweep
@@ -1997,13 +2047,7 @@ int b2_pressure_mg_add_level(b2_ctx* c, int64_t n_nodes, const double* x, int64_
     };
     upload_csr(L.P, L.Pv, (int)fine_n, L.n, P_indptr, P_indices, P_vals);
     upload_csr(L.R, L.Rv, L.n, (int)fine_cols, R_indptr, R_indices, R_vals);
-    if (c->mg.size() == 1) {  // index range of this level that the local restriction writes nonzeros into
-      c->mg_lo = L.n;
-      c->mg_hi = 0;
-      for (int r = 0; r < L.n; ++r)
-        if (R_indptr[r + 1] > R_indptr[r]) { c->mg_lo = std::min(c->mg_lo, r); c->mg_hi = std::max(c->mg_hi, r + 1); }
-      if (c->mg_hi <= c->mg_lo) c->mg_lo = c->mg_hi = 0;
-    }
+    if (c->mg.size() == 1) mg_set_restrict_range(c, R_indptr, L.n);
     mg_level_finish(c, L);
     B2_CUDA(cudaStreamSynchronize(c->stream));
   });
@@ -2013,9 +2057,66 @@ int b2_pressure_amg_build(b2_ctx* c) {
   return guarded(c, [&] {
     B2_REQUIRE(c->preassembled, "b2_pressure_amg_build: call it after b2_preassemble");
     B2_REQUIRE(c->mg.empty(), "b2_pressure_amg_build: the context already has a multigrid hierarchy");
-    B2_REQUIRE(c->nranks == 1, "b2_pressure_amg_build: the algebraic multigrid runs on one rank only");
     B2_REQUIRE(!c->has_pbc, "b2_pressure_amg_build: the pressure has Dirichlet dofs (the coarse solve assumes the constant null space)");
-    amg_build(c);
+    B2_REQUIRE(c->nranks == 1 || c->q_gid.p != nullptr,
+               "b2_pressure_amg_build: several ranks need the global pressure dof ids first (b2_set_pressure_global_ids)");
+    if (c->q_gid.p != nullptr) {
+      amg_build_gathered(c);
+      return;
+    }
+    DBuf<double> vals;
+    const CSR* pat = nullptr;
+    csr_values(c, B2_MAT_AP, 0, vals, &pat);
+    amg_build(c, c->pat[B2_PAT_QQ], std::move(vals), c->dinvAp.p);
+  });
+}
+
+int b2_set_pressure_global_ids(b2_ctx* c, int64_t n, const int64_t* gids) {
+  return guarded(c, [&] {
+    const Space& Q = c->sp[B2_SPACE_Q];
+    const int64_t ng = Q.n_global, n_owned = Q.n_owned;
+    B2_REQUIRE(n == Q.n_local(), "b2_set_pressure_global_ids: one global index per local pressure dof, owned then ghost");
+    B2_REQUIRE(ng > 0 && ng <= (1ll << 31), "b2_set_pressure_global_ids: set the global sizes first (b2_set_global_sizes), below 2^31");
+    // local checks first, but every rank takes part in the exchange below before any of them fails
+    int64_t bad = 0;  // 1: an index outside [0, n_global), 2: an index listed twice
+    for (int64_t i = 0; i < n; ++i)
+      if (gids[i] < 0 || gids[i] >= ng) bad = 1;
+    if (!bad) {
+      std::vector<int64_t> s(gids, gids + n);
+      std::sort(s.begin(), s.end());
+      if (std::adjacent_find(s.begin(), s.end()) != s.end()) bad = 2;
+    }
+    const int64_t mine[2] = {n_owned, bad};
+    const std::vector<int64_t> all = allgather_i64(c, mine, 2);
+    std::vector<int64_t> counts(c->nranks);
+    int64_t total = 0;
+    for (int q = 0; q < c->nranks; ++q) {
+      B2_REQUIRE(all[2 * q + 1] == 0, "b2_set_pressure_global_ids: rank " + std::to_string(q) +
+                                          (all[2 * q + 1] == 1 ? " has a global index outside [0, n_global)"
+                                                               : " lists the same global index twice"));
+      counts[q] = all[2 * q];
+      total += counts[q];
+    }
+    B2_REQUIRE(total == ng, "b2_set_pressure_global_ids: the ranks own " + std::to_string(total) + " dofs, not n_global = " +
+                                std::to_string(ng));
+    std::vector<int32_t> ids(gids, gids + n);
+    c->q_gid.alloc(n);
+    B2_CUDA(cudaMemcpyAsync(c->q_gid.p, ids.data(), sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+    // the owned indices of all ranks cover 0 .. n_global-1 exactly once
+    DBuf<int> owned;
+    owned.alloc(ng);
+    allgatherv(c, c->q_gid.p, counts, owned.p, ncclInt32, sizeof(int));
+    std::vector<int32_t> h(ng);
+    B2_CUDA(cudaMemcpyAsync(h.data(), owned.p, sizeof(int) * ng, cudaMemcpyDeviceToHost, c->stream));
+    B2_CUDA(cudaStreamSynchronize(c->stream));
+    std::vector<char> seen(ng, 0);
+    for (int32_t g : h) {
+      if (seen[g]) {
+        c->q_gid.release();
+        throw B2Error(-1, "b2_set_pressure_global_ids: global index " + std::to_string(g) + " is owned twice");
+      }
+      seen[g] = 1;
+    }
   });
 }
 
@@ -2429,16 +2530,14 @@ int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, DBuf<int>& agg) {
   return nc;
 }
 
-// Smoothed-aggregation hierarchy from the assembled Ap, coarsened until a level is small enough for the exact dense
-// solve, the coarsening ratio drops below 2, or 15 coarse levels (the single-block sub-cycle's tables hold 16).
-void amg_build(b2_ctx* c) {
+// Smoothed-aggregation hierarchy of the fine operator A0 (CSR with sorted columns, its values in CSR order, its inverse
+// diagonal), coarsened until a level is small enough for the exact dense solve, the coarsening ratio drops below 2, or
+// 15 coarse levels (the single-block sub-cycle's tables hold 16).  One rank passes Ap itself; several ranks pass the
+// gathered global Ap (amg_build_gathered), so that every rank builds the same hierarchy.
+void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0) {
   c->cfg_version++;
-  const CSR& qq = c->pat[B2_PAT_QQ];
-  DBuf<double> vals;  // values of the current operator in CSR order
-  const CSR* pat = nullptr;
-  csr_values(c, B2_MAT_AP, 0, vals, &pat);
-  const CSR* A = &qq;
-  const double* dinv = c->dinvAp.p;
+  const CSR* A = &A0;
+  const double* dinv = dinv0;
   c->mg_rho0 = amg_spectral_radius(c, *A, vals.p, dinv);
   c->mg_omega0 = 4.0 / (3.0 * c->mg_rho0);
   double omega_p = c->mg_omega0;
@@ -2487,6 +2586,75 @@ void amg_build(b2_ctx* c) {
     if (nc <= c->mg_dense_max || 2 * (int64_t)nc > n) break;
   }
   B2_CUDA(cudaStreamSynchronize(c->stream));
+}
+
+// Several ranks: every rank expands its owned rows of Ap into (global row << 32 | global col, value) pairs, the pairs
+// of all ranks are gathered in rank order, and every rank builds the global Ap from them and the hierarchy from that.
+// Each entry comes from exactly one rank (b2_set_pressure_global_ids checked that the owned rows cover the global
+// range once), so nothing is summed and every rank holds the same matrix bit for bit.  Levels 2 and below stay global
+// and replicated; level 1 is then cut back to this rank's owned rows: P_1 keeps the rows of the owned dofs in local
+// order, R_1 = P_1^T has local columns (ghost columns empty), the aggregates are those of the owned dofs.
+void amg_build_gathered(b2_ctx* c) {
+  const CSR& qq = c->pat[B2_PAT_QQ];
+  const Space& Q = c->sp[B2_SPACE_Q];
+  const int n_owned = qq.n_rows, ng = (int)Q.n_global;
+  CSR A;
+  DBuf<double> av;
+  {
+    DBuf<double> vals;
+    const CSR* pat = nullptr;
+    csr_values(c, B2_MAT_AP, 0, vals, &pat);
+    DBuf<unsigned long long> mk, keys;
+    DBuf<double> mv, kv;
+    mk.alloc(qq.nnz);
+    mv.alloc(qq.nnz);
+    B2_LAUNCH(c, k_amg_global_pairs, blocks_for(n_owned, 256), 256, n_owned, qq.rowptr.p, qq.cols.p, vals.p, c->q_gid.p, mk.p, mv.p);
+    const std::vector<int64_t> counts = allgather_i64(c, &qq.nnz, 1);
+    int64_t total = 0;
+    for (int64_t k : counts) total += k;
+    keys.alloc(total);
+    kv.alloc(total);
+    allgatherv(c, mk.p, counts, keys.p, ncclUint64, sizeof(unsigned long long));
+    allgatherv(c, mv.p, counts, kv.p, ncclDouble, sizeof(double));
+    mk.release();
+    mv.release();
+    vals.release();
+    amg_pairs_to_csr(c, keys, kv, total, ng, ng, A, av);
+    B2_REQUIRE(A.nnz == total, "algebraic multigrid: two ranks contributed the same entry of Ap");
+  }
+  DBuf<double> dinv;
+  dinv.alloc(ng);
+  B2_LAUNCH(c, k_amg_inv_diag, blocks_for(ng, 256), 256, ng, A.rowptr.p, A.cols.p, av.p, dinv.p);
+  amg_build(c, A, std::move(av), dinv.p);
+  A = CSR();
+  dinv.release();
+
+  MgLevel& L = c->mg[0];
+  CSR P;
+  DBuf<double> pv;
+  DBuf<int> len, agg;
+  P.n_rows = n_owned;
+  P.n_cols = L.n;
+  P.rowptr.alloc(n_owned + 1);
+  len.alloc(n_owned + 1);
+  len.zero(c->stream);
+  B2_LAUNCH(c, k_amg_row_lengths, blocks_for(n_owned, 256), 256, n_owned, L.P.rowptr.p, c->q_gid.p, len.p);
+  exclusive_sum(c, len.p, P.rowptr.p, (int64_t)n_owned + 1);
+  P.nnz = read_scalar(c, P.rowptr.p + n_owned);
+  P.cols.alloc(P.nnz);
+  pv.alloc(P.nnz);
+  agg.alloc(n_owned);
+  B2_LAUNCH(c, k_amg_gather_rows, blocks_for(n_owned, 256), 256, n_owned, L.P.rowptr.p, L.P.cols.p, L.Pv.p, L.agg.p, c->q_gid.p,
+            P.rowptr.p, P.cols.p, pv.p, agg.p);
+  L.P = std::move(P);
+  L.Pv = std::move(pv);
+  L.agg = std::move(agg);
+  amg_transpose(c, L.P, L.Pv.p, L.R, L.Rv);
+  L.R.n_cols = (int)Q.n_local();
+  std::vector<int32_t> rp(L.n + 1);
+  B2_CUDA(cudaMemcpyAsync(rp.data(), L.R.rowptr.p, sizeof(int) * (L.n + 1), cudaMemcpyDeviceToHost, c->stream));
+  B2_CUDA(cudaStreamSynchronize(c->stream));
+  mg_set_restrict_range(c, rp.data(), L.n);
 }
 
 }  // namespace

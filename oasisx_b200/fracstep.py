@@ -239,7 +239,8 @@ class FractionalStep_AB_CN:
             self._solver_p.updateOptions({"ksp_type": "preonly", "pc_type": "lu"})
 
         # optional multigrid for the pressure: "mg" takes the geometric hierarchy of a provider box; "gamg" / "hypre"
-        # take it too where it exists and otherwise, on one rank, the algebraic hierarchy built from Ap
+        # take it too where it exists and otherwise the algebraic hierarchy built from Ap (several ranks: from the
+        # global Ap gathered by global dof index)
         self._mg_levels = 0
         self._mg_kind = None  # "geometric" | "algebraic" | None
         pc_p = (solver_options.get("pressure") or {}).get("pc_type")
@@ -256,8 +257,9 @@ class FractionalStep_AB_CN:
             self._mg_levels = _mg.attach_pressure_multigrid(ctx, mesh, dof_nodes, self._nQ_owned, **mg_config)
             if self._mg_levels:
                 self._mg_kind = "geometric"
-            elif pc_p != "mg" and self._nranks == 1:
-                self._mg_levels = _mg.attach_pressure_amg(ctx, **mg_config)
+            elif pc_p != "mg":
+                gids = self._lp.Q.l2g if self._nranks > 1 else None
+                self._mg_levels = _mg.attach_pressure_amg(ctx, gids, **mg_config)
                 self._mg_kind = "algebraic" if self._mg_levels else None
             if self._mg_levels == 0:
                 logger.warning("pc_type=mg requested but the mesh carries no nested hierarchy: using Jacobi")

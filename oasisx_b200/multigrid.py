@@ -11,7 +11,7 @@ For meshes that come from DOLFINx the same C entry point accepts any nested hier
 ``dolfinx.mesh.refine`` [ext]) as long as P/R are supplied.
 
 Meshes without such a hierarchy get a smoothed-aggregation algebraic multigrid built on the device from the assembled
-pressure matrix instead (:func:`attach_pressure_amg`); the V-cycle is the same.
+pressure matrix instead (:func:`attach_pressure_amg`), on one rank or several; the V-cycle is the same.
 """
 from __future__ import annotations
 
@@ -112,11 +112,16 @@ def attach_pressure_multigrid(ctx, msh, dof_nodes: np.ndarray, n_owned: int, **c
     return len(levels)
 
 
-def attach_pressure_amg(ctx, **config) -> int:
+def attach_pressure_amg(ctx, global_ids: np.ndarray | None = None, **config) -> int:
     """Build the smoothed-aggregation hierarchy of the assembled pressure matrix on the device
-    (``b2_pressure_amg_build``: one rank, no pressure Dirichlet dofs) and apply `config` as
-    :func:`attach_pressure_multigrid` does (its ``omega`` only damps geometric levels).  Returns the number of coarse
-    levels."""
+    (``b2_pressure_amg_build``, no pressure Dirichlet dofs) and apply `config` as :func:`attach_pressure_multigrid` does
+    (its ``omega`` only damps geometric levels).  Returns the number of coarse levels.
+
+    On several ranks `global_ids` is the global index of every local pressure dof (``LocalSpace.l2g``), and every rank
+    must call this: the owned rows of all ranks are gathered into the global matrix, every rank builds the same
+    hierarchy from it, and level 1 keeps this rank's owned rows, as the geometric path does."""
+    if global_ids is not None:
+        ctx.set_pressure_global_ids(global_ids)
     ctx.pressure_amg_build()
     if config:
         ctx.pressure_mg_configure(**config)
