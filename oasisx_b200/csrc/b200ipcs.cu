@@ -894,7 +894,10 @@ double* mg_vcycle(b2_ctx* c, int l, const double* b, double* x, double* tmp, boo
     B2_LAUNCH(c, k_dense_matvec, blocks_for((int64_t)M.n * 32, 256), 256, M.n, c->mg_dense.p, b, x);
     return x;
   }
-  if (l >= c->mg_small_from) {
+  // the sub-cycle smooths every level down to the coarsest: it must not start at or above the exactly solved level
+  // (a geometric level of 5000 < n <= 8192 dofs can come right before it)
+  const bool above_dense = c->mg_dense_on && l - 1 <= c->mg_dense_level;
+  if (l >= c->mg_small_from && !above_dense) {
     // the rest of the hierarchy in one single-block kernel; b is c->mg[l-1].b by construction
     B2_LAUNCH(c, k_mg_small_cycle, 1, 1024, c->mg_dev.p, l - 1, (int)c->mg.size() - 1, c->mg_pre, c->mg_post, c->mg_coarse,
               c->mg_omega, c->d_mg_result);

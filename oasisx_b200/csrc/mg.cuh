@@ -318,11 +318,12 @@ k_cgz_rz(int64_t n, const double* __restrict__ r, const double* __restrict__ z, 
   cgz_reduce_finish<1>(s, partials, counter, fin, st, red_out);
 }
 
-// p = z + beta p
+// p = z + beta p; the first direction (beta = 0) is p = z and does not read p, which holds whatever the previous solve
+// left there (a NaN of a failed solve would survive 0 * p)
 __global__ void k_cgz_p(int64_t n, const double* __restrict__ z, double* __restrict__ p, const KryState* st) {
   const double beta = st->beta[0];
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    p[i] = fma(beta, p[i], z[i]);
+    p[i] = beta == 0.0 ? z[i] : fma(beta, p[i], z[i]);
 }
 
 // x += alpha p ; r -= alpha q ; sum rr

@@ -208,8 +208,9 @@ def make_oracle(msh, deg_u, tg: TaylorGreen, dt, **kw):
     return o
 
 
-def make_solver(msh, deg_u, tg: TaylorGreen, dt, solver_options=None, low_memory=False, **kw):
-    """The set-up of ``demo/taylor_green.py:135-182`` against oasisx_b200."""
+def make_solver(msh, deg_u, tg: TaylorGreen, dt, solver_options=None, low_memory=False, options=None, **kw):
+    """The set-up of ``demo/taylor_green.py:135-182`` against oasisx_b200; `options` adds to the solver's options
+    (e.g. ``{"multigrid": {...}}``)."""
     import oasisx_b200 as oasisx
 
     d = msh.geometry.dim
@@ -221,7 +222,7 @@ def make_solver(msh, deg_u, tg: TaylorGreen, dt, solver_options=None, low_memory
         lu = {"ksp_type": "preonly", "pc_type": "lu"}
         solver_options = {"tentative": lu, "pressure": lu, "scalar": lu}
     s = oasisx.FractionalStep_AB_CN(msh, ("Lagrange", deg_u), ("Lagrange", 1), bcs_u=bcs_u, bcs_p=[],
-                                    solver_options=solver_options, options={"low_memory_version": low_memory}, **kw)
+                                    solver_options=solver_options, options={"low_memory_version": low_memory, **(options or {})}, **kw)
     tg.t_u = -dt
     for i, f in enumerate(tg.components):
         s._u2[i].interpolate(f)
