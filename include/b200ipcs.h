@@ -198,11 +198,13 @@ int b2_pressure_mg_configure(b2_ctx* ctx, int nu_pre, int nu_post, int coarse_sw
  * MIS(2) of that graph with hash keys (Bell, Dalton and Olson 2012).  P = (I - 4/(3 rho) D^-1 A) T with T the
  * aggregate indicator, R = P^T, A_c = R A P, repeated until a level has at most 5000 dofs (solved exactly), the
  * coarsening ratio drops below 2, or 15 coarse levels; rho = 20 power iterations on D^-1 A.  Deterministic: the same
- * Ap gives the same hierarchy bit for bit.  Call after b2_preassemble on a context without multigrid levels and
- * without pressure Dirichlet dofs (the coarse solve relies on the constant null space); otherwise an error.
+ * Ap gives the same hierarchy bit for bit.  Call after b2_preassemble on a context without multigrid levels;
+ * otherwise an error.  Pressure Dirichlet dofs (b2_set_pressure_bc_dofs) join no aggregate: their rows of P_1 are
+ * zero, A_1 is the Galerkin operator of the interior block, and the exact coarse solve takes no null-space shift.  A
+ * Dirichlet row of Ap with a nonzero off-diagonal entry fails the build.
  * Several ranks (collective; b2_set_pressure_global_ids first; one rank takes the same path once it has been given
- * global ids, numbering the hierarchy by them): the owned rows of Ap of all ranks are gathered over
- * NCCL into the global matrix, and every rank builds the same hierarchy from it.  Levels 2 and below are global and
+ * global ids, numbering the hierarchy by them): the owned rows of Ap and their Dirichlet flags of all ranks are
+ * gathered over NCCL into the global matrix and mask, and every rank builds the same hierarchy from them.  Levels 2 and below are global and
  * replicated; level 1 keeps this rank's part only: P_1 the rows of its owned dofs (local order), R_1 = P_1^T with
  * local columns (ghost columns empty), the aggregates of its owned dofs.  Set-up memory on every GPU: the global
  * matrix and its sort buffers (DESIGN.md section 2). */

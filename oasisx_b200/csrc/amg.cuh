@@ -1,5 +1,6 @@
 // amg.cuh -- kernels of the smoothed-aggregation algebraic multigrid set-up (b2_pressure_amg_build): strength graph,
-// MIS(2) aggregation (Bell, Dalton and Olson 2012), power iteration for rho(D^-1 A), and the expand-sort-reduce sparse
+// MIS(2) aggregation (Bell, Dalton and Olson 2012) that keeps the pressure Dirichlet dofs out of every aggregate, power
+// iteration for rho(D^-1 A), and the expand-sort-reduce sparse
 // products behind P = (I - omega D^-1 A) T, R = P^T and A_c = R (A P), and on several ranks the gather of the global
 // fine matrix and the cut of level 1 back to each rank's owned rows.  Every step is deterministic: no floating-point
 // atomics, sums are taken sequentially in an order fixed by a stable sort, and the reductions of the power iteration
@@ -27,9 +28,20 @@ __device__ __forceinline__ unsigned long long amg_key(int i) {
 // j is a strong neighbour of i when j != i and a_ij != 0 (threshold 0)
 __device__ __forceinline__ bool amg_strong(int i, int j, double a) { return j != i && a != 0.0; }
 
-__global__ void k_amg_init(int n, int* __restrict__ state) {
+// excl (nullptr: none): nodes kept out of every aggregate (pressure Dirichlet dofs of the fine level); they start out
+// of the MIS and are never roots
+__global__ void k_amg_init(int n, const uint8_t* __restrict__ excl, int* __restrict__ state) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) state[i] = AMG_UNDECIDED;
+  if (i < n) state[i] = excl != nullptr && excl[i] ? AMG_OUT : AMG_UNDECIDED;
+}
+
+// an excluded row must be isolated in the strength graph (no nonzero off-diagonal entry): *err = 1 otherwise
+__global__ void k_amg_check_excluded(int n, const int* __restrict__ rp, const int* __restrict__ ci, const double* __restrict__ va,
+                                     const uint8_t* __restrict__ excl, int* __restrict__ err) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n || !excl[i]) return;
+  for (int p = rp[i]; p < rp[i + 1]; ++p)
+    if (amg_strong(i, ci[p], va[p])) atomicOr(err, 1);
 }
 
 // t[i] = (state_i, key_i): the MIS(2) tuple, state in the top two bits
@@ -86,13 +98,14 @@ __global__ void k_amg_pass1(int n, const int* __restrict__ rp, const int* __rest
 }
 
 // pass 2: a node left over joins the aggregate of its pass-1 neighbour with the largest key; MIS(2) maximality
-// guarantees one exists -- a node without one sets *err
+// guarantees one exists -- a node without one sets *err.  An excluded node keeps -1.
 __global__ void k_amg_pass2(int n, const int* __restrict__ rp, const int* __restrict__ ci, const double* __restrict__ va,
-                            const int* __restrict__ agg1, int* __restrict__ agg, int* __restrict__ err) {
+                            const uint8_t* __restrict__ excl, const int* __restrict__ agg1, int* __restrict__ agg,
+                            int* __restrict__ err) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   int a = agg1[i];
-  if (a < 0) {
+  if (a < 0 && !(excl != nullptr && excl[i])) {
     unsigned long long best = 0;
     for (int p = rp[i]; p < rp[i + 1]; ++p) {
       const int j = ci[p];
@@ -163,13 +176,20 @@ __global__ void k_amg_smoother(int n, const int* __restrict__ rp, const int* __r
   for (int p = rp[i]; p < rp[i + 1]; ++p) s[p] = (ci[p] == i ? 1.0 : 0.0) - w * va[p];
 }
 
-// tentative prolongator T[i, agg(i)] = 1 as CSR
-__global__ void k_amg_tentative(int n, const int* __restrict__ agg, int* __restrict__ rp, int* __restrict__ ci,
+// flag[i] = 1 where node i has an aggregate: the row lengths of T, whose exclusive scan is T's row pointer (rp[i] = i
+// when no node is excluded)
+__global__ void k_amg_kept_flags(int n, const int* __restrict__ agg, int* __restrict__ flag) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) flag[i] = agg[i] >= 0;
+}
+
+// tentative prolongator T[i, agg(i)] = 1 as CSR; the row of an excluded node (agg -1) is empty
+__global__ void k_amg_tentative(int n, const int* __restrict__ agg, const int* __restrict__ rp, int* __restrict__ ci,
                                 double* __restrict__ va) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i > n) return;
-  rp[i] = i;
-  if (i < n) { ci[i] = agg[i]; va[i] = 1.0; }
+  if (i >= n || agg[i] < 0) return;
+  ci[rp[i]] = agg[i];
+  va[rp[i]] = 1.0;
 }
 
 // row index of every stored entry of a CSR matrix
@@ -230,6 +250,19 @@ __global__ void k_amg_global_pairs(int n, const int* __restrict__ rp, const int*
     keys[p] = r | (unsigned)gid[ci[p]];
     vals[p] = va[p];
   }
+}
+
+// mask[gid] = flag of an owned row, from the gathered (global id << 8 | flag) of every rank
+__global__ void k_amg_scatter_mask(int64_t n, const unsigned long long* __restrict__ keys, uint8_t* __restrict__ mask) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n) mask[keys[t] >> 8] = (uint8_t)(keys[t] & 0xff);
+}
+
+// (global id << 8 | flag) of this rank's owned rows
+__global__ void k_amg_flag_keys(int n, const int* __restrict__ gid, const uint8_t* __restrict__ flag,
+                                unsigned long long* __restrict__ keys) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) keys[i] = ((unsigned long long)(unsigned)gid[i] << 8) | (flag[i] ? 1u : 0u);
 }
 
 // dinv_i = 1 / a_ii of a CSR matrix (every row of the gathered Ap holds its diagonal)

@@ -833,7 +833,8 @@ void mg_build_descriptors(b2_ctx* c) {
 }
 
 // dense inverse of (A_l + alpha e e^T) for coarse level index i (mg.cuh); alpha = A_00 / n keeps the shift at the
-// scale of the operator
+// scale of the operator.  An algebraic level of a pressure with Dirichlet dofs is the Galerkin operator of the interior
+// block, nonsingular: alpha = 0, or the "exact" solve would not be exact.
 void mg_build_dense(b2_ctx* c, int i) {
   MgLevel& M = c->mg[i];
   const int n = M.n;
@@ -844,7 +845,7 @@ void mg_build_dense(b2_ctx* c, int i) {
   double dinv0 = 0.0;
   B2_CUDA(cudaMemcpyAsync(&dinv0, M.dinv.p, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
   B2_CUDA(cudaStreamSynchronize(c->stream));
-  const double alpha = 1.0 / (dinv0 * n);
+  const double alpha = c->has_pbc && M.algebraic ? 0.0 : 1.0 / (dinv0 * n);
   B2_LAUNCH(c, k_dense_from_sell, n, 128, n, M.pat.slice_ptr.p, M.pat.scols.p, M.A.p, alpha, c->mg_dense.p);
   const dim3 grid((unsigned)blocks_for(n, 256), (unsigned)n);
   for (int k = 0; k < n; ++k) {
@@ -879,7 +880,7 @@ void mg_set_restrict_range(b2_ctx* c, const int32_t* R_indptr, int n) {
 }
 
 void csr_values(b2_ctx* c, int mat, int comp, DBuf<double>& out, const CSR** pat_out);
-void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0);
+void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0, const uint8_t* excl0);
 void amg_build_gathered(b2_ctx* c);
 
 // x_l <- V-cycle(b_l), zero initial guess.  Returns the buffer that holds the result.
@@ -948,6 +949,10 @@ double* mg_vcycle(b2_ctx* c, int l, const double* b, double* x, double* tmp, boo
   if (rz_done != nullptr) *rz_done = fuse_rz;
   return x;
 }
+
+// the pressure solve may take the V-cycle: a hierarchy exists, and with pressure Dirichlet dofs it is the algebraic one,
+// which keeps them out (geometric coarse levels are Neumann operators of the coarse meshes)
+bool mg_usable(const b2_ctx* c) { return !c->mg.empty() && (!c->has_pbc || c->mg[0].algebraic); }
 
 void cgz_finish(b2_ctx* c, int fin, int n) {
   if (c->nranks == 1 || c->peer_on) return;
@@ -1424,7 +1429,7 @@ void stage_pressure_solve(b2_ctx* c, double nu, int32_t* reason) {
     if (c->dp_hist >= 2) B2_CUDA(cudaMemcpyAsync(dp, t3, sizeof(double) * nq, cudaMemcpyDeviceToDevice, c->stream));
     c->dp_hist++;
   }
-  if (c->ksp[B2_SOLVER_PRESSURE].pc == 2 && !c->mg.empty() && !c->has_pbc)
+  if (c->ksp[B2_SOLVER_PRESSURE].pc == 2 && mg_usable(c))
     pcg_mg_solve(c, b2, dp, reason, &its);
   else
     krylov_solve(c, B2_SOLVER_PRESSURE, c->pat[B2_PAT_QQ], c->Ap.p, c->dinvAp.p, B2_SPACE_Q, 1, b2, dp, reason, &its);  // :578
@@ -2060,7 +2065,6 @@ int b2_pressure_amg_build(b2_ctx* c) {
   return guarded(c, [&] {
     B2_REQUIRE(c->preassembled, "b2_pressure_amg_build: call it after b2_preassemble");
     B2_REQUIRE(c->mg.empty(), "b2_pressure_amg_build: the context already has a multigrid hierarchy");
-    B2_REQUIRE(!c->has_pbc, "b2_pressure_amg_build: the pressure has Dirichlet dofs (the coarse solve assumes the constant null space)");
     B2_REQUIRE(c->nranks == 1 || c->q_gid.p != nullptr,
                "b2_pressure_amg_build: several ranks need the global pressure dof ids first (b2_set_pressure_global_ids)");
     if (c->q_gid.p != nullptr) {
@@ -2070,7 +2074,7 @@ int b2_pressure_amg_build(b2_ctx* c) {
     DBuf<double> vals;
     const CSR* pat = nullptr;
     csr_values(c, B2_MAT_AP, 0, vals, &pat);
-    amg_build(c, c->pat[B2_PAT_QQ], std::move(vals), c->dinvAp.p);
+    amg_build(c, c->pat[B2_PAT_QQ], std::move(vals), c->dinvAp.p, c->is_bc_q.p);
   });
 }
 
@@ -2496,8 +2500,9 @@ double amg_spectral_radius(b2_ctx* c, const CSR& A, const double* va, const doub
   return h[1] / h[2];
 }
 
-// MIS(2) aggregation of the strength graph of A; returns the number of aggregates
-int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, DBuf<int>& agg) {
+// MIS(2) aggregation of the strength graph of A; returns the number of aggregates.  excl (nullptr: none): nodes kept
+// out of every aggregate, agg = -1
+int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, const uint8_t* excl, DBuf<int>& agg) {
   const int n = A.n_rows;
   B2_REQUIRE(n < (1 << 30), "algebraic multigrid: at most 2^30 dofs");
   const int g = blocks_for(n, 256);
@@ -2508,7 +2513,7 @@ int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, DBuf<int>& agg) {
   t0.alloc(n);
   m1.alloc(n);
   m2.alloc(n);
-  B2_LAUNCH(c, k_amg_init, g, 256, n, state.p);
+  B2_LAUNCH(c, k_amg_init, g, 256, n, excl, state.p);
   for (int round = 0;; ++round) {
     B2_REQUIRE(round <= n, "algebraic multigrid: MIS(2) did not terminate");
     cnt.zero(c->stream);
@@ -2528,7 +2533,7 @@ int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, DBuf<int>& agg) {
   agg.alloc(n);
   cnt.zero(c->stream);
   B2_LAUNCH(c, k_amg_pass1, g, 256, n, A.rowptr.p, A.cols.p, va, state.p, id.p, agg1.p);
-  B2_LAUNCH(c, k_amg_pass2, g, 256, n, A.rowptr.p, A.cols.p, va, agg1.p, agg.p, cnt.p);
+  B2_LAUNCH(c, k_amg_pass2, g, 256, n, A.rowptr.p, A.cols.p, va, excl, agg1.p, agg.p, cnt.p);
   B2_REQUIRE(read_scalar(c, cnt.p) == 0, "algebraic multigrid: a node was left without an aggregate");
   return nc;
 }
@@ -2537,10 +2542,23 @@ int amg_aggregate(b2_ctx* c, const CSR& A, const double* va, DBuf<int>& agg) {
 // diagonal), coarsened until a level is small enough for the exact dense solve, the coarsening ratio drops below 2, or
 // 15 coarse levels (the single-block sub-cycle's tables hold 16).  One rank passes Ap itself; several ranks pass the
 // gathered global Ap (amg_build_gathered), so that every rank builds the same hierarchy.
-void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0) {
+// excl0 flags the pressure Dirichlet dofs of A0 (identity rows, zeroed columns).  They join no aggregate: T has an
+// empty row there, so P = (I - omega D^-1 A0) T is zero on those rows, R = P^T zero on those columns, and A_1 = R A0 P
+// is the Galerkin operator of the interior block, SPD without a null space.  Coarse levels exclude nothing.  An
+// all-zero mask gives the hierarchy of no mask bit for bit.
+void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0, const uint8_t* excl0) {
   c->cfg_version++;
   const CSR* A = &A0;
   const double* dinv = dinv0;
+  const uint8_t* excl = excl0;
+  {
+    DBuf<int> err;
+    err.alloc(1);
+    err.zero(c->stream);
+    B2_LAUNCH(c, k_amg_check_excluded, blocks_for(A0.n_rows, 256), 256, A0.n_rows, A0.rowptr.p, A0.cols.p, vals.p, excl0, err.p);
+    B2_REQUIRE(read_scalar(c, err.p) == 0,
+               "algebraic multigrid: a pressure Dirichlet row of Ap has a nonzero off-diagonal entry");
+  }
   c->mg_rho0 = amg_spectral_radius(c, *A, vals.p, dinv);
   c->mg_omega0 = 4.0 / (3.0 * c->mg_rho0);
   double omega_p = c->mg_omega0;
@@ -2548,18 +2566,23 @@ void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0)
   while (c->mg.size() < 15) {
     const int n = A->n_rows;
     DBuf<int> agg;
-    const int nc = amg_aggregate(c, *A, vals.p, agg);
-    if (nc >= n) break;  // no coarsening at all
+    const int nc = amg_aggregate(c, *A, vals.p, excl, agg);
+    if (nc == 0 || nc >= n) break;  // every dof excluded, or no coarsening at all
     // P = (I - omega_P D^-1 A) T
     CSR T;
     DBuf<double> tv, sv;
+    DBuf<int> kept;
     T.n_rows = n;
     T.n_cols = nc;
-    T.nnz = n;
     T.rowptr.alloc(n + 1);
-    T.cols.alloc(n);
-    tv.alloc(n);
-    B2_LAUNCH(c, k_amg_tentative, blocks_for(n + 1, 256), 256, n, agg.p, T.rowptr.p, T.cols.p, tv.p);
+    kept.alloc(n + 1);
+    kept.zero(c->stream);
+    B2_LAUNCH(c, k_amg_kept_flags, blocks_for(n, 256), 256, n, agg.p, kept.p);
+    exclusive_sum(c, kept.p, T.rowptr.p, (int64_t)n + 1);
+    T.nnz = read_scalar(c, T.rowptr.p + n);
+    T.cols.alloc(T.nnz);
+    tv.alloc(T.nnz);
+    B2_LAUNCH(c, k_amg_tentative, blocks_for(n, 256), 256, n, agg.p, T.rowptr.p, T.cols.p, tv.p);
     sv.alloc(A->nnz);
     B2_LAUNCH(c, k_amg_smoother, blocks_for(n, 256), 256, n, A->rowptr.p, A->cols.p, vals.p, dinv, omega_p, sv.p);
     c->mg.emplace_back();
@@ -2586,6 +2609,7 @@ void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0)
     vals = std::move(acv);
     A = &L.pat;
     dinv = L.dinv.p;
+    excl = nullptr;
     if (nc <= c->mg_dense_max || 2 * (int64_t)nc > n) break;
   }
   B2_CUDA(cudaStreamSynchronize(c->stream));
@@ -2594,15 +2618,18 @@ void amg_build(b2_ctx* c, const CSR& A0, DBuf<double> vals, const double* dinv0)
 // Several ranks: every rank expands its owned rows of Ap into (global row << 32 | global col, value) pairs, the pairs
 // of all ranks are gathered in rank order, and every rank builds the global Ap from them and the hierarchy from that.
 // Each entry comes from exactly one rank (b2_set_pressure_global_ids checked that the owned rows cover the global
-// range once), so nothing is summed and every rank holds the same matrix bit for bit.  Levels 2 and below stay global
-// and replicated; level 1 is then cut back to this rank's owned rows: P_1 keeps the rows of the owned dofs in local
-// order, R_1 = P_1^T has local columns (ghost columns empty), the aggregates are those of the owned dofs.
+// range once), so nothing is summed and every rank holds the same matrix bit for bit.  The pressure Dirichlet flags of
+// the owned rows are gathered the same way, as (global id << 8 | flag), into the global mask.  Levels 2 and below stay
+// global and replicated; level 1 is then cut back to this rank's owned rows: P_1 keeps the rows of the owned dofs in
+// local order, R_1 = P_1^T has local columns (ghost columns empty), the aggregates are those of the owned dofs (-1 on
+// a Dirichlet dof).
 void amg_build_gathered(b2_ctx* c) {
   const CSR& qq = c->pat[B2_PAT_QQ];
   const Space& Q = c->sp[B2_SPACE_Q];
   const int n_owned = qq.n_rows, ng = (int)Q.n_global;
   CSR A;
   DBuf<double> av;
+  DBuf<uint8_t> mask;
   {
     DBuf<double> vals;
     const CSR* pat = nullptr;
@@ -2624,13 +2651,22 @@ void amg_build_gathered(b2_ctx* c) {
     vals.release();
     amg_pairs_to_csr(c, keys, kv, total, ng, ng, A, av);
     B2_REQUIRE(A.nnz == total, "algebraic multigrid: two ranks contributed the same entry of Ap");
+    const int64_t mine = n_owned;
+    const std::vector<int64_t> owned = allgather_i64(c, &mine, 1);
+    mk.alloc(n_owned);
+    keys.alloc(ng);
+    B2_LAUNCH(c, k_amg_flag_keys, blocks_for(n_owned, 256), 256, n_owned, c->q_gid.p, c->is_bc_q.p, mk.p);
+    allgatherv(c, mk.p, owned, keys.p, ncclUint64, sizeof(unsigned long long));
+    mask.alloc(ng);
+    B2_LAUNCH(c, k_amg_scatter_mask, blocks_for(ng, 256), 256, (int64_t)ng, keys.p, mask.p);
   }
   DBuf<double> dinv;
   dinv.alloc(ng);
   B2_LAUNCH(c, k_amg_inv_diag, blocks_for(ng, 256), 256, ng, A.rowptr.p, A.cols.p, av.p, dinv.p);
-  amg_build(c, A, std::move(av), dinv.p);
+  amg_build(c, A, std::move(av), dinv.p, mask.p);
   A = CSR();
   dinv.release();
+  mask.release();
 
   MgLevel& L = c->mg[0];
   CSR P;
@@ -3035,7 +3071,7 @@ int b2_ksp_solve(b2_ctx* c, int solver, int mat, const double* b, double* x, int
     B2_LAUNCH(c, k_fill, pgrid(c, n), 256, n, 1.0, dinv.p);
     B2_LAUNCH(c, k_inv_diag, blocks_for(pat->n_rows, 256), 256, pat->n_rows, pat->slice_ptr.p, pat->diag_t.p, v->p, dinv.p);
     int32_t its = 0;
-    if (mat == B2_MAT_AP && c->ksp[solver].pc == 2 && !c->mg.empty() && !c->has_pbc && solver == B2_SOLVER_PRESSURE) {
+    if (mat == B2_MAT_AP && c->ksp[solver].pc == 2 && mg_usable(c) && solver == B2_SOLVER_PRESSURE) {
       B2_CUDA(cudaMemcpyAsync(c->vec(B2_VEC_B2), db.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, c->stream));
       B2_CUDA(cudaMemcpyAsync(c->vec(B2_VEC_DP), dx.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, c->stream));
       pcg_mg_solve(c, c->vec(B2_VEC_B2), c->vec(B2_VEC_DP), reason, &its);

@@ -173,7 +173,8 @@ k_mg_small_cycle(const MgDev* __restrict__ lv, int l0, int l_last, int pre, int 
 // ---- exact solve on the coarsest used level -------------------------------------------------------
 // A level with a few thousand unknowns is solved exactly by ONE dense mat-vec with the precomputed
 // inverse of (A_l + alpha e e^T) (A_l is the singular Neumann stiffness, e = ones; the shift makes it
-// SPD and leaves the action on mean-free right-hand sides unchanged).  2197^2 doubles = 39 MB read by
+// SPD and leaves the action on mean-free right-hand sides unchanged).  With pressure Dirichlet dofs the algebraic A_l
+// is already SPD and alpha = 0 (mg_build_dense).  2197^2 doubles = 39 MB read by
 // the whole machine (~10 us) replaces ~30 block-synchronised phases of the single-block sub-cycle
 // (~190 us), and the V-cycle stays a symmetric positive definite preconditioner.
 __global__ void k_dense_from_sell(int n, const int* __restrict__ slice_ptr, const int* __restrict__ cols,

@@ -240,21 +240,25 @@ class FractionalStep_AB_CN:
 
         # optional multigrid for the pressure: "mg" takes the geometric hierarchy of a provider box; "gamg" / "hypre"
         # take it too where it exists and otherwise the algebraic hierarchy built from Ap (several ranks: from the
-        # global Ap gathered by global dof index)
+        # global Ap gathered by global dof index).  With PressureBCs only the algebraic hierarchy applies: it keeps the
+        # Dirichlet dofs out of its aggregates, while the geometric coarse levels are Neumann operators.
         self._mg_levels = 0
         self._mg_kind = None  # "geometric" | "algebraic" | None
         pc_p = (solver_options.get("pressure") or {}).get("pc_type")
-        if pc_p in ("mg", "gamg", "hypre") and not self._bcs_p:
+        if pc_p == "mg" and self._bcs_p:
+            logger.warning("pc_type=mg requested but the geometric hierarchy does not handle PressureBCs: using Jacobi")
+        elif pc_p in ("mg", "gamg", "hypre"):
             from . import multigrid as _mg
 
-            dof_nodes = getattr(self._Q, "_dof_nodes", None)
-            if dof_nodes is None:  # P1: every local dof sits on the node its cells put it on
-                cell_nodes, cell_dofs = (self._lp.cell_nodes, self._lp.Q.cell_dofs) if self._lp is not None else (
-                    mesh.geometry.dofmap, self._Q.dofmap.list)
-                dof_nodes = np.empty(self._Q.num_dofs, dtype=np.int64)
-                dof_nodes[cell_dofs.ravel()] = cell_nodes.ravel()
             mg_config = options.get("multigrid") or {}
-            self._mg_levels = _mg.attach_pressure_multigrid(ctx, mesh, dof_nodes, self._nQ_owned, **mg_config)
+            if not self._bcs_p:
+                dof_nodes = getattr(self._Q, "_dof_nodes", None)
+                if dof_nodes is None:  # P1: every local dof sits on the node its cells put it on
+                    cell_nodes, cell_dofs = (self._lp.cell_nodes, self._lp.Q.cell_dofs) if self._lp is not None else (
+                        mesh.geometry.dofmap, self._Q.dofmap.list)
+                    dof_nodes = np.empty(self._Q.num_dofs, dtype=np.int64)
+                    dof_nodes[cell_dofs.ravel()] = cell_nodes.ravel()
+                self._mg_levels = _mg.attach_pressure_multigrid(ctx, mesh, dof_nodes, self._nQ_owned, **mg_config)
             if self._mg_levels:
                 self._mg_kind = "geometric"
             elif pc_p != "mg":

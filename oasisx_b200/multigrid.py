@@ -10,7 +10,8 @@ on the coarse mesh by the library (``b2_pressure_mg_add_level``).
 For meshes that come from DOLFINx the same C entry point accepts any nested hierarchy (e.g. from
 ``dolfinx.mesh.refine`` [ext]) as long as P/R are supplied.
 
-Meshes without such a hierarchy get a smoothed-aggregation algebraic multigrid built on the device from the assembled
+Meshes without such a hierarchy, and problems with PressureBCs (whose Dirichlet dofs the coarse meshes' Neumann
+operators here do not know), get a smoothed-aggregation algebraic multigrid built on the device from the assembled
 pressure matrix instead (:func:`attach_pressure_amg`), on one rank or several; the V-cycle is the same.
 """
 from __future__ import annotations
@@ -114,8 +115,9 @@ def attach_pressure_multigrid(ctx, msh, dof_nodes: np.ndarray, n_owned: int, **c
 
 def attach_pressure_amg(ctx, global_ids: np.ndarray | None = None, **config) -> int:
     """Build the smoothed-aggregation hierarchy of the assembled pressure matrix on the device
-    (``b2_pressure_amg_build``, no pressure Dirichlet dofs) and apply `config` as :func:`attach_pressure_multigrid` does
-    (its ``omega`` only damps geometric levels).  Returns the number of coarse levels.
+    (``b2_pressure_amg_build``) and apply `config` as :func:`attach_pressure_multigrid` does (its ``omega`` only damps
+    geometric levels).  Returns the number of coarse levels.  Pressure Dirichlet dofs join no aggregate: the rows of P
+    are zero there and the coarsest level is solved exactly without the null-space shift.
 
     On several ranks `global_ids` is the global index of every local pressure dof (``LocalSpace.l2g``), and every rank
     must call this: the owned rows of all ranks are gathered into the global matrix, every rank builds the same

@@ -1,12 +1,14 @@
 #!/usr/bin/env python3
 """Pressure solve with the smoothed-aggregation multigrid against Jacobi-PCG and the geometric multigrid.
 
-    python tools/bench_amg.py [--sizes 32 64 96] [--steps 20] [--warmup 3] [--box 96] [--out FILE]
+    python tools/bench_amg.py [--sizes 32 64 96] [--steps 20] [--warmup 3] [--box 96] [--channel 64 96] [--out FILE]
     python -m torch.distributed.run --nproc-per-node=G tools/bench_amg.py --sizes 64 --box 0 [...]   (G ranks)
 
 One JSON line per case, 3D Taylor-Green P2-P1 with the benchmark's solver settings (bench.KRYLOV):
   jittered N^3 meshes (no geometric hierarchy), pressure on the algebraic hierarchy ("gamg") and on Jacobi;
-  the N^3 provider box with the algebraic hierarchy forced through the Context API against the geometric one.
+  the N^3 provider box with the algebraic hierarchy forced through the Context API against the geometric one;
+  --channel: the open channel (inlet, no-slip walls, PressureBC outlet; tests/channel_problem.py) on the N^3 provider
+  box and the jittered N^3 mesh, the algebraic hierarchy (its Dirichlet dofs excluded) against Jacobi.
 The algebraic hierarchy is built on a solver set up with Jacobi (b2_pressure_amg_build, host clock around it ending
 in a device synchronise), then the pressure slot is switched to it.  Reported: set-up time, levels (n, nnz), operator
 complexity sum nnz(A_l) / nnz(A_0), mean pressure iterations and stage_ms.pressure over the timed steps, steps/s from
@@ -36,6 +38,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench  # noqa: E402
 from oasisx_b200 import mesh as bmesh  # noqa: E402
 from oasisx_b200.comm import HostComm  # noqa: E402
+from channel_problem import channel  # noqa: E402
 from problems import TaylorGreen, jittered_mesh, make_mesh, make_solver  # noqa: E402
 
 COMM = HostComm.from_env()
@@ -48,8 +51,9 @@ def card() -> dict:
     return {"gpu": name, "power_limit": power}
 
 
-def run_case(msh, label: str, pc: str, steps: int, warmup: int) -> dict:
-    """pc: 'jacobi', 'mg' (geometric), or 'amg' (algebraic, built through the Context API)."""
+def run_case(msh, label: str, pc: str, steps: int, warmup: int, flow: str = "taylor_green") -> dict:
+    """pc: 'jacobi', 'mg' (geometric), or 'amg' (algebraic, built through the Context API).  flow: 'taylor_green' or
+    'channel'."""
     dt, nu = bench.DT, bench.NU
     comm = COMM
     if comm.size > 1:
@@ -58,13 +62,19 @@ def run_case(msh, label: str, pc: str, steps: int, warmup: int) -> dict:
     opts = copy.deepcopy(bench.KRYLOV)
     opts["pressure"]["pc_type"] = "mg" if pc == "mg" else "jacobi"
     t0 = time.perf_counter()
-    s = make_solver(msh, 2, tg, dt, solver_options=opts, device=int(os.environ.get("LOCAL_RANK", "0")))
+    device = int(os.environ.get("LOCAL_RANK", "0"))
+    if flow == "channel":
+        # outlet pressure 0: with the reference test's 4.0 the flow enters through the outlet and the step diverges at
+        # the benchmark's viscosity within one step, with Jacobi as with the multigrid (B200, 64^3)
+        s, _, inlet = channel(msh, deg=2, solver_options=opts, device=device, p_out=0.0)
+    else:
+        s = make_solver(msh, 2, tg, dt, solver_options=opts, device=device)
     ctx = s._ctx
     ctx.synchronize()
     t_solver = comm.allreduce(time.perf_counter() - t0, "max")
     lp = s._lp
     dofs = 3 * s._Vi[0][0].num_dofs + s._Q.num_dofs if lp is None else 3 * lp.V.n_global + lp.Q.n_global
-    rec = {"case": label, "pc": pc, "ranks": comm.size, "dofs": dofs, "solver_setup_s": round(t_solver, 3)}
+    rec = {"case": label, "flow": flow, "pc": pc, "ranks": comm.size, "dofs": dofs, "solver_setup_s": round(t_solver, 3)}
     if pc == "amg":
         comm.Barrier()
         ctx.synchronize()
@@ -91,18 +101,22 @@ def run_case(msh, label: str, pc: str, steps: int, warmup: int) -> dict:
         rec["levels"] = levels
         rec["operator_complexity"] = round(sum(v["nnz_A"] for v in levels) / levels[0]["nnz_A"], 4)
     tg.t_u, tg.t_p = 0.0, -dt / 2
-    for _ in range(warmup):
+
+    def advance():
         tg.t_u += dt
         tg.t_p += dt
+        if flow == "channel":
+            inlet.t += dt
         s.solve(dt, nu, max_iter=1)
+
+    for _ in range(warmup):
+        advance()
     ctx.synchronize()
     comm.Barrier()
     ctx.event_record(0)
     its, ms_p = [], []
     for _ in range(steps):
-        tg.t_u += dt
-        tg.t_p += dt
-        s.solve(dt, nu, max_iter=1)
+        advance()
         st = ctx.stats()
         its.append(st.its_pressure)
         ms_p.append(st.ms_pressure)
@@ -126,6 +140,8 @@ def main():
     ap.add_argument("--box", type=int, default=96, help="provider box for geometric vs algebraic (0: skip)")
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--channel", type=int, nargs="*", default=[],
+                    help="open channel with a PressureBC outlet on the N^3 provider box and jittered mesh")
     ap.add_argument("--out", default=None, help="append the JSON lines to this file too")
     args = ap.parse_args()
     info = card() if COMM.rank == 0 else {}
@@ -136,8 +152,15 @@ def main():
     if args.box:
         msh = make_mesh(3, args.box)
         cases += [(msh, f"box{args.box}", pc) for pc in ("amg", "mg")]
-    for msh, label, pc in cases:
-        rec = dict(info, **run_case(msh, label, pc, args.steps, args.warmup))
+    cases = [c + ("taylor_green",) for c in cases]
+    for N in args.channel:
+        for kind, msh in (("box", make_mesh(3, N)), ("jittered", jittered_mesh(3, N, seed=1))):
+            cases += [(msh, f"channel_{kind}{N}", pc, "channel") for pc in ("amg", "jacobi")]
+    for msh, label, pc, flow in cases:
+        try:
+            rec = dict(info, **run_case(msh, label, pc, args.steps, args.warmup, flow))
+        except Exception as e:  # a case that fails is reported as such, and the others still run
+            rec = dict(info, case=label, flow=flow, pc=pc, ranks=COMM.size, error=str(e))
         if COMM.rank != 0:
             continue
         line = json.dumps(rec)
