@@ -700,16 +700,20 @@ void gmres_solve(b2_ctx* c, const KSPOpts& o, const CSR& pat, const double* vals
 
 // Solves K systems  A x_k = b_k  (interleaved storage) with the options of solver `which`.
 void chebyshev_solve(b2_ctx* c, int which, const CSR& pat, const double* vals, const double* dinv, int space, int K,
-                     const double* b, double* x, int32_t* reasons, int32_t* its);
+                     const double* b, double* x, int32_t* reasons, int32_t* its, DBuf<double>* w);
 
+// work: K-component work vectors of the operator's space (five for BiCGStab, three otherwise); nullptr: the step's own
+// wv / wq, which hold gdim velocity components or one pressure component
 void krylov_solve(b2_ctx* c, int which, const CSR& pat, const double* vals, const double* dinv_jacobi, int space,
                   int K, const double* b, double* x, int32_t* reasons, int32_t* its, DBuf<double>* work = nullptr) {
   KSPOpts& o = c->ksp[which];
-  if (o.type == 2 && work == nullptr) {
-    chebyshev_solve(c, which, pat, vals, dinv_jacobi, space, K, b, x, reasons, its);
+  DBuf<double>* w = work != nullptr ? work : (space == B2_SPACE_V ? c->wv : c->wq);
+  if (o.type == 2) {
+    chebyshev_solve(c, which, pat, vals, dinv_jacobi, space, K, b, x, reasons, its, w);
     return;
   }
-  DBuf<double>* w = work != nullptr ? work : (space == B2_SPACE_V ? c->wv : c->wq);
+  // krylov_init / krylov_iterations run every type other than CG as BiCGStab
+  B2_REQUIRE(o.type == 0 || o.type == 1 || o.type == 3, "unknown ksp type " + std::to_string(o.type));
   // CG: Jacobi through dinv in the vector kernels.  BiCGStab and GMRES: left preconditioning D^-1 A x = D^-1 b -- dinv
   // scales the right-hand side in k_bcgs_init / k_gmres_residual and every operator application in the SpMM epilogue
   // (the matrix is stored as assembled).  pc_type none: dinv = 1.
@@ -1053,10 +1057,9 @@ void read_sums(b2_ctx* c, int n);
 // [eig_lo, eig_hi].  No reductions inside the iteration; the residual norm is checked after the predicted
 // number of iterations and then every 4.
 void chebyshev_solve(b2_ctx* c, int which, const CSR& pat, const double* vals, const double* dinv, int space, int K,
-                     const double* b, double* x, int32_t* reasons, int32_t* its) {
+                     const double* b, double* x, int32_t* reasons, int32_t* its, DBuf<double>* w) {
   KSPOpts& o = c->ksp[which];
   B2_REQUIRE(o.eig_hi > o.eig_lo && o.eig_lo > 0.0, "ksp_type chebyshev needs ksp_chebyshev_eigenvalues lo,hi");
-  DBuf<double>* w = space == B2_SPACE_V ? c->wv : c->wq;
   double *r = w[0].p, *d = w[1].p, *q = w[2].p;
   const int64_t n = pat.n_rows;
   const int ld = pat.n_cols;

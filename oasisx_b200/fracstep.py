@@ -222,7 +222,8 @@ class FractionalStep_AB_CN:
         self._solver_u = KSPSolver(comm, solver_options.get("tentative"), prefix="tentative_velocity")
         self._solver_p = KSPSolver(comm, solver_options.get("pressure"), prefix="pressure_correction")
         self._solver_c = KSPSolver(comm, solver_options.get("scalar"), prefix="velocity_update")
-        if (solver_options.get("scalar") or {}).get("ksp_type") == "chebyshev" and "ksp_chebyshev_eigenvalues" not in solver_options["scalar"]:
+        cheb_bounds = (solver_options.get("scalar") or {}).get("ksp_type") == "chebyshev" and "ksp_chebyshev_eigenvalues" not in solver_options["scalar"]
+        if cheb_bounds:
             # rigorous bounds of spec(D^-1 M): extreme generalised eigenvalues of the reference element mass
             # matrix against its own diagonal (Wathen 1987) -- mesh independent for affine simplices
             lo, hi = _fem.mass_jacobi_bounds(gdim, deg_u)
@@ -232,6 +233,9 @@ class FractionalStep_AB_CN:
         self._solver_c.bind(ctx, L.SOLVER_SCALAR)
         if self._rotational:
             self._solver_proj = KSPSolver(comm, solver_options.get("scalar"), prefix="oasis_projector")
+            if cheb_bounds:  # the rotational projection solves with MQ, the P1 pressure mass matrix
+                lo, hi = _fem.mass_jacobi_bounds(gdim, 1)
+                self._solver_proj.updateOptions({"ksp_chebyshev_eigenvalues": f"{lo!r},{hi!r}"})
             self._solver_proj.bind(ctx, L.SOLVER_PROJECTOR)
         if len(self._bcs_p) == 0 and "ksp_type" not in (solver_options.get("pressure") or {}):
             # fracstep.py:562-576 forces a direct solve of the singular system; the device

@@ -84,10 +84,16 @@ class Projector:
         self._ctx: L.Context = _projection_context(space, device)
         # which device space carries this degree in that context (a solver's context may be P1-P1)
         self._slot = self._space_slot(space)
-        for k, v in (petsc_options or {}).items():
-            if k in ("ksp_type", "pc_type", "ksp_rtol", "ksp_atol", "ksp_max_it", "ksp_gmres_restart",
-                     "ksp_gmres_cgs_refinement_type"):
-                self._ctx.set_solver_option(L.SOLVER_PROJECTOR, k, v)
+        self._options = {k: v for k, v in (petsc_options or {}).items()
+                         if k in ("ksp_type", "pc_type", "ksp_rtol", "ksp_atol", "ksp_max_it", "ksp_gmres_restart",
+                                  "ksp_gmres_cgs_refinement_type", "ksp_chebyshev_eigenvalues")}
+        if self._options.get("ksp_type") == "chebyshev" and "ksp_chebyshev_eigenvalues" not in self._options:
+            # bounds of spec(D^-1 M) for the target's degree (fracstep.py does the same for the velocity update).  Dirichlet
+            # rows turn M into an identity-bordered principal submatrix: its Jacobi-scaled spectrum interlaces with the
+            # full one, and the identity's eigenvalue 1 lies inside the bounds, so they still hold.
+            lo, hi = _fem.mass_jacobi_bounds(space.mesh.geometry.dim, space.degree)
+            self._options["ksp_chebyshev_eigenvalues"] = f"{lo!r},{hi!r}"
+        self._push_options()
         degree = int((metadata or {}).get("quadrature_degree", 4))
         self._pts, self._w = simplex_rule(space.mesh.geometry.dim, degree)
         self._x = _fem.Function(space)
@@ -100,6 +106,11 @@ class Projector:
         self.assemble_rhs()
 
     # ---- helpers ---------------------------------------------------------------------------
+    def _push_options(self):
+        """The context's projector solver slot is shared by every Projector on it: each solve restates its options."""
+        for k, v in self._options.items():
+            self._ctx.set_solver_option(L.SOLVER_PROJECTOR, k, v)
+
     def _space_slot(self, sp: _fem.FunctionSpace) -> int:
         n = sp._scalar.num_dofs
         if self._ctx.space_size(L.SPACE_V) == n and self._ctx.space_degree(L.SPACE_V) == sp.degree:
@@ -177,6 +188,7 @@ class Projector:
         if assemble_rhs:
             self.assemble_rhs()
         ctx, bs, n = self._ctx, self._space.bs, self._space._scalar.num_dofs
+        self._push_options()
         self._push_bcs()
         ctx.project_load_rhs(self._slot, self._rhs)  # the right-hand side this object assembled last, all components
         out, reasons = ctx.project_solve(n, bs)      # one Krylov run on bs systems sharing the mass matrix
